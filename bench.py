@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU)
     python bench.py --impl reference --steps K --warmup W    # the reference's own CPU implementation on the host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + the last timed step's results as DIR/*.npy
 
 A "step" is one data-parallel training step of `base_model` on a batch of 64 synthetic 772x1032 grayscale images per
 GPU (BASELINE configs[1]): forward, YOGOLoss, backward, gradient all-reduce (N > 1, bucketed, overlapped with backward,
@@ -416,6 +417,7 @@ def run_ours(args):
     loss_fn = yogo_b200.YOGOLoss().to(dev)
     trainer = DataParallelTrainer(net, loss_fn, total_steps=10000, overlap=bool(args.overlap))
     trainer.broadcast_state()
+    initial = trainer.snapshot()   # seeded: the same on every run with the same arguments
     use_graph = bool(args.graph)
 
     nbuf = 2  # distinct host batches, alternated
@@ -452,16 +454,26 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     launches0 = L.load().yg_launch_count()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0, e1, e_pause, e_resume = (torch.cuda.Event(enable_timing=True) for _ in range(4))
     e0.record()
-    for i in range(args.steps):
-        loss = resident_step(i)
+    for i in range(args.steps - 1):
+        resident_step(i)
+    e_pause.record()
+    # The last timed step starts again from the seeded initial state (the restore is not timed).  The reductions of the
+    # kernels vary the last bits of a few gradients from run to run and AdamW spreads such differences over the steps
+    # that follow; restarting makes the last step compute from the same parameters, optimizer state and BatchNorm
+    # statistics on every run, so that its results (final_loss, --dump-outputs) are reproducible.
+    trainer.restore(initial)
+    e_resume.record()
+    loss = resident_step(args.steps - 1)
     e1.record()
     barrier()
     launches = L.load().yg_launch_count() - launches0
     if use_graph:
         launches = trainer.graph_launches * args.steps
-    ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, net)
+    ms = e0.elapsed_time(e_pause) + e_resume.elapsed_time(e1)
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -575,9 +587,26 @@ def run_ours(args):
                                     "sample": f"8 images/step of the same workload, fp32, {what}, 3 timed steps"}
     if rank == 0:
         print(json.dumps(line), flush=True)
-    sys.stdout.flush()
-    sys.stderr.flush()
-    os._exit(0)   # nothing left to do; skip interpreter teardown of CUDA / NCCL state
+
+
+def dump_outputs(out_dir, loss, net):
+    """What the last timed step hands its caller, as float32 .npy files: the loss, the updated parameters and the
+    (clamped) gradients they were updated with, both concatenated in `net.named_parameters()` order, and the BatchNorm
+    running statistics in `net.named_buffers()` order.  The step starts from the seeded initial state with seeded images,
+    labels and dropout masks, so the same arguments give the same inputs on every run and two builds can be compared
+    file by file."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    params = [p for _, p in net.named_parameters()]
+    arrays = {
+        "loss": loss.detach().float().reshape(1),
+        "params": torch.cat([p.detach().reshape(-1) for p in params]),
+        "grads": torch.cat([p.grad.reshape(-1) for p in params]),
+        "bn_running_stats": torch.cat([b.reshape(-1) for n, b in net.named_buffers() if "running_" in n]),
+    }
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def kernel_breakdown(trainer, dev_imgs, dev_labs, args, L):
@@ -709,7 +738,10 @@ def main():
     ap.add_argument("--fp32-x3", type=int, default=1, help="--dtype fp32: run the convolutions as split-bf16 x3 on the tensor cores")
     ap.add_argument("--tc-or", type=int, default=0, help="OR these bits into the conv engine's option word (A/B experiments)")
     ap.add_argument("--overlap", type=int, default=1, help="N > 1: all-reduce gradient buckets on a side stream while backward continues")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed training step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -17,3 +17,10 @@ def zoo_inputs(z, case):
     img = synth_images(N, H, W, seed=seed, channels=ch)
     lab = synth_labels(N, net.Sy, net.Sx, 7, K, seed=seed + 100)
     return name, net, img, lab, ostride
+
+
+def grad_sample(g, n):
+    """The `n` elements of the flat gradient `g` that a model_zoo.npz / model_full.npz case stores: every
+    ceil(size / 4096)-th, and of those every second one where the fixture keeps half (make_golden.py, `shrink`)."""
+    g = g[:: max(1, -(-g.size // 4096))]
+    return g if g.size == n else g[::2]

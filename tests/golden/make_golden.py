@@ -6,7 +6,7 @@ Run in the build container only (the reference does not exist on the GPU box):
 
 The reference is imported unmodified with the stubs of SURVEY.md 8c for modules that are
 off the hot path and absent here (matplotlib, zarr, ruamel.yaml; np.unicode_).
-Outputs are small .npz files committed next to this script.
+Outputs are small .npz files committed next to this script; `shrink` keeps each under 1 MB.
 """
 import os
 import sys
@@ -489,9 +489,78 @@ def golden_zoo(ref, out, table, fname, out_stride=1, pick_seed=False):
     np.savez_compressed(os.path.join(out, fname), **cases)
 
 
+FULL_OUT_STRIDE = 4
+ZOO_GRAD_KEEP = 2048
+
+
+def shrink(out):
+    """Keeps every fixture under 1 MB without changing a result of the reference.  Applying it again changes nothing.
+      - model_base.npz: the weights are replaced by their SHA-256 digest; tests/_golden.py regenerates them from the
+        seed of `_run_model` and checks the digest.
+      - nms.npz, nms2: the class probabilities of the cells at or below the objectness threshold are zeroed.  format_preds
+        drops those cells before it reads anything else, so no row or count can change; the oracle re-checks it here.
+      - model_full.npz: outputs on every FULL_OUT_STRIDE-th grid row and column (recorded in the cfg row).
+      - model_zoo.npz: gradient samples of more than ZOO_GRAD_KEEP elements keep every second one
+        (tests/_zoo_cases.py::grad_sample)."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    from _golden import digest
+    from oracle.yogo_oracle import format_preds_np, prediction_class_counts_np
+
+    def rewrite(fname, edit):
+        path = os.path.join(out, fname)
+        with np.load(path) as npz:
+            z = dict(npz.items())
+        if edit(z):
+            np.savez_compressed(path, **z)
+
+    def base(z):
+        sd = {k: z.pop(k) for k in list(z) if k.startswith("sd.")}
+        if sd:
+            z["digest.sd"] = np.array(digest(sd))
+        return bool(sd)
+
+    def nms(z):
+        p = z["nms2_pred"].copy()
+        obj, iou, xyxy, mincls = z["nms2_cfg"]
+        p[:, 5:] *= (p[:, 4:5] > np.float32(obj))
+        for b in range(p.shape[0]):
+            rows = format_preds_np(p[b], obj, iou, "xyxy" if xyxy else "cxcywh", mincls)
+            exp = z["nms2_rows"][z["nms2_offsets"][b]:z["nms2_offsets"][b + 1]]
+            assert rows.shape == exp.shape and np.array_equal(rows.view(np.uint32), exp.view(np.uint32))
+        assert np.array_equal(prediction_class_counts_np(p, obj, iou, mincls), z["nms2_counts"])
+        changed = not np.array_equal(p, z["nms2_pred"])
+        z["nms2_pred"] = p
+        return changed
+
+    def full(z):
+        changed = False
+        for k in [k for k in z if k.endswith(".cfg")]:
+            case, step = k[:-4], FULL_OUT_STRIDE // int(z[k][6])
+            if step > 1:
+                for o in (case + ".train.out", case + ".eval.out"):
+                    z[o] = z[o][:, :, ::step, ::step].copy()
+                z[k][6] = FULL_OUT_STRIDE
+                changed = True
+        return changed
+
+    def zoo(z):
+        big = [k for k in z if ".train.grad." in k and z[k].size > ZOO_GRAD_KEEP]
+        for k in big:
+            z[k] = z[k][::2].copy()
+        return bool(big)
+
+    rewrite("model_base.npz", base)
+    rewrite("nms.npz", nms)
+    rewrite("model_full.npz", full)
+    rewrite("model_zoo.npz", zoo)
+
+
 if __name__ == "__main__":
     torch.set_num_threads(1)
     torch.use_deterministic_algorithms(True)
+    if "--only-shrink" in sys.argv:  # shrink the committed fixtures alone (no reference needed)
+        shrink(HERE)
+        sys.exit(0)
     ref = import_reference()
     if "--only-match" in sys.argv:   # regenerate match.npz alone
         golden_match(ref, HERE)
@@ -503,6 +572,7 @@ if __name__ == "__main__":
         golden_zoo(ref, HERE, ZOO, "model_zoo.npz", pick_seed=True)
         torch.set_num_threads(16)
         golden_zoo(ref, HERE, FULL, "model_full.npz", out_stride=2)
+        shrink(HERE)
         sys.exit(0)
     golden_loss(ref, HERE)
     golden_nms(ref, HERE)
@@ -512,6 +582,7 @@ if __name__ == "__main__":
     golden_zoo(ref, HERE, ZOO, "model_zoo.npz", pick_seed=True)
     torch.set_num_threads(16)
     golden_zoo(ref, HERE, FULL, "model_full.npz", out_stride=2)
+    shrink(HERE)
     for f in sorted(os.listdir(HERE)):
         if f.endswith(".npz"):
             print(f, os.path.getsize(os.path.join(HERE, f)))

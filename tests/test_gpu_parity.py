@@ -11,15 +11,12 @@ import pytest
 import torch
 
 import yogo_b200
+from _golden import load as _load
 from yogo_b200 import _lib as L
 from oracle import yogo_oracle as O
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-
-
-def _load(golden_dir, name):
-    return np.load(os.path.join(golden_dir, name))
 
 
 def _rel(a, b):
@@ -838,7 +835,7 @@ def test_full_size_train_step_vs_oracle_fp32():
 
 
 # ----------------------------------------------------------------------------- every definition, RGB, BASELINE geometry
-from _zoo_cases import ZOO_CASES, zoo_inputs  # noqa: E402
+from _zoo_cases import ZOO_CASES, grad_sample, zoo_inputs  # noqa: E402
 
 FULL_CASES = ["full_base_model", "full_silu_model", "full_double_filters"]
 
@@ -864,7 +861,7 @@ def _zoo_step(z, case, dtype, impl="auto"):
     for k, p in net.named_parameters():
         g = p.grad.detach().cpu().numpy().reshape(-1)
         exp = z[prefix + "grad." + k]
-        g = g[:: max(1, -(-g.size // 4096))]
+        g = grad_sample(g, exp.size)
         scale = float(np.linalg.norm(exp))
         if k in zero_keys:
             scale = max(scale, float(z[prefix + "gradnorm." + zero_keys[k]][0]))

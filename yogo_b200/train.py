@@ -251,8 +251,7 @@ class DataParallelTrainer:
 
         # warm-up on a side stream (allocator pools, NCCL communicator and channel setup, library caches); parameters,
         # optimizer state, module buffers and the CUDA RNG stream (Dropout2d masks) are restored afterwards
-        snap = (self.flat_p.clone(), self.exp_avg.clone(), self.exp_avg_sq.clone(),
-                [b.clone() for b in self.net.buffers()], self.flat_g.clone())
+        snap = self.snapshot()
         rng = torch.cuda.get_rng_state(dev)
         self._hyper.copy_(self._hyper_host(1))
         s = torch.cuda.Stream(device=dev)
@@ -276,12 +275,23 @@ class DataParallelTrainer:
             pool = graph.pool()
             self._graphs.append(graph)
             self._graph_losses.append(loss)
-        self.flat_p.copy_(snap[0]); self.exp_avg.copy_(snap[1]); self.exp_avg_sq.copy_(snap[2]); self.flat_g.copy_(snap[4])
-        for b, v in zip(self.net.buffers(), snap[3]):
-            b.copy_(v)
+        self.restore(snap)
         torch.cuda.set_rng_state(rng, dev)
         torch.cuda.synchronize()
         self._graph = self._graphs[0]
+
+    def snapshot(self):
+        """Copies of the step count, parameters, gradients, optimizer state and module buffers, for `restore`."""
+        return (self.step_count, [t.clone() for t in (self.flat_p, self.flat_g, self.exp_avg, self.exp_avg_sq)],
+                [b.clone() for b in self.net.buffers()])
+
+    def restore(self, snap) -> None:
+        """Puts back what `snapshot` copied (stream-ordered copies on the current stream)."""
+        self.step_count = snap[0]
+        for t, v in zip((self.flat_p, self.flat_g, self.exp_avg, self.exp_avg_sq), snap[1]):
+            t.copy_(v)
+        for b, v in zip(self.net.buffers(), snap[2]):
+            b.copy_(v)
 
     def disable_cuda_graph(self) -> None:
         """Drop the captured graphs and the memory pool they pin.  With several ranks the graphs hold captured NCCL work and
