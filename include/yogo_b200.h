@@ -225,6 +225,29 @@ int yg_format_preds_batch(const float* preds, int B, int num_classes, int Sy, in
 int yg_box_iou_cost(const float* labels, int label_stride, int n_labels, const float* preds, int pred_stride,
                     int n_preds, float* cost, void* stream);
 
+/* Batched matching (format_preds_and_labels_v2 for a whole batch, the assignment solved on the device).
+ * yg_compact_labels: labels (B,6,Sy,Sx) fp32 -> rows (B, Sy*Sx, 6), image b's labelled cells (label[0] != 0, NaN
+ * included) packed at rows[b][0..n_labels[b]) in grid order.
+ * yg_lsap_batch: scipy.optimize.linear_sum_assignment of n fp32 matrices in one launch, identical indices.  desc (device,
+ * n x 4 int64) per matrix = [cost_off (floats into costs, row-major), ws_off (8-byte words into workspace, each matrix
+ * needs yg_lsap_workspace_words(rows, cols), a host function), out_off, rows | cols << 32]; out_rows / out_cols (int64)
+ * get the min(rows, cols) assigned pairs at out_off in ascending row; status[n] (int32) is always written with a
+ * yg_lsap_status, and outputs of a matrix whose status is not YG_LSAP_OK are undefined.
+ * yg_match_batch: after yg_format_preds_batch (xyxy rows) and yg_compact_labels, with desc[b] = (rows = labels of image b,
+ * cols = its kept predictions) and gather_off (device, B x 2 int64) = offsets of image b's missed / extra rows: one
+ * launch each for the cost matrices (into costs, same expression as yg_box_iou_cost), the assignment and the gather of
+ * out_preds (K, 5+C) / out_labels (K, 6) matched pairs in ascending label, missed (., 6) labels in ascending label and
+ * extra (., 5+C) predictions in ascending prediction index.  max_labels / max_preds bound the per-image counts. */
+enum { YG_LSAP_OK = 0, YG_LSAP_INVALID = 1 /* NaN or -inf entry */, YG_LSAP_INFEASIBLE = 2 /* a row cannot be assigned */ };
+int yg_compact_labels(const float* labels, int B, int Sy, int Sx, float* rows, int* n_labels, void* stream);
+long long yg_lsap_workspace_words(int rows, int cols);
+int yg_lsap_batch(const float* costs, const void* desc, int n, void* workspace, long long* out_rows, long long* out_cols,
+                  int* status, void* stream);
+int yg_match_batch(const float* label_rows, const float* pred_rows, int B, int cells, int num_classes, int max_labels,
+                   int max_preds, const void* desc, const long long* gather_off, float* costs, void* workspace,
+                   long long* pair_rows, long long* pair_cols, int* status, float* out_preds, float* out_labels,
+                   float* missed, float* extra, void* stream);
+
 /* ---- input side (SURVEY.md 8f N3) --------------------------------------------------------
  * RandomHorizontal/VerticalFlipWithBBs (data/data_transforms.py:51-98) of a whole batch, out of place:
  * images (N,C,H,W) uint8 (YG_U8) or fp32, labels (N,6,Sy,Sx) = [mask,x1,y1,x2,y2,class] with x1' = 1 - x2, x2' = 1 - x1

@@ -140,6 +140,14 @@ _PROTOS = {
          c_void_p, c_size_t, c_void_p],
     ),
     "yg_box_iou_cost": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "yg_compact_labels": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "yg_lsap_workspace_words": (c_longlong, [c_int, c_int]),
+    "yg_lsap_batch": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "yg_match_batch": (
+        c_int,
+        [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    ),
     "yg_flip_images": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_flip_labels": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_format_labels_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

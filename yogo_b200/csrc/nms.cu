@@ -40,25 +40,6 @@ struct NmsWs {
   unsigned long long* mask;     // [G][cells][nw] bit j of word w of row i: candidate 64 w + j (> i) is suppressed by i
 };
 
-// exclusive scan of one flag per thread over the block; returns rank, total via reference
-template <int THREADS>
-__device__ __forceinline__ int block_rank(bool flag, int* warp_tot /*[32]*/, int& total) {
-  const unsigned b = __ballot_sync(0xffffffffu, flag);
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int r = __popc(b & ((1u << lane) - 1u));
-  __syncthreads();  // protect warp_tot reuse
-  if (lane == 0) warp_tot[wid] = __popc(b);
-  __syncthreads();
-  int base = 0, tot = 0;
-  for (int w = 0; w < THREADS / 32; ++w) {
-    const int t = warp_tot[w];
-    if (w < wid) base += t;
-    tot += t;
-  }
-  total = tot;
-  return base + r;
-}
-
 __device__ __forceinline__ bool iou_gt(const float4 a, const float area_a, const float4 b, const float area_b,
                                        const double thr) {
   // torchvision/csrc/ops/cpu/nms_kernel.cpp semantics
@@ -464,35 +445,7 @@ extern "C" int yg_format_preds_batch(const float* preds, int B, int num_classes,
 namespace yg {
 __global__ void box_iou_cost_kernel(const float* __restrict__ a, int a_stride, int na, const float* __restrict__ b, int b_stride,
                                     int nb, float* __restrict__ cost) {
-  __shared__ float sb[256][5];
-  const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  const int i0 = blockIdx.y * 16;
-  // this thread's prediction box
-  float bx1 = 0.f, by1 = 0.f, bx2 = 0.f, by2 = 0.f, barea = 0.f;
-  if (j < nb) {
-    const float* r = b + (long long)j * b_stride;
-    bx1 = r[0]; by1 = r[1]; bx2 = r[2]; by2 = r[3];
-    barea = __fmul_rn(__fsub_rn(bx2, bx1), __fsub_rn(by2, by1));
-  }
-  // 16 label boxes of this block row through shared memory
-  if (threadIdx.x < 16 && i0 + threadIdx.x < na) {
-    const float* r = a + (long long)(i0 + threadIdx.x) * a_stride;
-    sb[threadIdx.x][0] = r[0]; sb[threadIdx.x][1] = r[1]; sb[threadIdx.x][2] = r[2]; sb[threadIdx.x][3] = r[3];
-    sb[threadIdx.x][4] = __fmul_rn(__fsub_rn(r[2], r[0]), __fsub_rn(r[3], r[1]));
-  }
-  __syncthreads();
-  if (j >= nb) return;
-  for (int k = 0; k < 16 && i0 + k < na; ++k) {
-    const float ax1 = sb[k][0], ay1 = sb[k][1], ax2 = sb[k][2], ay2 = sb[k][3], aarea = sb[k][4];
-    const float ltx = ax1 > bx1 ? ax1 : bx1, lty = ay1 > by1 ? ay1 : by1;
-    const float rbx = ax2 < bx2 ? ax2 : bx2, rby = ay2 < by2 ? ay2 : by2;
-    float w = __fsub_rn(rbx, ltx), h = __fsub_rn(rby, lty);
-    w = w < 0.f ? 0.f : w;   // clamp(min=0) keeps NaN
-    h = h < 0.f ? 0.f : h;
-    const float inter = __fmul_rn(w, h);
-    const float uni = __fsub_rn(__fadd_rn(aarea, barea), inter);
-    cost[(long long)(i0 + k) * nb + j] = __fsub_rn(1.f, __fdiv_rn(inter, uni));
-  }
+  box_iou_cost_tile(a, a_stride, na, b, b_stride, nb, cost, blockIdx.x * blockDim.x + threadIdx.x, blockIdx.y * 16);
 }
 }  // namespace yg
 

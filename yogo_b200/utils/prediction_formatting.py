@@ -6,7 +6,7 @@ prediction_formatting.py:166-330) and ``format_to_numpy`` (:96-156)."""
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Literal, Optional, Tuple, get_args
+from typing import List, Literal, Optional, Sequence, Tuple, get_args
 
 import numpy as np
 import torch
@@ -193,6 +193,135 @@ def format_preds_and_labels_v2(
         missed_labels=formatted_labels[label_free],
         extra_predictions=formatted_preds[pred_free],
     )
+
+
+_LSAP_ERRORS = {1: "matrix contains invalid numeric entries", 2: "cost matrix is infeasible"}   # scipy's messages
+
+
+def _lsap_status_check(status: torch.Tensor, what: str) -> None:
+    """Raise scipy's ValueError for the first matrix the solver rejected (one device->host read)."""
+    st = status.cpu().numpy()
+    bad = np.flatnonzero(st)
+    if bad.size:
+        k = int(bad[0])
+        raise ValueError(f"{_LSAP_ERRORS.get(int(st[k]), 'assignment failed')} ({what} {k})")
+
+
+def _upload_int64(table: np.ndarray, dev: torch.device) -> torch.Tensor:
+    return torch.from_numpy(np.ascontiguousarray(table, dtype=np.int64)).pin_memory().to(dev, non_blocking=True)
+
+
+def _exclusive_cumsum(x: np.ndarray) -> np.ndarray:
+    out = np.zeros_like(x)
+    np.cumsum(x[:-1], out=out[1:])
+    return out
+
+
+def _lsap_plan(rows: np.ndarray, cols: np.ndarray) -> Tuple[np.ndarray, int]:
+    """Descriptor table of yg_lsap_batch / yg_match_batch for matrices of the given shapes (include/yogo_b200.h): int64
+    [n, 4] = cost offset, workspace offset (8-byte words), output offset, rows | cols << 32, then for yg_match_batch
+    [n, 2] = offsets of each image's missed (rows - k) and extra (cols - k) rows, k = min(rows, cols).  Returns the flat
+    table and the workspace size in 8-byte words."""
+    lib = L.load()
+    rows, cols = np.asarray(rows, dtype=np.int64), np.asarray(cols, dtype=np.int64)
+    k = np.minimum(rows, cols)
+    words = np.array([lib.yg_lsap_workspace_words(int(r), int(c)) for r, c in zip(rows, cols)], dtype=np.int64)
+    desc = np.stack([_exclusive_cumsum(rows * cols), _exclusive_cumsum(words), _exclusive_cumsum(k), rows | (cols << 32)], 1)
+    goff = np.stack([_exclusive_cumsum(rows - k), _exclusive_cumsum(cols - k)], 1)
+    return np.concatenate([desc.reshape(-1), goff.reshape(-1)]), int(words.sum())
+
+
+@L.on_device(lambda costs: costs[0] if len(costs) else None)
+def linear_sum_assignment_batch(costs: Sequence[torch.Tensor]) -> List[Tuple[torch.Tensor, torch.Tensor]]:
+    """``scipy.optimize.linear_sum_assignment`` of several 2-D fp32 CUDA matrices (shapes may differ) in one launch of
+    the device solver (csrc/match.cu, one warp per matrix).  Returns int64 ``(row_ind, col_ind)`` per matrix on the
+    matrices' device, identical to scipy's.  Raises scipy's ValueError, naming the matrix, for NaN or -inf entries and
+    for a matrix whose +inf entries leave a row unassignable.  One host synchronisation (the solver status)."""
+    costs = list(costs)
+    if not costs:
+        return []
+    dev = costs[0].device
+    for k, c in enumerate(costs):
+        if c.ndim != 2:
+            raise ValueError(f"expected a matrix (2-D array), got a {c.ndim} array (cost matrix {k})")
+        L.require_cuda(c, "cost matrices")
+        if c.device != dev:
+            raise ValueError(f"cost matrix {k} is on {c.device}, cost matrix 0 on {dev}; all must be on one device")
+        if c.dtype != torch.float32:
+            raise ValueError(f"cost matrix {k} has dtype {c.dtype}; the solver takes torch.float32")
+    lib = L.lib()
+    n = len(costs)
+    rows = np.array([c.shape[0] for c in costs], dtype=np.int64)
+    cols = np.array([c.shape[1] for c in costs], dtype=np.int64)
+    k = np.minimum(rows, cols)
+    table, words = _lsap_plan(rows, cols)
+    flat = torch.cat([c.detach().reshape(-1) for c in costs])
+    out = torch.empty((2, max(int(k.sum()), 1)), dtype=torch.int64, device=dev)
+    status = torch.empty(n, dtype=torch.int32, device=dev)
+    ws = L.workspace.get("lsap", 8 * words, dev)
+    desc = _upload_int64(table, dev)
+    L.check(lib.yg_lsap_batch(flat.data_ptr(), desc.data_ptr(), n, ws.data_ptr(), out[0].data_ptr(), out[1].data_ptr(),
+                              status.data_ptr(), L.stream()))
+    _lsap_status_check(status, "cost matrix")
+    offs = _exclusive_cumsum(k)
+    return [(out[0, o:o + m], out[1, o:o + m]) for o, m in zip(offs.tolist(), k.tolist())]
+
+
+@L.on_device(lambda preds, *a, **k: preds)
+def format_preds_and_labels_batch(
+    preds: torch.Tensor,
+    labels: torch.Tensor,
+    objectness_thresh: float = 0.5,
+    min_class_confidence_threshold: float = 0.0,
+) -> Tuple[PredictionLabelMatch, torch.Tensor]:
+    """``format_preds_and_labels_v2`` for a whole batch: preds (B, 5+C, Sy, Sx) and labels (B, 6, Sy, Sx) on one CUDA
+    device -> (match, counts).  ``match`` is bit-identical to ``PredictionLabelMatch.concat`` of the per-image results
+    (matched pairs in ascending label index, missed labels, extra predictions in NMS order, image after image);
+    ``counts`` is a (B, 3) int64 CPU tensor of [matched, missed, extra] per image, for ``torch.split``.
+
+    Threshold + NMS, label gather, cost matrices, assignment (the device solver of ``linear_sum_assignment_batch``) and the
+    output gather are batched launches; the call synchronises twice whatever B is: once to read the per-image counts that
+    size the outputs, once to read the solver status (scipy's ValueError is raised for an image with a NaN cost, e.g. a
+    zero-area label and a zero-area prediction that do not overlap)."""
+    if preds.ndim != 4:
+        raise ValueError(f"expected batched predictions (B, pred_shape, Sy, Sx), got {tuple(preds.shape)}")
+    if labels.ndim != 4 or labels.shape[0] != preds.shape[0] or labels.shape[1] != 6 or labels.shape[2:] != preds.shape[2:]:
+        raise ValueError(f"expected batched labels (B, 6, Sy, Sx) matching predictions {tuple(preds.shape)}, got {tuple(labels.shape)}")
+    L.require_cuda(preds, "predictions")
+    L.require_cuda(labels, "labels")
+    if labels.device != preds.device:
+        raise ValueError(f"predictions on {preds.device} and labels on {labels.device}: both must be on one device")
+    rows, keep_count, _, _ = format_preds_batch(preds, objectness_thresh, 0.5, "xyxy", min_class_confidence_threshold)
+    lib = L.lib()
+    B, D, Sy, Sx = preds.shape
+    cells = Sy * Sx
+    dev = rows.device
+    lab = labels.detach().float().contiguous()
+    label_rows = torch.empty((B, cells, 6), dtype=torch.float32, device=dev)
+    n_labels = torch.empty(B, dtype=torch.int32, device=dev)
+    L.check(lib.yg_compact_labels(lab.data_ptr(), B, Sy, Sx, label_rows.data_ptr(), n_labels.data_ptr(), L.stream()))
+    cnt = torch.stack([n_labels, keep_count]).cpu().numpy().astype(np.int64)   # host synchronisation 1
+    N, M = cnt[0], cnt[1]
+    K = np.minimum(N, M)
+    counts = torch.from_numpy(np.stack([K, N - K, M - K], 1).astype(np.int64)).reshape(B, 3)
+    plan, words = _lsap_plan(N, M)
+    table = _upload_int64(plan, dev)
+    Kt, Nt, Mt = int(K.sum()), int(N.sum()), int(M.sum())
+    costs = torch.empty(max(int((N * M).sum()), 1), dtype=torch.float32, device=dev)
+    pairs = torch.empty((2, max(Kt, 1)), dtype=torch.int64, device=dev)
+    status = torch.empty(max(B, 1), dtype=torch.int32, device=dev)
+    ws = L.workspace.get("lsap", 8 * words, dev)
+    out_preds = torch.empty((Kt, D), dtype=torch.float32, device=dev)
+    out_labels = torch.empty((Kt, 6), dtype=torch.float32, device=dev)
+    missed = torch.empty((Nt - Kt, 6), dtype=torch.float32, device=dev)
+    extra = torch.empty((Mt - Kt, D), dtype=torch.float32, device=dev)
+    L.check(lib.yg_match_batch(label_rows.data_ptr(), rows.data_ptr(), B, cells, D - 5, int(N.max(initial=0)), int(M.max(initial=0)),
+                               table.data_ptr(), table[4 * B:].data_ptr(), costs.data_ptr(), ws.data_ptr(), pairs[0].data_ptr(),
+                               pairs[1].data_ptr(), status.data_ptr(), out_preds.data_ptr(), out_labels.data_ptr(),
+                               missed.data_ptr(), extra.data_ptr(), L.stream()))
+    if B:
+        _lsap_status_check(status[:B], "image")   # host synchronisation 2
+    return PredictionLabelMatch(preds=out_preds, labels=out_labels, missed_labels=missed, extra_predictions=extra), counts
 
 
 def format_to_numpy(img_id: int, prediction_tensor, img_h: int, img_w: int, np_dtype=np.float32) -> np.ndarray:
