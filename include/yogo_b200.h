@@ -248,6 +248,41 @@ int yg_match_batch(const float* label_rows, const float* pred_rows, int B, int c
                    long long* pair_rows, long long* pair_cols, int* status, float* out_preds, float* out_labels,
                    float* missed, float* extra, void* stream);
 
+/* Evaluation metrics (yogo_b200.metrics.Metrics), after yg_match_batch with the same rows, desc and gather_off.
+ * yg_confusion_batch: adds to confusion (int64, row-major nb x nb, nb = num_classes + 1 with include_background, else
+ * num_classes; rows = true class, columns = predicted class) the confusion matrix of
+ * PredictionLabelMatch.convert_background_errors(num_classes + 1): matched pairs (int(label[5]), argmax of the class
+ * columns and an appended 0), missed labels (int(label[5]), num_classes), extra predictions (num_classes, argmax of the
+ * class columns and an appended 0); without background only matched pairs, argmax over the class columns alone.
+ * out_preds / out_labels / missed / extra are yg_match_batch's outputs; lsap_status[B] its status (images whose status is
+ * not YG_LSAP_OK are skipped).  label_status[B] (int32) is written 1 for an image with a label class outside
+ * [0, num_classes) (such labels are not counted), else 0.
+ * yg_coco_match_batch: COCOeval.evaluateImg (bbox, no crowd, area "all", maxDet 100) of every image and class.  Detections
+ * are the kept xyxy rows of yg_format_preds_batch (pred_rows (B, cells, 5+C)), class = argmax of the class columns,
+ * score = objectness; ground truths are yg_compact_labels' rows (class int(label[5]), box label[1:5]).  iou_thrs (HOST,
+ * YG_COCO_IOU_THRS doubles) are COCO's np.linspace(.5, .95, 10).  Writes one record per kept detection, image b's at
+ * [prefix of the kept counts of images < b, + its kept count), in (class, rank) order: records (int32 n x 4) = [score
+ * (fp32 bits), class, image0 + b, rank | matched mask << 16] with rank the position within (image, class) by score
+ * descending then row index, and bit t of the mask set when the detection matched a ground truth at iou_thrs[t] (only
+ * ranks < 100 are matched); keys (int64 n) = class << 32 | a 32-bit key ascending in descending score, for a stable sort.
+ * Adds the per-class ground-truth counts to gt_count (int64 [num_classes]).  max_labels / max_preds bound the per-image
+ * counts (they size the shared memory).
+ * yg_coco_accumulate: COCOeval.accumulate over n_records records in the order perm (int64) that stably sorts keys
+ * (sorted_keys = keys[perm]), for every class, IoU threshold and maxDet in (1, 10, 100); rec_thrs (HOST,
+ * YG_COCO_REC_THRS doubles) = np.linspace(0, 1, 101).  precision (double [T][R][num_classes][3]) and recall
+ * (double [T][num_classes][3]) are overwritten, COCOeval's eval["precision"] / eval["recall"] without the area axis: -1
+ * for a class with gt_count 0. */
+enum { YG_COCO_IOU_THRS = 10, YG_COCO_REC_THRS = 101 };
+int yg_confusion_batch(const float* out_preds, const float* out_labels, const float* missed, const float* extra, int B,
+                       int num_classes, int include_background, const void* desc, const long long* gather_off,
+                       const int* lsap_status, int* label_status, long long* confusion, void* stream);
+int yg_coco_match_batch(const float* pred_rows, const float* label_rows, int B, int cells, int num_classes, int max_labels,
+                        int max_preds, const void* desc, const long long* gather_off, long long image0, const double* iou_thrs,
+                        int* records, long long* keys, long long* gt_count, void* stream);
+int yg_coco_accumulate(const int* records, const long long* sorted_keys, const long long* perm, long long n_records,
+                       const long long* gt_count, int num_classes, const double* rec_thrs, double* precision, double* recall,
+                       void* stream);
+
 /* ---- input side (SURVEY.md 8f N3) --------------------------------------------------------
  * RandomHorizontal/VerticalFlipWithBBs (data/data_transforms.py:51-98) of a whole batch, out of place:
  * images (N,C,H,W) uint8 (YG_U8) or fp32, labels (N,6,Sy,Sx) = [mask,x1,y1,x2,y2,class] with x1' = 1 - x2, x2' = 1 - x1

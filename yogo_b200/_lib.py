@@ -148,7 +148,20 @@ _PROTOS = {
         [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
     ),
-    "yg_flip_images": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "yg_confusion_batch": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    ),
+    "yg_coco_match_batch": (
+        c_int,
+        [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_longlong, C.POINTER(c_double), c_void_p,
+         c_void_p, c_void_p, c_void_p],
+    ),
+    "yg_coco_accumulate": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_int, C.POINTER(c_double), c_void_p, c_void_p, c_void_p],
+    ),
+    "yg_flip_images":(c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_flip_labels": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_format_labels_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "yg_dropout_scales": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p]),

@@ -165,10 +165,28 @@ __device__ __forceinline__ int block_rank(bool flag, int* warp_tot /*[32]*/, int
   return base + r;
 }
 
-// One tile of the matching cost cost[i][j] = 1 - box_iou(a_i, b_j) (torchvision.ops.box_iou = _box_inter_union):
-// column j (this thread's prediction box) of label rows i0 .. i0 + 15.  Every operation is a single correctly rounded
-// fp32 operation in torchvision's order (never contracted to FMA), so the matrix is bit-identical to the reference's.
-// Shared by yg_box_iou_cost (nms.cu) and the batched matching (match.cu); call with a block-uniform i0.
+// box_iou(a, b) of torchvision.ops (_box_inter_union) for two xyxy boxes with their areas (x2 - x1) * (y2 - y1)
+// precomputed the same way.  Every operation is a single correctly rounded fp32 operation in torchvision's order (never
+// contracted to FMA).  The one copy of the IoU expression: the matching cost tile below and the COCO matching
+// (metrics.cu) both use it.
+__device__ __forceinline__ float box_iou_f(float ax1, float ay1, float ax2, float ay2, float aarea, float bx1, float by1,
+                                           float bx2, float by2, float barea) {
+  const float ltx = ax1 > bx1 ? ax1 : bx1, lty = ay1 > by1 ? ay1 : by1;
+  const float rbx = ax2 < bx2 ? ax2 : bx2, rby = ay2 < by2 ? ay2 : by2;
+  float w = __fsub_rn(rbx, ltx), h = __fsub_rn(rby, lty);
+  w = w < 0.f ? 0.f : w;   // clamp(min=0) keeps NaN
+  h = h < 0.f ? 0.f : h;
+  const float inter = __fmul_rn(w, h);
+  const float uni = __fsub_rn(__fadd_rn(aarea, barea), inter);
+  return __fdiv_rn(inter, uni);
+}
+__device__ __forceinline__ float box_area_f(float x1, float y1, float x2, float y2) {
+  return __fmul_rn(__fsub_rn(x2, x1), __fsub_rn(y2, y1));
+}
+
+// One tile of the matching cost cost[i][j] = 1 - box_iou(a_i, b_j): column j (this thread's prediction box) of label
+// rows i0 .. i0 + 15, bit-identical to the reference's matrix.  Shared by yg_box_iou_cost (nms.cu) and the batched
+// matching (match.cu); call with a block-uniform i0.
 __device__ __forceinline__ void box_iou_cost_tile(const float* __restrict__ a, int a_stride, int na, const float* __restrict__ b,
                                                   int b_stride, int nb, float* __restrict__ cost, int j, int i0) {
   __shared__ float sb[16][5];
@@ -177,27 +195,29 @@ __device__ __forceinline__ void box_iou_cost_tile(const float* __restrict__ a, i
   if (j < nb) {
     const float* r = b + (long long)j * b_stride;
     bx1 = r[0]; by1 = r[1]; bx2 = r[2]; by2 = r[3];
-    barea = __fmul_rn(__fsub_rn(bx2, bx1), __fsub_rn(by2, by1));
+    barea = box_area_f(bx1, by1, bx2, by2);
   }
   // 16 label boxes of this block row through shared memory
   if (threadIdx.x < 16 && i0 + threadIdx.x < na) {
     const float* r = a + (long long)(i0 + threadIdx.x) * a_stride;
     sb[threadIdx.x][0] = r[0]; sb[threadIdx.x][1] = r[1]; sb[threadIdx.x][2] = r[2]; sb[threadIdx.x][3] = r[3];
-    sb[threadIdx.x][4] = __fmul_rn(__fsub_rn(r[2], r[0]), __fsub_rn(r[3], r[1]));
+    sb[threadIdx.x][4] = box_area_f(r[0], r[1], r[2], r[3]);
   }
   __syncthreads();
   if (j >= nb) return;
   for (int k = 0; k < 16 && i0 + k < na; ++k) {
-    const float ax1 = sb[k][0], ay1 = sb[k][1], ax2 = sb[k][2], ay2 = sb[k][3], aarea = sb[k][4];
-    const float ltx = ax1 > bx1 ? ax1 : bx1, lty = ay1 > by1 ? ay1 : by1;
-    const float rbx = ax2 < bx2 ? ax2 : bx2, rby = ay2 < by2 ? ay2 : by2;
-    float w = __fsub_rn(rbx, ltx), h = __fsub_rn(rby, lty);
-    w = w < 0.f ? 0.f : w;   // clamp(min=0) keeps NaN
-    h = h < 0.f ? 0.f : h;
-    const float inter = __fmul_rn(w, h);
-    const float uni = __fsub_rn(__fadd_rn(aarea, barea), inter);
-    cost[(long long)(i0 + k) * nb + j] = __fsub_rn(1.f, __fdiv_rn(inter, uni));
+    const float iou = box_iou_f(sb[k][0], sb[k][1], sb[k][2], sb[k][3], sb[k][4], bx1, by1, bx2, by2, barea);
+    cost[(long long)(i0 + k) * nb + j] = __fsub_rn(1.f, iou);
   }
 }
+
+// one cost matrix of the batched matching: host-built, uploaded as int64 [4] = cost_off, ws_off (8-byte words), out_off,
+// rows | cols << 32 (rows = labels, cols = kept predictions of one image).  Read by match.cu and metrics.cu.
+struct LsapDesc {
+  long long cost_off;
+  long long ws_off;
+  long long out_off;
+  int rows, cols;
+};
 
 }  // namespace yg

@@ -22,14 +22,6 @@ constexpr int MATCH_MAX_CELLS = 16384;   // Sy*Sx limit, as format_preds
 constexpr int MATCH_THREADS = 256;       // gather kernel
 constexpr int LABEL_THREADS = 1024;      // label compaction
 
-// one cost matrix: host-built, uploaded as int64 [4] = cost_off, ws_off (8-byte words), out_off, rows | cols << 32
-struct LsapDesc {
-  long long cost_off;
-  long long ws_off;
-  long long out_off;
-  int rows, cols;
-};
-
 // per-matrix workspace in 8-byte words: double u[nr], v[nc], spc[nc]; int path[nc], row4col[nc], remaining[nc],
 // visited[nc], col4row[nr] (nr <= nc after the transpose)
 __host__ __device__ inline long long lsap_words(int rows, int cols) {

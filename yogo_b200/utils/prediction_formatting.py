@@ -267,22 +267,26 @@ def linear_sum_assignment_batch(costs: Sequence[torch.Tensor]) -> List[Tuple[tor
     return [(out[0, o:o + m], out[1, o:o + m]) for o, m in zip(offs.tolist(), k.tolist())]
 
 
-@L.on_device(lambda preds, *a, **k: preds)
-def format_preds_and_labels_batch(
-    preds: torch.Tensor,
-    labels: torch.Tensor,
-    objectness_thresh: float = 0.5,
-    min_class_confidence_threshold: float = 0.0,
-) -> Tuple[PredictionLabelMatch, torch.Tensor]:
-    """``format_preds_and_labels_v2`` for a whole batch: preds (B, 5+C, Sy, Sx) and labels (B, 6, Sy, Sx) on one CUDA
-    device -> (match, counts).  ``match`` is bit-identical to ``PredictionLabelMatch.concat`` of the per-image results
-    (matched pairs in ascending label index, missed labels, extra predictions in NMS order, image after image);
-    ``counts`` is a (B, 3) int64 CPU tensor of [matched, missed, extra] per image, for ``torch.split``.
+@dataclass
+class _BatchMatch:
+    """Everything the batched matching computes, before its solver status is read: the match and its per-image counts,
+    and the intermediates that the metrics reuse (yogo_b200.metrics)."""
 
-    Threshold + NMS, label gather, cost matrices, assignment (the device solver of ``linear_sum_assignment_batch``) and the
-    output gather are batched launches; the call synchronises twice whatever B is: once to read the per-image counts that
-    size the outputs, once to read the solver status (scipy's ValueError is raised for an image with a NaN cost, e.g. a
-    zero-area label and a zero-area prediction that do not overlap)."""
+    match: PredictionLabelMatch
+    counts: torch.Tensor       # (B, 3) int64 CPU: matched, missed, extra per image
+    rows: torch.Tensor         # (B, Sy*Sx, 5+C) xyxy rows of format_preds_batch, image b's first keep_count[b] are kept
+    keep_count: torch.Tensor   # (B,) int32
+    label_rows: torch.Tensor   # (B, Sy*Sx, 6) labelled cells in grid order (yg_compact_labels), first n_labels[b] valid
+    n_labels: torch.Tensor     # (B,) int32
+    n_host: np.ndarray         # n_labels and keep_count on the host (int64)
+    m_host: np.ndarray
+    table: torch.Tensor        # device plan of _lsap_plan: desc (B x 4), then gather offsets (B x 2)
+    status: torch.Tensor       # (B,) solver status on the device, not yet read
+
+
+def _match_batch(preds: torch.Tensor, labels: torch.Tensor, objectness_thresh: float,
+                 min_class_confidence_threshold: float) -> _BatchMatch:
+    """The body of format_preds_and_labels_batch up to (not including) the read of the solver status."""
     if preds.ndim != 4:
         raise ValueError(f"expected batched predictions (B, pred_shape, Sy, Sx), got {tuple(preds.shape)}")
     if labels.ndim != 4 or labels.shape[0] != preds.shape[0] or labels.shape[1] != 6 or labels.shape[2:] != preds.shape[2:]:
@@ -319,9 +323,30 @@ def format_preds_and_labels_batch(
                                table.data_ptr(), table[4 * B:].data_ptr(), costs.data_ptr(), ws.data_ptr(), pairs[0].data_ptr(),
                                pairs[1].data_ptr(), status.data_ptr(), out_preds.data_ptr(), out_labels.data_ptr(),
                                missed.data_ptr(), extra.data_ptr(), L.stream()))
-    if B:
-        _lsap_status_check(status[:B], "image")   # host synchronisation 2
-    return PredictionLabelMatch(preds=out_preds, labels=out_labels, missed_labels=missed, extra_predictions=extra), counts
+    match = PredictionLabelMatch(preds=out_preds, labels=out_labels, missed_labels=missed, extra_predictions=extra)
+    return _BatchMatch(match, counts, rows, keep_count, label_rows, n_labels, N, M, table, status[:B])
+
+
+@L.on_device(lambda preds, *a, **k: preds)
+def format_preds_and_labels_batch(
+    preds: torch.Tensor,
+    labels: torch.Tensor,
+    objectness_thresh: float = 0.5,
+    min_class_confidence_threshold: float = 0.0,
+) -> Tuple[PredictionLabelMatch, torch.Tensor]:
+    """``format_preds_and_labels_v2`` for a whole batch: preds (B, 5+C, Sy, Sx) and labels (B, 6, Sy, Sx) on one CUDA
+    device -> (match, counts).  ``match`` is bit-identical to ``PredictionLabelMatch.concat`` of the per-image results
+    (matched pairs in ascending label index, missed labels, extra predictions in NMS order, image after image);
+    ``counts`` is a (B, 3) int64 CPU tensor of [matched, missed, extra] per image, for ``torch.split``.
+
+    Threshold + NMS, label gather, cost matrices, assignment (the device solver of ``linear_sum_assignment_batch``) and the
+    output gather are batched launches; the call synchronises twice whatever B is: once to read the per-image counts that
+    size the outputs, once to read the solver status (scipy's ValueError is raised for an image with a NaN cost, e.g. a
+    zero-area label and a zero-area prediction that do not overlap)."""
+    r = _match_batch(preds, labels, objectness_thresh, min_class_confidence_threshold)
+    if preds.shape[0]:
+        _lsap_status_check(r.status, "image")   # host synchronisation 2
+    return r.match, r.counts
 
 
 def format_to_numpy(img_id: int, prediction_tensor, img_h: int, img_w: int, np_dtype=np.float32) -> np.ndarray:
