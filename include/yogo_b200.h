@@ -283,6 +283,35 @@ int yg_coco_accumulate(const int* records, const long long* sorted_keys, const l
                        const long long* gt_count, int num_classes, const double* rec_thrs, double* precision, double* recall,
                        void* stream);
 
+/* ROC and calibration error (torchmetrics MulticlassROC(thresholds=None) / MulticlassCalibrationError(norm="l1")) over the
+ * rows of convert_background_errors(num_classes + 1): matched pairs (score = class columns and an appended 0, target
+ * int(label[5])), missed labels (one-hot background, target int(label[5])), extra predictions (class columns and a 0,
+ * target num_classes); without background the matched pairs alone over the num_classes columns.  nb = the columns.
+ * yg_score_rows_batch: after yg_match_batch with the same outputs, desc, gather_off and lsap_status (n_matched / n_extra =
+ * the row counts of out_preds / extra).  *softmax_flag (device int, overwritten) = 1 when a class value of the matched or
+ * (with background) extra rows lies outside [0, 1] or is NaN; then every score row is softmaxed (fp64, rounded to fp32).
+ * With scores (float R x nb) and targets (int32 R) non-null, image b's rows are written at [out_off + gather_off[2b] +
+ * gather_off[2b+1], + N + M - K) (with background; else [out_off, + K)) in matched / missed / extra order.  nan_status[B]
+ * (int32) is written 1 for an image with a NaN score.  Calibration: confidence = row maximum, prediction = its first
+ * maximum, bin = bucketize(confidence, bin_bounds, right=True) - 1 with bin_bounds (HOST, bins + 1 floats, bins <= 255)
+ * torch.linspace(0, 1, bins + 1); partials (device, B * (bins + 1) * 16 bytes) hold the per-image sums, and bin_count,
+ * bin_correct (int64 [bins + 1]) and bin_conf (double [bins + 1], the confidence sums) are overwritten with their sums over
+ * the images in order.  Images whose lsap_status is not YG_LSAP_OK contribute nothing.
+ * yg_roc_keys: keys[k * rows + r] = k << 32 | a 32-bit key ascending in descending scores[r][k] (-0 keyed as +0).
+ * yg_roc_curves: after sorting those keys (sorted_keys = keys[perm], int64), per class k the curve of _binary_clf_curve
+ * with the point (0, 0, threshold 1) prepended: fpr / tpr (double) and thresholds (float) of class k at [k * (rows + 1),
+ * + lengths[k]) (int64 [nb]); fpr = fps / fps_last (all 0 without negatives), tpr = tps / tps_last (all 0 without
+ * positives), the thresholds are the scores.  auc (double [nb]) = the trapezoidal area, -1 for a class without positive or
+ * negative rows. */
+int yg_score_rows_batch(const float* out_preds, const float* out_labels, const float* missed, const float* extra,
+                        long long n_matched, long long n_extra, int B, int num_classes, int include_background, const void* desc,
+                        const long long* gather_off, const int* lsap_status, const float* bin_bounds, int bins, int* softmax_flag,
+                        float* scores, int* targets, int* nan_status, void* partials, long long* bin_count,
+                        long long* bin_correct, double* bin_conf, void* stream);
+int yg_roc_keys(const float* scores, long long rows, int nb, long long* keys, void* stream);
+int yg_roc_curves(const long long* sorted_keys, const long long* perm, const int* targets, long long rows, int nb, double* fpr,
+                  double* tpr, float* thresholds, long long* lengths, double* auc, void* stream);
+
 /* ---- input side (SURVEY.md 8f N3) --------------------------------------------------------
  * RandomHorizontal/VerticalFlipWithBBs (data/data_transforms.py:51-98) of a whole batch, out of place:
  * images (N,C,H,W) uint8 (YG_U8) or fp32, labels (N,6,Sy,Sx) = [mask,x1,y1,x2,y2,class] with x1' = 1 - x2, x2' = 1 - x1

@@ -161,6 +161,16 @@ _PROTOS = {
         c_int,
         [c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_int, C.POINTER(c_double), c_void_p, c_void_p, c_void_p],
     ),
+    "yg_score_rows_batch": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_longlong, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+         C.POINTER(c_float), c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    ),
+    "yg_roc_keys": (c_int, [c_void_p, c_longlong, c_int, c_void_p, c_void_p]),
+    "yg_roc_curves": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    ),
     "yg_flip_images":(c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_flip_labels": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_format_labels_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -7,8 +7,15 @@
 //                           detections ranked by score within their class, then one warp per (class, IoU threshold) walks
 //                           the first 100 and takes ground truths greedily; one record per kept detection
 //   coco_accumulate_kernel  one CTA per (class, IoU threshold, maxDet): COCOeval.accumulate over the score-sorted records
+//   score_format_kernel     torchmetrics' format rule of one update: does any class value lie outside [0, 1]
+//   score_rows_kernel       one CTA per image: the score rows of convert_background_errors (softmaxed or not) with their
+//                           targets, NaN rows flagged, confidence / accuracy binned into per-CTA partials;
+//                           score_bins_reduce_kernel sums the partials in image order
+//   roc_keys_kernel,        compute(): class-major keys of every score; after a sort, one CTA per class walks its segment
+//   roc_curve_kernel        (block scans of positives and of distinct-score boundaries) and writes the ROC curve and AUC
 //
-// tools/coco_eval_np.py restates the same algorithm in numpy; the GPU tests compare against it bit for bit.
+// tools/coco_eval_np.py and tools/roc_ece_np.py restate the same algorithms in numpy; the GPU tests compare against them
+// bit for bit.
 #include "common.cuh"
 
 namespace yg {
@@ -255,8 +262,265 @@ __global__ void __launch_bounds__(COCO_ACC_THREADS) coco_accumulate_kernel(
   }
 }
 
+// ---- ROC and calibration: score rows ---------------------------------------------------------------------------------
+// The rows are those of convert_background_errors(C + 1) (matched, missed, extra; without background the matched pairs
+// alone), grouped by image: image b's start at out_off + gather_off[2b] + gather_off[2b + 1] (prefix of N + M - K).
+constexpr int MET_MAX_BINS = 255;        // calibration bins; bins + 1 <= SCORE_THREADS, one accumulating thread per bin
+constexpr int SCORE_THREADS = 256;
+constexpr int ROC_THREADS = 512;
+struct BinBounds { float b[MET_MAX_BINS + 1]; };
+
+// torchmetrics' format rule: *flag = 1 when a class value of the matched (and, with background, extra) rows lies outside
+// [0, 1] or is NaN; the caller zeroes *flag
+__global__ void score_format_kernel(const float* __restrict__ out_preds, const float* __restrict__ extra, long long n_matched,
+                                    long long n_extra, int C, int* __restrict__ flag) {
+  const long long nm = n_matched * C, n = nm + n_extra * C;
+  bool bad = false;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const long long j = i < nm ? i : i - nm;
+    const float x = (i < nm ? out_preds : extra)[(j / C) * (5 + C) + 5 + j % C];
+    bad |= !(x >= 0.f && x <= 1.f);
+  }
+  if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) atomicOr(flag, 1);
+}
+
+// column k of a score row before the format rule: the class columns and the appended 0 of a prediction row, or the
+// one-hot background row of a missed label (src == nullptr)
+__device__ __forceinline__ float raw_score(const float* __restrict__ src, int k, int C) {
+  return src ? (k < C ? src[5 + k] : 0.f) : (k == C ? 1.f : 0.f);
+}
+
+// One CTA per image.  Each row: its nb scores (softmaxed in fp64 over all nb columns when *softmax_flag) into
+// scores[row][.] and its target into targets[row] (when scores != nullptr); confidence = the row maximum of the stored
+// scores, prediction = its first maximum, bin = bucketize(conf, bounds, right=True) - 1.  The per-bin sums go to
+// partials[b] in a fixed order: rows in chunks of SCORE_THREADS, thread t sums bin t over a chunk in row order.
+__global__ void __launch_bounds__(SCORE_THREADS) score_rows_kernel(
+    const float* __restrict__ out_preds, const float* __restrict__ out_labels, const float* __restrict__ missed,
+    const float* __restrict__ extra, int C, int with_bg, const LsapDesc* __restrict__ desc, const long long* __restrict__ gather_off,
+    const int* __restrict__ lsap_status, const int* __restrict__ softmax_flag, const __grid_constant__ BinBounds bounds, int bins,
+    float* __restrict__ scores, int* __restrict__ targets, int* __restrict__ nan_status, unsigned char* __restrict__ partials) {
+  __shared__ float sb[MET_MAX_BINS + 1];
+  __shared__ float chunk_conf[SCORE_THREADS];
+  __shared__ int chunk_key[SCORE_THREADS];   // bin << 1 | correct, -1 for no row
+  __shared__ int nan_row;
+  const int b = blockIdx.x, tid = threadIdx.x, nb = C + (with_bg ? 1 : 0), nbin = bins + 1;
+  double* p_conf = reinterpret_cast<double*>(partials) + (long long)b * nbin;
+  int* p_count = reinterpret_cast<int*>(partials + (long long)gridDim.x * nbin * 8) + (long long)b * nbin * 2;
+  for (int i = tid; i < nbin; i += SCORE_THREADS) sb[i] = bounds.b[i];
+  if (tid == 0) nan_row = 0;
+  const bool ok = lsap_status[b] == YG_LSAP_OK;   // else the gather wrote no rows; the caller raises the solver's error
+  const LsapDesc d = desc[b];
+  const int N = ok ? d.rows : 0, M = ok ? d.cols : 0, K = min(N, M);
+  const int n_rows = with_bg ? N + M - K : K;
+  const long long row0 = with_bg ? d.out_off + gather_off[2 * b] + gather_off[2 * b + 1] : d.out_off;
+  const bool softmax = *softmax_flag != 0;
+  __syncthreads();
+  double acc_conf = 0.0;
+  int acc_count = 0, acc_correct = 0;
+  for (int c0 = 0; c0 < n_rows; c0 += SCORE_THREADS) {
+    const int t = c0 + tid;
+    int key = -1;
+    float conf = 0.f;
+    if (t < n_rows) {
+      // target: int(label[5]) (-1 for a class outside [0, C): the confusion kernel's check raises), C for an extra row
+      const float* src;
+      int target;
+      if (t < K) {
+        src = out_preds + (d.out_off + t) * (5 + C);
+        target = label_class(out_labels[(d.out_off + t) * 6 + 5], C);
+      } else if (t < N) {
+        src = nullptr;
+        target = label_class(missed[(gather_off[2 * b] + t - K) * 6 + 5], C);
+      } else {
+        src = extra + (gather_off[2 * b + 1] + t - N) * (5 + C);
+        target = C;
+      }
+      double m = -INFINITY;
+      for (int k = 0; k < nb; ++k) m = fmax(m, (double)raw_score(src, k, C));
+      double s = 0.0;
+      if (softmax)
+        for (int k = 0; k < nb; ++k) s += exp((double)raw_score(src, k, C) - m);
+      float best = 0.f;
+      int arg = 0;
+      bool has_nan = false;   // a NaN class value, or an infinite one under the softmax
+      for (int k = 0; k < nb; ++k) {
+        const float x = raw_score(src, k, C);
+        const float v = softmax ? (float)(exp((double)x - m) / s) : x;
+        has_nan |= v != v;
+        if (k == 0 || v > best) { best = v; arg = k; }
+        if (scores) scores[(row0 + t) * nb + k] = v;
+      }
+      if (scores) targets[row0 + t] = target;
+      if (has_nan) nan_row = 1;
+      int lo = 0, hi = nbin;   // boundaries <= best
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (sb[mid] <= best) lo = mid + 1; else hi = mid; }
+      key = ((lo > 0 ? lo - 1 : 0) << 1) | (arg == target ? 1 : 0);
+      conf = best;
+    }
+    chunk_key[tid] = key;
+    chunk_conf[tid] = conf;
+    __syncthreads();
+    if (tid < nbin) {
+      const int lim = min(SCORE_THREADS, n_rows - c0);
+      for (int i = 0; i < lim; ++i) {
+        const int kk = chunk_key[i];
+        if ((kk >> 1) == tid) { acc_conf += (double)chunk_conf[i]; ++acc_count; acc_correct += kk & 1; }
+      }
+    }
+    __syncthreads();
+  }
+  if (tid < nbin) { p_conf[tid] = acc_conf; p_count[2 * tid] = acc_count; p_count[2 * tid + 1] = acc_correct; }
+  if (tid == 0) nan_status[b] = nan_row;
+}
+
+// the fixed-order second step: bin i of every CTA partial, images in order
+__global__ void score_bins_reduce_kernel(const unsigned char* __restrict__ partials, int B, int nbin, long long* __restrict__ count,
+                                         long long* __restrict__ correct, double* __restrict__ conf) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nbin) return;
+  const double* p_conf = reinterpret_cast<const double*>(partials);
+  const int* p_count = reinterpret_cast<const int*>(partials + (long long)B * nbin * 8);
+  double s = 0.0;
+  long long n = 0, c = 0;
+  for (int b = 0; b < B; ++b) {
+    s += p_conf[(long long)b * nbin + i];
+    n += p_count[((long long)b * nbin + i) * 2];
+    c += p_count[((long long)b * nbin + i) * 2 + 1];
+  }
+  count[i] = n;
+  correct[i] = c;
+  conf[i] = s;
+}
+
+// ---- ROC curves ------------------------------------------------------------------------------------------------------
+// key[k * R + r] = k << 32 | score_desc_key(score[r][k]); -0 is keyed as +0 so that equal scores form one group
+__global__ void roc_keys_kernel(const float* __restrict__ scores, long long R, int nb, long long* __restrict__ keys) {
+  const long long n = R * nb;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const long long k = i / R, r = i - k * R;
+    const float s = scores[r * nb + k];
+    keys[i] = (k << 32) | score_desc_key(s == 0.f ? 0.f : s);
+  }
+}
+
+__device__ __forceinline__ float desc_key_score(unsigned key) {
+  const unsigned u = ~key;
+  return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
+}
+
+// One CTA per class k over its sorted segment: _binary_clf_curve (one point at the last row of every distinct score,
+// tps = positives so far, fps = rows so far - tps) after the prepended point (0, 0, threshold 1); fpr / tpr in fp64.
+// AUC = sum over points of (fps_j - fps_j-1) * (tps_j + tps_j-1), an exact integer, over 2 * fps_last * tps_last.
+__global__ void __launch_bounds__(ROC_THREADS) roc_curve_kernel(
+    const long long* __restrict__ sorted_keys, const long long* __restrict__ perm, const int* __restrict__ targets, long long R,
+    double* __restrict__ fpr, double* __restrict__ tpr, float* __restrict__ thresholds, long long* __restrict__ lengths,
+    double* __restrict__ auc) {
+  __shared__ int warp_tot[32];
+  __shared__ long long pt_tps[ROC_THREADS], pt_row[ROC_THREADS];
+  __shared__ unsigned long long area;
+  __shared__ long long n_pos;
+  const int k = blockIdx.x, tid = threadIdx.x;
+  const long long seg = (long long)k * R, out0 = (long long)k * (R + 1);
+  if (tid == 0) { area = 0ull; n_pos = 0; }
+  __syncthreads();
+  long long cnt = 0;
+  for (long long r = tid; r < R; r += ROC_THREADS) cnt += targets[r] == k;
+  atomicAdd(reinterpret_cast<unsigned long long*>(&n_pos), (unsigned long long)cnt);
+  __syncthreads();
+  const long long P = n_pos, F = R - P;
+  const double dP = (double)P, dF = (double)F;
+  if (tid == 0) { fpr[out0] = 0.0; tpr[out0] = 0.0; thresholds[out0] = 1.f; }
+  long long tps_carry = 0, pts = 0, prev_tps = 0, prev_row = -1;   // prev_*: the last point so far (the prepended one)
+  unsigned long long my_area = 0ull;
+  for (long long c0 = 0; c0 < R; c0 += ROC_THREADS) {
+    const long long i = c0 + tid;
+    bool pos = false, last = false;
+    unsigned key = 0u;
+    if (i < R) {
+      key = (unsigned)sorted_keys[seg + i];
+      pos = targets[perm[seg + i] - seg] == k;
+      last = i == R - 1 || (unsigned)sorted_keys[seg + i + 1] != key;
+    }
+    int tot_pos, tot_last;
+    const int r_pos = block_rank<ROC_THREADS>(pos, warp_tot, tot_pos);
+    const int r_last = block_rank<ROC_THREADS>(last, warp_tot, tot_last);
+    const long long tps = tps_carry + r_pos + (pos ? 1 : 0);
+    if (last) { pt_tps[r_last] = tps; pt_row[r_last] = i; }
+    __syncthreads();
+    if (last) {
+      const long long fps = i + 1 - tps, o = out0 + pts + 1 + r_last;
+      const long long ptp = r_last ? pt_tps[r_last - 1] : prev_tps, prw = r_last ? pt_row[r_last - 1] : prev_row;
+      my_area += (unsigned long long)(fps - (prw + 1 - ptp)) * (unsigned long long)(tps + ptp);
+      fpr[o] = F > 0 ? __ddiv_rn((double)fps, dF) : 0.0;
+      tpr[o] = P > 0 ? __ddiv_rn((double)tps, dP) : 0.0;
+      thresholds[o] = desc_key_score(key);
+    }
+    if (tot_last) { prev_tps = pt_tps[tot_last - 1]; prev_row = pt_row[tot_last - 1]; }
+    tps_carry += tot_pos;
+    pts += tot_last;
+    __syncthreads();   // pt_* are rewritten by the next chunk
+  }
+  atomicAdd(&area, my_area);
+  __syncthreads();
+  if (tid == 0) {
+    lengths[k] = pts + 1;
+    auc[k] = (P > 0 && F > 0) ? __ddiv_rn((double)area, __dmul_rn(2.0 * dF, dP)) : -1.0;
+  }
+}
+
 }  // namespace yg
 using namespace yg;
+
+extern "C" int yg_score_rows_batch(const float* out_preds, const float* out_labels, const float* missed, const float* extra,
+                                   long long n_matched, long long n_extra, int B, int num_classes, int include_background,
+                                   const void* desc, const long long* gather_off, const int* lsap_status, const float* bin_bounds,
+                                   int bins, int* softmax_flag, float* scores, int* targets, int* nan_status, void* partials,
+                                   long long* bin_count, long long* bin_correct, double* bin_conf, void* stream) {
+  YG_CHECK_ARG(B >= 0 && num_classes >= 1 && num_classes <= MET_MAX_CLASSES && n_matched >= 0 && n_extra >= 0,
+               "score_rows_batch: B = %d, num_classes = %d", B, num_classes);
+  YG_CHECK_ARG(bins >= 1 && bins <= MET_MAX_BINS, "score_rows_batch: %d bins, between 1 and %d are supported", bins, MET_MAX_BINS);
+  YG_CHECK_ARG(bin_bounds && softmax_flag && bin_count && bin_correct && bin_conf && (B == 0 || (desc && gather_off && lsap_status &&
+               nan_status && partials)), "score_rows_batch: null pointer");
+  YG_CHECK_ARG(!scores == !targets, "score_rows_batch: scores and targets go together");
+  cudaStream_t st = (cudaStream_t)stream;
+  YG_CUDA(cudaMemsetAsync(softmax_flag, 0, sizeof(int), st));
+  const long long n_values = (n_matched + (include_background ? n_extra : 0)) * num_classes;
+  if (n_values > 0) {
+    score_format_kernel<<<(int)std::min<long long>(cdiv(n_values, 256), 1184), 256, 0, st>>>(
+        out_preds, extra, n_matched, include_background ? n_extra : 0, num_classes, softmax_flag);
+    YG_LAUNCH_CHECK("score_format");
+  }
+  BinBounds bb;
+  for (int i = 0; i <= bins; ++i) bb.b[i] = bin_bounds[i];
+  if (B > 0) {
+    score_rows_kernel<<<B, SCORE_THREADS, 0, st>>>(out_preds, out_labels, missed, extra, num_classes, include_background ? 1 : 0,
+                                                   (const LsapDesc*)desc, gather_off, lsap_status, softmax_flag, bb, bins, scores,
+                                                   targets, nan_status, (unsigned char*)partials);
+    YG_LAUNCH_CHECK("score_rows");
+  }
+  score_bins_reduce_kernel<<<cdiv(bins + 1, 256), 256, 0, st>>>((const unsigned char*)partials, B, bins + 1, bin_count, bin_correct,
+                                                                bin_conf);
+  YG_LAUNCH_CHECK("score_bins_reduce");
+  return YG_OK;
+}
+
+extern "C" int yg_roc_keys(const float* scores, long long rows, int nb, long long* keys, void* stream) {
+  YG_CHECK_ARG(rows >= 0 && rows < 0x7fffffffLL && nb >= 1 && nb <= MET_MAX_CLASSES + 1, "roc_keys: rows = %lld, nb = %d", rows, nb);
+  if (rows == 0) return YG_OK;
+  YG_CHECK_ARG(scores && keys, "roc_keys: null pointer");
+  roc_keys_kernel<<<(int)std::min<long long>(cdiv(rows * nb, 256), 4736), 256, 0, (cudaStream_t)stream>>>(scores, rows, nb, keys);
+  YG_LAUNCH_CHECK("roc_keys");
+  return YG_OK;
+}
+
+extern "C" int yg_roc_curves(const long long* sorted_keys, const long long* perm, const int* targets, long long rows, int nb,
+                             double* fpr, double* tpr, float* thresholds, long long* lengths, double* auc, void* stream) {
+  YG_CHECK_ARG(rows >= 0 && rows < 0x7fffffffLL && nb >= 1 && nb <= MET_MAX_CLASSES + 1, "roc_curves: rows = %lld, nb = %d", rows, nb);
+  YG_CHECK_ARG(fpr && tpr && thresholds && lengths && auc && (rows == 0 || (sorted_keys && perm && targets)), "roc_curves: null pointer");
+  roc_curve_kernel<<<nb, ROC_THREADS, 0, (cudaStream_t)stream>>>(sorted_keys, perm, targets, rows, fpr, tpr, thresholds, lengths, auc);
+  YG_LAUNCH_CHECK("roc_curves");
+  return YG_OK;
+}
 
 extern "C" int yg_confusion_batch(const float* out_preds, const float* out_labels, const float* missed, const float* extra, int B,
                                   int num_classes, int include_background, const void* desc, const long long* gather_off,
