@@ -44,18 +44,12 @@ int yg_device_check(void);
  * shape qualifies, SIMT otherwise).  Used by the parity tests to cross-check both. */
 int yg_set_conv_impl(int impl);
 int yg_get_conv_impl(void);
-/* debug/tuning switch of the tcgen05 engine (default 25 + 8192 + 16384): bit 0 = weights resident in shared memory when they fit,
- * bit 1 = cp.async producer for 16/32-channel operands, bit 2 = L2 prefetch warp, bit 3 = W-fold of small-channel
- * stride-1 layers, bit 4 = column-pair fold of small-channel stride-2 dgrad, bits 5-6 = cap the K chunk at 32 / 16,
- * bits 7-11 = profiling knobs of tools/bench_conv.py (skip stores / MMAs / epilogue / TMA, cycle counters),
- * bit 12 = swizzle-phase experiment, bit 13 = 2-D halo boxes, bit 14 = CTA pairs (cta_group::2) for 128->128 layers,
- * bit 15 = CTA pairs for stride-2 dgrad (slower), bit 16 = mma.sync wgrad also for 32->64 stride 2 (slower),
- * bit 17 = no mma.sync wgrad at all, bit 18 = no CTA pairs for N = 64 stride-1 dgrad,
- * bit 19 = no merged row taps (one N = 192 MMA) in the 64-input-channel wgrad, bit 20 = stride-2 wgrad fetches the dz tile once
- * per parity group instead of once per tile, bit 21 = fp32 tensors as split-bf16 "x3" convolutions on the tensor cores
- * (csrc/x3.cu; off by default: the exact SIMT kernels are the fp32 parity path), bit 22 = MMA issue by the per-tap table walk
- * instead of the flat host-built list (same MMAs in the same order; slower), bits 24-26 = A-operand pipeline depth of the
- * tcgen05 conv engine: 0 = at most 4 stages (default), 1..6 = at most 2..7, 7 = every stage that fits in shared memory. */
+/* option word of the convolution engines (default 0).  yg_set_tc_options returns YG_ERR_INVALID for any other bit.
+ * bits 7-11 = profiling knobs of the tcgen05 engine read by tools/bench_conv.py: 7 = no global stores, 8 = no MMA issue,
+ * 9 = the epilogue skips its TMEM loads and math, 10 = no TMA loads, 11 = cycle counters of the MMA and epilogue warps
+ * (read with yg_tc_debug_read);
+ * bit 21 = fp32 tensors as split-bf16 "x3" convolutions on the tensor cores (csrc/x3.cu; yogo_b200.set_fp32_tensor_cores;
+ * off by default: the exact SIMT kernels are the fp32 parity path). */
 int yg_set_tc_options(int options);
 int yg_get_tc_options(void);
 /* profiling hook: copies n (<= 2048) cycle counters written by the engine's MMA warps (8 per CTA) to host memory. */

@@ -399,6 +399,11 @@ SHAPES = [
     (1, 10, 14, 128, 128, 3, 1),
     (2, 10, 14, 48, 96, 3, 1),
     (2, 10, 14, 24, 12, 1, 1),
+    # stride-2 dgrad with folded column pairs (Cin <= 32, even W)
+    (2, 21, 38, 32, 64, 3, 2),
+    # W-folded dgrad whose folded K of 256 channels spans 4 K chunks (one MMA issue list per chunk), fold 4 and fold 2
+    (2, 12, 20, 16, 64, 3, 1),
+    (2, 12, 18, 32, 128, 3, 1),
     # double_filters / triple_filters widths (model_defns.py:130-227): N = 256 MMAs, non-resident weights
     (2, 9, 11, 128, 256, 3, 1),
     (1, 10, 14, 256, 256, 3, 1),
@@ -1085,44 +1090,6 @@ def test_conv_outputs_stay_inside_their_buffers(shape):
     assert bool(torch.isfinite(dx.float()).all()) and bool(torch.isfinite(dw).all())
 
 
-@pytest.mark.parametrize("shape", [(2, 40, 64, 16, 32, 1), (2, 39, 36, 64, 128, 1), (2, 41, 38, 32, 64, 2), (2, 37, 36, 128, 128, 2),
-                                   (2, 33, 24, 128, 128, 1), (1, 38, 40, 48, 96, 1)])
-def test_flat_mma_issue_list_is_bit_identical_to_the_table_walk(shape):
-    """The MMA warp issues from a flat host-built list (one word per MMA, structurally zero K steps of W-folded layers left out);
-    option bit 22 restores the per-tap table walk.  Same MMAs in the same order: forward and dgrad outputs must be bit-identical
-    (W-folded, CTA-pair, stride-2 parity-class and streamed-weight configurations)."""
-    import ctypes as C
-    N, H, W, Cin, Cout, s = shape
-    lib = L.lib()
-    g = torch.Generator().manual_seed(sum(shape))
-    dt = torch.bfloat16
-    Ho, Wo = (H - 1) // s + 1, (W - 1) // s + 1
-    x = torch.randn(N, H, W, Cin, generator=g).to(DEV).to(dt)
-    w = (torch.randn(Cout, Cin, 3, 3, generator=g) / (Cin * 9) ** 0.5).to(DEV)
-    b = (torch.randn(Cout, generator=g) * 0.1).to(DEV)
-    dz = torch.randn(N, Ho, Wo, Cout, generator=g).to(DEV).to(dt)
-    xmask = torch.randint(0, 255, (N * H * W * Cin // 8,), generator=g, dtype=torch.uint8).to(DEV)
-    outs = []
-    base = lib.yg_get_tc_options()
-    try:
-        for bit in (0, 1 << 22):
-            L.check(lib.yg_set_tc_options(base | bit))
-            y = torch.zeros(N, Ho, Wo, Cout, dtype=dt, device=DEV)
-            m = torch.zeros(y.numel() // 8, dtype=torch.uint8, device=DEV)
-            ep = L.FwdEpilogue(None, b.data_ptr(), L.ACT_LRELU, None, None, None, m.data_ptr())
-            L.check(lib.yg_conv_fwd(x.data_ptr(), w.data_ptr(), y.data_ptr(), 1, N, H, W, Cin, Cout, 3, s, C.byref(ep), L.stream()))
-            dx = torch.zeros(N, H, W, Cin, dtype=dt, device=DEV)
-            be = L.BwdEpilogue(x.data_ptr(), L.ACT_LRELU, None, None, None, None, None, None, xmask.data_ptr())
-            L.check(lib.yg_conv_dgrad(dz.data_ptr(), w.data_ptr(), dx.data_ptr(), 1, N, H, W, Cin, Cout, 3, s, C.byref(be), L.stream()))
-            torch.cuda.synchronize()
-            outs.append((y, m, dx))
-    finally:
-        L.check(lib.yg_set_tc_options(base))
-    assert bool(outs[0][0].float().abs().sum() > 0) and bool(outs[0][2].float().abs().sum() > 0)
-    for a, b_ in zip(outs[0], outs[1]):
-        assert torch.equal(a, b_)
-
-
 FULL_LAYERS = [
     # (N, H, W, Cin, Cout, stride): every 3x3 layer of base_model / double_filters at the 772x1032 geometry
     (3, 386, 516, 16, 32, 1), (3, 386, 516, 32, 64, 2), (3, 193, 258, 64, 128, 1), (3, 193, 258, 128, 128, 2),
@@ -1248,7 +1215,8 @@ def test_conv_tensors_larger_than_4GiB():
 
 @pytest.mark.parametrize("shape", [(2, 19, 35, 16, 32, 1), (1, 8, 32, 16, 32, 1), (3, 21, 37, 32, 64, 2), (2, 40, 70, 16, 32, 1)])
 def test_small_channel_wgrad_on_mma_sync_matches_autograd(shape):
-    """wgrad_hmma.cu (16->32 by default, 32->64 stride 2 with option bit 16) against autograd of the CPU convolution."""
+    """Small-channel weight gradients against autograd of the CPU convolution: wgrad_hmma.cu for 16->32 stride 1, the tcgen05
+    wgrad for 32->64 stride 2."""
     N, H, W, Cin, Cout, s = shape
     g = torch.Generator().manual_seed(sum(shape))
     lib = L.lib()
@@ -1263,17 +1231,13 @@ def test_small_channel_wgrad_on_mma_sync_matches_autograd(shape):
     dz = torch.randn(y.shape, generator=g)
     dzd = dz.permute(0, 2, 3, 1).contiguous().to(DEV).bfloat16()
     y.backward(dzd.float().permute(0, 3, 1, 2).cpu())
-    lib.yg_set_tc_options(25 + 8192 + 16384 + 65536)
-    try:
-        dw = torch.empty(Cout, Cin, 3, 3, device=DEV)
-        db = torch.empty(Cout, device=DEV)
-        nb = lib.yg_conv_wgrad_workspace(N, H, W, Cin, Cout, 3, s)
-        ws = torch.empty(max(nb, 16), dtype=torch.uint8, device=DEV)
-        L.check(lib.yg_conv_wgrad(xd.data_ptr(), dzd.data_ptr(), dw.data_ptr(), db.data_ptr(), 1, N, H, W, Cin, Cout, 3, s, 0.0,
-                                  ws.data_ptr(), nb, L.stream()))
-        assert _rel(dw.cpu(), wr.grad) < 1e-4 and _rel(db.cpu(), br.grad) < 1e-4
-    finally:
-        lib.yg_set_tc_options(25 + 8192 + 16384)
+    dw = torch.empty(Cout, Cin, 3, 3, device=DEV)
+    db = torch.empty(Cout, device=DEV)
+    nb = lib.yg_conv_wgrad_workspace(N, H, W, Cin, Cout, 3, s)
+    ws = torch.empty(max(nb, 16), dtype=torch.uint8, device=DEV)
+    L.check(lib.yg_conv_wgrad(xd.data_ptr(), dzd.data_ptr(), dw.data_ptr(), db.data_ptr(), 1, N, H, W, Cin, Cout, 3, s, 0.0,
+                              ws.data_ptr(), nb, L.stream()))
+    assert _rel(dw.cpu(), wr.grad) < 1e-4 and _rel(db.cpu(), br.grad) < 1e-4
 
 
 def test_multi_rank_equivalence(tmp_path):

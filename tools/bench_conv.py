@@ -33,13 +33,15 @@ def main():
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--impl", default="auto")
     ap.add_argument("--stats", type=int, default=0)
-    ap.add_argument("--tc-options", type=int, default=24601)
+    ap.add_argument("--tc-options", type=int, default=None, help="option word of include/yogo_b200.h (default: leave as is)")
     ap.add_argument("--no-saved", type=int, default=0)
     ap.add_argument("--mask", type=int, default=0)
     args = ap.parse_args()
     lib = L.lib()
     L.set_conv_impl(args.impl)
-    lib.yg_set_tc_options(args.tc_options)
+    if args.tc_options is not None:
+        L.check(lib.yg_set_tc_options(args.tc_options))
+    opt = lib.yg_get_tc_options()
     dev = "cuda:0"
     N = args.batch
     peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json"))) if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else {"bf16_tflops": 1590.0, "hbm_gbs": 6650.0}
@@ -89,9 +91,9 @@ def main():
             ms = e0.elapsed_time(e1) / max(args.reps, 1)   # --reps 0: one launch per op (ncu captures)
             tf = flops / ms / 1e9
             act_bytes = (N * H * W * Cin + N * Ho * Wo * Cout) * 2
-            rec = {"opt": args.tc_options, "layer": li, "op": name, "shape": [N, H, W, Cin, Cout, s], "ms": round(ms, 4), "TFLOPs": round(tf, 1),
+            rec = {"opt": opt, "layer": li, "op": name, "shape": [N, H, W, Cin, Cout, s], "ms": round(ms, 4), "TFLOPs": round(tf, 1),
                    "frac_bf16_peak": round(tf / peaks["bf16_tflops"], 3), "min_GBps": round(act_bytes / ms / 1e6, 1)}
-            if (args.tc_options >> 11) & 1 and name != "wgrad":
+            if (opt >> 11) & 1 and name != "wgrad":
                 import numpy as np
                 buf = np.zeros(148 * 16, dtype=np.uint64)
                 L.check(lib.yg_tc_debug_read(buf.ctypes.data, buf.size))

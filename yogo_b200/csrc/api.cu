@@ -167,10 +167,8 @@ extern "C" int yg_conv_wgrad(const void* x, const void* dz, float* dw, float* db
     set_error("conv_wgrad: tcgen05 path forced but shape unsupported");
     return YG_ERR_INVALID;
   }
-  // 16 -> 32 channels: warp-level tensor cores without W-fold waste (wgrad_hmma.cu: 0.54 -> 0.38 ms on base L2).  The 32 -> 64
-  // stride-2 variant is correct but bound by the legacy mma.sync rate (0.55 vs 0.47 ms): only with option bit 16; bit 17 disables both
-  if (g_conv_impl != YG_IMPL_SIMT && !(yg_get_tc_options_raw() & 131072) && wgrad_hmma_supported(dtype, W, Cin, Cout, ks, stride) &&
-      (Cin == 16 || (yg_get_tc_options_raw() & 65536)))
+  // 16 -> 32 channels: warp-level tensor cores without W-fold waste (wgrad_hmma.cu: 0.54 -> 0.38 ms on base L2)
+  if (g_conv_impl != YG_IMPL_SIMT && wgrad_hmma_supported(dtype, W, Cin, Cout, ks, stride))
     return conv_wgrad_hmma(x, dz, dw, dbias, N, H, W, Cin, Cout, ks, stride, clip, workspace, workspace_bytes, (cudaStream_t)stream);
   if (tc_ok && g_conv_impl != YG_IMPL_SIMT)
     return conv_wgrad_tc(x, dz, dw, dbias, N, H, W, Cin, Cout, ks, stride, clip, workspace, workspace_bytes, (cudaStream_t)stream);

@@ -18,8 +18,8 @@
 //   epilogue    tcgen05.ld 32x32b -> registers -> bias / folded BN / activation / Dropout2d scale / sign mask (fwd),
 //               activation backward from the sign mask or the saved tensor, optional BN sums (dgrad), 16-byte bf16
 //               stores; straight-line 32-column fast paths for the common flavours; the YOGO head transform.
-// Warp roles (352 threads): warp 0 TMA producer, warp 1 MMA issuer + TMEM owner, warps 2-9 epilogue, warp 10 optional
-// L2 prefetch.  The weight-gradient kernel (wgrad_tc_kernel, below) has its own header.
+// Warp roles (352 threads): warp 0 TMA producer, warp 1 MMA issuer + TMEM owner, warps 2-9 epilogue, warp 10 idle (see
+// conv_tc_kernel).  The weight-gradient kernel (wgrad_tc_kernel, below) has its own header.
 #include "common.cuh"
 #include <cuda.h>
 #include <cudaTypedefs.h>
@@ -29,8 +29,11 @@
 namespace yg {
 
 constexpr int TC_TH = 8, TC_TW = 16;          // output tile (pixels), M = 128
-// conv_tc_kernel: (1 or 2) producer warps + 1 MMA warp + 8 epilogue warps
+// conv_tc_kernel: 1 producer warp + 1 MMA warp + 8 epilogue warps + 1 idle warp
 constexpr int TC_MAX_GROUPS = 9, TC_MAX_TAPS = 9, TW_MAX_TAPS = 3;
+// MMA issue list bounds: W-folded layers have a folded K <= 256 (see fold_factor), i.e. at most 16 K steps of 16 per tap:
+// 9 taps x 16 = 144 MMAs per tile in at most 16 per-chunk lists; every other layer has one list of at most 9 taps x 4 K steps
+constexpr int TC_MAX_LISTS = 16, TC_MAX_MMAS = 144;
 constexpr int TC_SMEM_BUDGET = 227 * 1024 - 14 * 1024;
 constexpr uint32_t TC_SPIN_LIMIT = 1u << 24;   // bounded mbarrier spin: trap instead of hanging the GPU
 
@@ -48,12 +51,6 @@ struct TcGroup {
   unsigned kmask[TC_MAX_TAPS];  // bit kk: global 16-wide K step kk of this tap has non-zero weights (W-folded convs)
 };
 
-struct TcSrc {            // A-operand source as seen by the cp.async producer (element strides)
-  const bf16* base;
-  int Wd, Hd;
-  long long sw, sh, sn;
-};
-
 struct TcClass {   // one output-parity class of a stride-2 dgrad (or the whole problem when ncls == 1)
   int g0, ng, gpi;          // its groups: p.g[g0 .. g0+ng), merged gpi at a time into one pipeline item
   int TSH, TSW, oh0, ow0;   // tile-space extent and output offset
@@ -65,20 +62,14 @@ struct TcParams {
   int bt_stride;                    // weight-tile slots per group in a streamed-weight stage
   int cta2;                         // CTA pairs (cta_group::2): M = 256 per MMA, each CTA holds BN/2 rows of every weight tile
   int ncls, cls_rot;                // classes and the rotation period max(1, grid / ncls) (see tile_class)
-  unsigned long long fd_ncls, fd_rot, fd_nnt, fd_tw, fd_th;   // ceil(2^32 / d): division by multiply-high (decode_tile)
-  // class-per-round tile order (CTA pairs with parity classes): round k of the persistent grid works on class k % ncls
-  // for every CTA (a pair always shares its class, sibling classes of a spatial tile run in consecutive rounds)
-  int cls_round, grid, tpc;           // flag, grid size, tiles per class
-  unsigned long long fd_grid, fd_ocr;
+  unsigned long long fd_ncls, fd_rot, fd_nnt, fd_tw, fd_th, fd_ocr;   // ceil(2^32 / d): division by multiply-high (decode_tile)
   TcClass cls[4];
   int b_resident, resb_bytes;     // all weight tiles live in smem for the whole kernel
-  TcSrc src[4];
   int OH, OW, OC, osh, osw;       // output tensor (NHWC) and tile-space -> output strides (rows, columns)
   int OCr;                        // real channel count (OC / W-fold factor): per-channel arrays are indexed modulo OCr
   int BN, kchunks, nstages, nacc;
   int a_box_bytes, b_stage_bytes;   // bytes reserved per A box / per stage for streamed weight tiles
   int ntaps_total;                  // weight slices in the packed weight tensor (9 for 3x3, 1 for 1x1)
-  int pf_ahead;           // L2 prefetch distance in tiles (0 = off)
   int a_stage_bytes, b_tap_bytes, tmem_cols;
   TcGroup g[TC_MAX_GROUPS];
   void* out;
@@ -93,18 +84,15 @@ struct TcParams {
   const void* saved; const float* bn_scale; const float* bn_shift; const float* bn_mean; const float* bn_invstd;
   double* bn_sums;
   int* error_flag;
-  // MMA issue table (host-built, read through the constant bank = uniform loads): per (group, tap) the operand
-  // offsets inside a stage in 16-byte descriptor units and the K-step mask; ebeg[g] = first entry of group g
-  uint32_t tab_a[27], tab_b[27], tab_km[27], tab_hi[27];   // tab_hi: high descriptor word of A (SBO = box row pitch)
-  int ebeg[TC_MAX_GROUPS + 1];
-  // The same table flattened to one word per MMA (A offset | B offset << 16, 16-byte units; K steps with structurally zero
-  // weights of W-folded layers left out), so the issue loop is load - add - issue instead of a per-tap mask walk.
-  // flat_rng[L][g] = first MMA of group g in list L; W-folded layers have one list per K chunk (L = kc, at most 2),
-  // everything else one list for all chunks.
-  int flat_on, flat_perkc;
-  int flat_rng[2][TC_MAX_GROUPS + 1];
-  uint32_t flat_ab[108];
-  int shift_exp[TC_MAX_GROUPS];   // experiment (option bit 12): extra A start offset in bytes per group
+  // MMA issue list (host-built, read through the constant bank = uniform loads): one word per MMA, A offset | B offset << 16
+  // inside a stage in 16-byte descriptor units, K steps with structurally zero weights of W-folded layers left out, so the
+  // issue loop is load - add - issue.  flat_rng[L][g] = first MMA of group g in list L; W-folded layers have one list per
+  // K chunk (L = kc), everything else one list for all chunks.  a_hi[g]: high descriptor word of group g's A operand
+  // (SBO = box row pitch: the parity boxes of one stride-2 pipeline item differ in width).
+  int flat_perkc;
+  int flat_rng[TC_MAX_LISTS][TC_MAX_GROUPS + 1];
+  uint32_t flat_ab[TC_MAX_MMAS];
+  uint32_t a_hi[TC_MAX_GROUPS];
   int io_f32;  // the epilogue reads `saved` and writes `out` / `preact` as fp32 (split-bf16 "x3" convolutions of fp32 tensors, see x3.cu)
   int debug;   // profiling knobs (tools/bench_conv.py): 1 = no global stores, 2 = no MMA issue, 4 = epilogue skips TMEM loads and math, 8 = no TMA loads, 16 = MMA-warp cycle counters -> g_tc_dbg
 };
@@ -121,30 +109,17 @@ __device__ __forceinline__ int fdiv(int n, unsigned long long m) {   // n / d fo
 }
 __device__ __forceinline__ int tile_class(const TcParams& p, int tile) {
   if (p.ncls == 1) return 0;
-  if (p.cls_round) {
-    const int round = fdiv(tile, p.fd_grid);
-    return round - fdiv(round, p.fd_ncls) * p.ncls;
-  }
   const int sp = fdiv(tile, p.fd_ncls), c = tile - sp * p.ncls;
   const int x = c + fdiv(sp, p.fd_rot);
   return x - fdiv(x, p.fd_ncls) * p.ncls;
 }
 // tile index -> (class, N tile, tile column, tile row, image); the class is the fastest index.  Division by multiply-high:
 // every role decodes every tile, and four runtime integer divisions cost several hundred cycles of a single warp.
-// Padding tiles (CTA pairs, class-per-round order) decode to n >= N: all their loads are out of bounds (zero fill) and
-// the epilogue stores nothing.
+// The padding tile of a CTA pair decodes to n >= N: all its loads are out of bounds (zero fill) and the epilogue stores
+// nothing.
 __device__ __forceinline__ void decode_tile(const TcParams& p, int tile, int& cls, int& nt, int& tw, int& th, int& n) {
-  int t;
-  if (p.cls_round) {
-    const int round = fdiv(tile, p.fd_grid), b = tile - round * p.grid;
-    const int rc = fdiv(round, p.fd_ncls);
-    cls = round - rc * p.ncls;
-    t = rc * p.grid + b;                       // spatial index inside the class
-    if (t >= p.tpc) { nt = 0; tw = 0; th = 0; n = p.N; return; }
-  } else {
-    cls = tile_class(p, tile);
-    t = fdiv(tile, p.fd_ncls);
-  }
+  cls = tile_class(p, tile);
+  int t = fdiv(tile, p.fd_ncls);
   int q = fdiv(t, p.fd_nnt); nt = t - q * p.n_ntiles; t = q;
   q = fdiv(t, p.fd_tw); tw = t - q * p.tiles_w; t = q;
   q = fdiv(t, p.fd_th); th = t - q * p.tiles_h; n = q;
@@ -437,20 +412,15 @@ __device__ __forceinline__ float lane_transpose_reduce16(float (&v)[16], int lan
 __device__ __forceinline__ float round_bf16(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
 
 // ------------------------------------------------------------------------------------------ kernel
-// PROD = 0: A operand by TMA (one producer lane).  PROD = 1: A operand by cp.async from two producer warps
-// writing the swizzled layout by hand - for 16/32-channel tensors, whose 32/64-byte rows make TMA
-// request-rate bound (~4-8 cycles per row measured) - with all weights resident in shared memory.
-template <int KC, int MODE, int PROD, int CTA2 = 0>
-__global__ void __launch_bounds__((PROD ? 2 : 1) * 32 + 320, 1)
+// 352 threads, of which warp 10 has no role: with a 320-thread bound ptxas allocates the 168 registers differently and the
+// dgrad instantiations spill more (52 instead of 40 bytes, 60 instead of 56 for CTA pairs; nvcc 12.9 -Xptxas -v).
+template <int KC, int MODE, int CTA2 = 0>
+__global__ void __launch_bounds__(352, 1)
 conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcParams p) {
-  constexpr int PW = PROD ? 2 : 1;             // producer warps; MMA warp = PW; epilogue warps PW+1 .. PW+8
-  constexpr int NTHREADS = PW * 32 + 320;      // + 1 MMA warp + 8 epilogue warps + 1 L2-prefetch warp
-  constexpr int CPR = KC / 8;                  // 16-byte chunks per operand row
-  constexpr int LAG = 2;                       // cp.async groups kept in flight per producer thread
+  constexpr int NTHREADS = 352;
   constexpr uint32_t ROW_BYTES = KC * 2;
   constexpr uint32_t SBO = 8 * ROW_BYTES;
   constexpr uint32_t LAYOUT = KC == 64 ? 2u : (KC == 32 ? 4u : 6u);
-  constexpr int KSTEPS = KC / 16;
 
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   // SWIZZLE_128B operands need 1024-byte aligned stage bases: align by hand, do not trust the attribute
@@ -464,7 +434,6 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
   uint64_t* tempty_bar = tfull_bar + 4;
   uint64_t* resb_bar = tempty_bar + 4;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(resb_bar + 2);
-  volatile int* prod_iter = reinterpret_cast<volatile int*>(tmem_slot + 1);  // producer's tile-loop counter
   float* s_stat = reinterpret_cast<float*>(tmem_slot + 4);  // [2][256]
   float* s_const = s_stat + 2 * 256;                        // [4][512] per-channel epilogue constants
   float* s_ds = s_const + 4 * 512;                          // [2][256] Dropout2d scales of the image each epilogue group works on
@@ -481,13 +450,12 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < 4; ++i) prefetch_tmap(&maps.a[i]);
     prefetch_tmap(&maps.b);
-    for (int i = 0; i < p.nstages; ++i) { mbar_init(&full_bar[i], PROD ? 64 : 1); mbar_init(&empty_bar[i], 1); }
+    for (int i = 0; i < p.nstages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
     // the two epilogue warp groups alternate tiles (4 arrivals per accumulator and CTA); only with several N tiles per CTA and
     // fused statistics do all eight warps share every tile (they then flush the statistics together)
     const bool alt0 = !(p.n_ntiles > 1 && ((MODE == 0 ? p.stats : p.bn_sums) != nullptr));
     for (int i = 0; i < p.nacc; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], (alt0 ? 4 : 8) * (CTA2 ? 2 : 1)); }
     mbar_init(&resb_bar[0], 1);
-    *prod_iter = 0;
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     if (p.b_resident && !CTA2) {
@@ -498,7 +466,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
           tma_load_3d(resb + (size_t)(tap * p.kchunks + kc) * p.b_tap_bytes, &maps.b, &resb_bar[0], kc * KC, 0, tap);
     }
   }
-  if (warp == PW) { if (CTA2) tmem_alloc2(tmem_slot, (uint32_t)p.tmem_cols); else tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols); }
+  if (warp == 1) { if (CTA2) tmem_alloc2(tmem_slot, (uint32_t)p.tmem_cols); else tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols); }
   // epilogue constants and statistics accumulators (the N tile is fixed per CTA only when n_ntiles == 1,
   // so constants are indexed by absolute channel and reloaded per tile below when needed)
   for (int i = threadIdx.x; i < 2 * 256; i += NTHREADS) s_stat[i] = 0.f;
@@ -532,124 +500,58 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
   }
 
 
-  if (warp < PW) {
-    if (PROD == 0) {
-      // ===================================================================== TMA producer
-      // the whole warp runs the loop (uniform control flow), one elected lane issues
-      {
-        const uint32_t leader = elect_one();
-        int stage = 0;
-        uint32_t phase = 0;
-        int iter = 0;
-        const int nstages = p.nstages, kchunks = p.kchunks, b_resident = p.b_resident;
-        for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-          if (lane == 0) *prod_iter = iter;
-          ++iter;
-          int ci, nt, tw, th, n;
-          decode_tile(p, tile, ci, nt, tw, th, n);
-          const TcClass& C = p.cls[ci];
-          const int cg0 = C.g0, cg1 = C.g0 + C.ng, gpi = C.gpi;
-          for (int kc = 0; kc < kchunks; ++kc) {
-            for (int g0 = cg0; g0 < cg1; g0 += gpi) {
-              mbar_wait(&empty_bar[stage], phase ^ 1u, p.error_flag, 1);
-              unsigned char* sa = smem + (size_t)stage * stage_bytes;
-              unsigned char* sb = sa + p.a_stage_bytes;
-              if (p.debug & 8) {
-                mbar_arrive_p(&full_bar[stage], leader);
-                if (++stage == nstages) { stage = 0; phase ^= 1u; }
-                continue;
-              }
-              uint32_t bytes = 0;
-              for (int gi = g0; gi < g0 + gpi; ++gi)
-                bytes += (uint32_t)(p.g[gi].rows * p.g[gi].cols * (int)ROW_BYTES + (b_resident ? 0 : p.g[gi].ntaps * p.b_tap_bytes));
-              if (CTA2) {
-                // both CTAs load their own A boxes; the bytes of both are expected on the leader's barrier
-                if (cta_rank == 0) mbar_expect_tx_p(&full_bar[stage], 2u * bytes, leader);
-                const uint32_t lbar = map_to_cta(smem_u32(&full_bar[stage]), 0u);
-                for (int gi = g0; gi < g0 + gpi; ++gi) {
-                  const TcGroup& g = p.g[gi];
-                  tma2_load_4d_p(sa + (size_t)(gi - g0) * p.a_box_bytes, &maps.a[g.map], lbar, kc * KC,
-                                 tw * p.TW + g.dw, th * p.TH + g.dh, n, leader);
-                }
-                if (++stage == nstages) { stage = 0; phase ^= 1u; }
-                continue;
-              }
-              mbar_expect_tx_p(&full_bar[stage], bytes, leader);
-              for (int gi = g0; gi < g0 + gpi; ++gi) {
-                const TcGroup& g = p.g[gi];
-                tma_load_4d_p(sa + (size_t)(gi - g0) * p.a_box_bytes, &maps.a[g.map], &full_bar[stage], kc * KC,
-                              tw * p.TW + g.dw, th * p.TH + g.dh, n, leader);
-                if (!b_resident)
-                  for (int tp = 0; tp < g.ntaps; ++tp)
-                    tma_load_3d_p(sb + (size_t)((gi - g0) * p.bt_stride + tp) * p.b_tap_bytes, &maps.b, &full_bar[stage],
-                                  kc * KC, nt * BN, g.widx[tp], leader);
-              }
-              if (++stage == nstages) { stage = 0; phase ^= 1u; }
-            }
+  if (warp == 0) {
+    // ===================================================================== TMA producer
+    // the whole warp runs the loop (uniform control flow), one elected lane issues
+    const uint32_t leader = elect_one();
+    int stage = 0;
+    uint32_t phase = 0;
+    const int nstages = p.nstages, kchunks = p.kchunks, b_resident = p.b_resident;
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+      int ci, nt, tw, th, n;
+      decode_tile(p, tile, ci, nt, tw, th, n);
+      const TcClass& C = p.cls[ci];
+      const int cg0 = C.g0, cg1 = C.g0 + C.ng, gpi = C.gpi;
+      for (int kc = 0; kc < kchunks; ++kc) {
+        for (int g0 = cg0; g0 < cg1; g0 += gpi) {
+          mbar_wait(&empty_bar[stage], phase ^ 1u, p.error_flag, 1);
+          unsigned char* sa = smem + (size_t)stage * stage_bytes;
+          unsigned char* sb = sa + p.a_stage_bytes;
+          if (p.debug & 8) {
+            mbar_arrive_p(&full_bar[stage], leader);
+            if (++stage == nstages) { stage = 0; phase ^= 1u; }
+            continue;
           }
-        }
-      }
-    } else {
-      // ===================================================================== cp.async producer (64 threads)
-      const int ptid = threadIdx.x;  // 0..63
-      int stage = 0;
-      uint32_t phase = 0;
-      int issued = 0;
-      int hist[LAG] = {0, 0};        // stages of the last LAG committed groups (oldest first)
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-        int t = tile;
-        const TcClass& C = p.cls[tile_class(p, t)]; t /= p.ncls;
-        t /= p.n_ntiles;
-        const int tw = t % p.tiles_w; t /= p.tiles_w;
-        const int th = t % p.tiles_h;
-        const int n = t / p.tiles_h;
-        for (int kc = 0; kc < p.kchunks; ++kc) {
-          for (int g0 = C.g0; g0 < C.g0 + C.ng; g0 += C.gpi) {
-            mbar_wait(&empty_bar[stage], phase ^ 1u, p.error_flag, 1);
-            for (int gi = g0; gi < g0 + C.gpi; ++gi) {
+          uint32_t bytes = 0;
+          for (int gi = g0; gi < g0 + gpi; ++gi)
+            bytes += (uint32_t)(p.g[gi].rows * p.g[gi].cols * (int)ROW_BYTES + (b_resident ? 0 : p.g[gi].ntaps * p.b_tap_bytes));
+          if (CTA2) {
+            // both CTAs load their own A boxes; the bytes of both are expected on the leader's barrier
+            if (cta_rank == 0) mbar_expect_tx_p(&full_bar[stage], 2u * bytes, leader);
+            const uint32_t lbar = map_to_cta(smem_u32(&full_bar[stage]), 0u);
+            for (int gi = g0; gi < g0 + gpi; ++gi) {
               const TcGroup& g = p.g[gi];
-              const TcSrc& src = p.src[g.map];
-              const uint32_t sa = smem_u32(smem + (size_t)stage * stage_bytes) + (uint32_t)((gi - g0) * p.a_box_bytes);
-              const bf16* nbase = src.base + (long long)n * src.sn + kc * KC;
-              const int nchunk = g.rows * TC_TW * CPR;
-              for (int i = ptid; i < nchunk; i += 64) {
-                const int prow = i / CPR, j = i % CPR;
-                const int h = th * TC_TH + g.dh + prow / TC_TW, w = tw * TC_TW + g.dw + prow % TC_TW;
-                const bool ok = h >= 0 && h < src.Hd && w >= 0 && w < src.Wd;
-                const bf16* gp = ok ? nbase + (long long)h * src.sh + (long long)w * src.sw + j * 8 : src.base;
-                const uint32_t off = (uint32_t)prow * ROW_BYTES;
-                const uint32_t dst = sa + off + ((uint32_t)(j ^ (int)((off >> 7) & (CPR - 1))) << 4);
-                const int nbytes = ok ? 16 : 0;   // src-size 0 = zero fill (the conv padding)
-                asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(gp), "r"(nbytes) : "memory");
-              }
+              tma2_load_4d_p(sa + (size_t)(gi - g0) * p.a_box_bytes, &maps.a[g.map], lbar, kc * KC,
+                             tw * p.TW + g.dw, th * p.TH + g.dh, n, leader);
             }
-            asm volatile("cp.async.commit_group;" ::: "memory");
-            ++issued;
-            if (issued > LAG) {
-              // the group committed LAG items ago has landed: publish it to the async proxy, release the stage
-              asm volatile("cp.async.wait_group 2;" ::: "memory");
-              asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-              mbar_arrive(&full_bar[hist[0]]);
-            }
-            hist[0] = hist[1];
-            hist[1] = stage;
-            if (++stage == p.nstages) { stage = 0; phase ^= 1u; }
+            if (++stage == nstages) { stage = 0; phase ^= 1u; }
+            continue;
           }
+          mbar_expect_tx_p(&full_bar[stage], bytes, leader);
+          for (int gi = g0; gi < g0 + gpi; ++gi) {
+            const TcGroup& g = p.g[gi];
+            tma_load_4d_p(sa + (size_t)(gi - g0) * p.a_box_bytes, &maps.a[g.map], &full_bar[stage], kc * KC,
+                          tw * p.TW + g.dw, th * p.TH + g.dh, n, leader);
+            if (!b_resident)
+              for (int tp = 0; tp < g.ntaps; ++tp)
+                tma_load_3d_p(sb + (size_t)((gi - g0) * p.bt_stride + tp) * p.b_tap_bytes, &maps.b, &full_bar[stage],
+                              kc * KC, nt * BN, g.widx[tp], leader);
+          }
+          if (++stage == nstages) { stage = 0; phase ^= 1u; }
         }
-      }
-      // drain
-      if (issued >= 2) {
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_arrive(&full_bar[hist[0]]);
-      }
-      if (issued >= 1) {
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_arrive(&full_bar[hist[1]]);
       }
     }
-  } else if (warp == PW) {
+  } else if (warp == 1) {
     // ===================================================================== MMA issuer
     // instruction descriptor: D=f32 [4,6)=1, A=bf16 [7,10)=1, B=bf16 [10,13)=1, K-major A/B, N>>3 [17,23), M>>4 [24,29)
     const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | (((CTA2 ? 256u : 128u) >> 4) << 24);
@@ -689,42 +591,16 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
           // whole warp, uniform control flow; the elected lane issues (predicate inside the asm)
           const uint32_t ast = desc0_lo + (uint32_t)stage * stage_units;
           const uint32_t bst = b_resident ? bres0_lo + (uint32_t)kc * tap_units : ast + a_units;
-          const int e1 = p.ebeg[g0 + gpi];
-          if (p.flat_on) {
-            // measured on the W-folded 16-channel layer: the mask walk below cost ~80 cycles per 48-cycle MMA
-            const int L = p.flat_perkc ? kc : 0;
-            const int i0 = p.flat_rng[L][g0], i1 = (p.debug & 2) ? i0 : p.flat_rng[L][g0 + gpi];
-            const uint32_t a_hi = p.tab_hi[p.ebeg[g0]];
+          const int L = p.flat_perkc ? kc : 0;
+          for (int gi = g0; gi < g0 + gpi; ++gi) {
+            const uint32_t a_hi = p.a_hi[gi];
+            const int i0 = p.flat_rng[L][gi], i1 = (p.debug & 2) ? i0 : p.flat_rng[L][gi + 1];
 #pragma unroll 4
             for (int i = i0; i < i1; ++i) {
               const uint32_t ab = p.flat_ab[i];
               if (CTA2) umma2_bf16_lh2_p(d_tmem, ast + (ab & 0xFFFFu), a_hi, bst + (ab >> 16), desc_hi, idesc, started, leader);
               else umma_bf16_lh2_p(d_tmem, ast + (ab & 0xFFFFu), a_hi, bst + (ab >> 16), desc_hi, idesc, started, leader);
               started = 1u;
-            }
-          } else
-          for (int e = p.ebeg[g0]; e < e1; ++e) {
-            // descriptors advance by 32 bytes (2 units of 16 B) per K step
-            const uint32_t ad0 = ast + p.tab_a[e], bd0 = bst + p.tab_b[e], a_hi = p.tab_hi[e];
-            // (all ones = no structural zeros: also for K > 512 channels, whose K steps do not fit the 32-bit mask)
-            const unsigned kmr = p.tab_km[e];
-            const unsigned km = kmr == 0xFFFFFFFFu ? ((1u << KSTEPS) - 1u) : ((kmr >> (kc * KSTEPS)) & ((1u << KSTEPS) - 1u));
-            if (p.debug & 2) continue;
-            if (km == (1u << KSTEPS) - 1u) {
-#pragma unroll
-              for (int k = 0; k < KSTEPS; ++k) {
-                if (CTA2) umma2_bf16_lh2_p(d_tmem, ad0 + 2u * k, a_hi, bd0 + 2u * k, desc_hi, idesc, started, leader);
-                else umma_bf16_lh2_p(d_tmem, ad0 + 2u * k, a_hi, bd0 + 2u * k, desc_hi, idesc, started, leader);
-                started = 1u;
-              }
-            } else {
-#pragma unroll
-              for (int k = 0; k < KSTEPS; ++k) {
-                if (!((km >> k) & 1u)) continue;   // structurally zero weights (W-folded convolution)
-                if (CTA2) umma2_bf16_lh2_p(d_tmem, ad0 + 2u * k, a_hi, bd0 + 2u * k, desc_hi, idesc, started, leader);
-                else umma_bf16_lh2_p(d_tmem, ad0 + 2u * k, a_hi, bd0 + 2u * k, desc_hi, idesc, started, leader);
-                started = 1u;
-              }
             }
           }
           if (prof) t2 = clock64();
@@ -749,45 +625,13 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       d[0] = c_tempty; d[1] = c_full; d[2] = c_issue; d[3] = c_commit; d[4] = c_rest; d[5] = c_items;
       d[6] = (unsigned long long)(t_loop0 - t_kernel0); d[7] = (unsigned long long)(clock64() - t_kernel0);   // loop entry, loop exit
     }
-  } else if (warp == PW + 9) {
-    // ===================================================================== L2 prefetch warp
-    // Pulls the A-operand halo boxes of the tile TC_PF_AHEAD iterations ahead from HBM into L2 with plain
-    // prefetch instructions, so that the TMA loads of the (shared-memory-limited, 2-3 stage) pipeline see L2
-    // latency instead of HBM latency.  Costs no shared memory and no TMA issue slots.
-    if (PROD == 0 && p.pf_ahead > 0) {
-      int iter = 0;
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++iter) {
-        while (iter > *prod_iter + p.pf_ahead) __nanosleep(256);
-        int t = tile;
-        const TcClass& C = p.cls[tile_class(p, t)]; t /= p.ncls;
-        t /= p.n_ntiles;
-        const int tw = t % p.tiles_w; t /= p.tiles_w;
-        const int th = t % p.tiles_h;
-        const int n = t / p.tiles_h;
-        for (int gi = C.g0; gi < C.g0 + C.ng; ++gi) {
-          const TcGroup& g = p.g[gi];
-          const TcSrc& src = p.src[g.map];
-          const int npx = g.rows * TC_TW;
-          // one 128-byte line per (pixel, 64-channel slice); contiguous pixels share lines when C < 64
-          const int lines_per_px = (p.kchunks * KC * 2 + 127) / 128;
-          for (int i = lane; i < npx * lines_per_px; i += 32) {
-            const int px = i / lines_per_px, ln = i % lines_per_px;
-            const int h = th * TC_TH + g.dh + px / TC_TW, w = tw * TC_TW + g.dw + px % TC_TW;
-            if (h >= 0 && h < src.Hd && w >= 0 && w < src.Wd) {
-              const bf16* a = src.base + (long long)n * src.sn + (long long)h * src.sh + (long long)w * src.sw + ln * 64;
-              asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
-            }
-          }
-        }
-      }
-    }
-  } else {
+  } else if (warp < 10) {
     // ===================================================================== epilogue (8 warps)
     // warp w may only touch TMEM lanes [32*(w&3), +32).  The eight warps form two groups of four (one warp per lane
     // quarter); the groups ALTERNATE TILES, so the fixed per-tile work (decode, barrier waits, hand-back) is paid by four warps
     // instead of eight - the epilogue, not the tensor pipe, bounds most layers.
     const int q = warp & 3;
-    const int half = (warp - (PW + 1)) >> 2;
+    const int half = (warp - 2) >> 2;
     const int m = q * 32 + lane;       // row of the tile = pixel
     const int hl = m >> p.tw_shift, wl = m & (p.TW - 1);
     int acc_it = 0;
@@ -813,7 +657,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
     const int e_TH = p.TH, e_TW = p.TW, e_osh = p.osh, e_osw = p.osw, e_total = p.total_tiles, e_nacc = p.nacc;
     const bool alt = !(e_nnt > 1 && ((MODE == 0 ? (const void*)e_stats : (const void*)e_bn_sums) != nullptr));
     const bool ds_smem = e_dropscale != nullptr && alt && e_OC <= 256;   // else the scales are read through L1 per chunk
-    const bool eprof = (p.debug & 16) != 0 && warp == PW + 1;
+    const bool eprof = (p.debug & 16) != 0 && warp == 2;
     long long ec_tfull = 0, ec_ld = 0, ec_pre = 0, ec_math = 0, ec_store = 0, ec_rest = 0, ec_tiles = 0, eprev = clock64();
     const bool io_f32 = p.io_f32 != 0;
     const bool use_mask = MODE == 1 && p.actmask_in && e_act == YG_ACT_LRELU && !has_bn && (BN % 32) == 0 && (e_OC % 32) == 0 && !io_f32;
@@ -844,7 +688,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       const float* dsrow = e_dropscale ? e_dropscale + (long long)(n < p.N ? n : p.N - 1) * e_OCr : nullptr;
       if (ds_smem && n != ds_n) {
         // stage the row of this image in this group's half of the shared buffer, already expanded to folded channels
-        const int tg = (int)threadIdx.x - (PW + 1) * 32 - half * 128;
+        const int tg = (int)threadIdx.x - 64 - half * 128;
         if (half == 0) asm volatile("bar.sync 1, 128;" ::: "memory"); else asm volatile("bar.sync 2, 128;" ::: "memory");
         for (int i = tg; i < e_OC; i += 128) s_ds[half * 256 + i] = dsrow[i - fdiv(i, p.fd_ocr) * e_OCr];
         if (half == 0) asm volatile("bar.sync 1, 128;" ::: "memory"); else asm volatile("bar.sync 2, 128;" ::: "memory");
@@ -1455,7 +1299,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       if (e_nnt > 1 && (e_stats || e_bn_sums)) {
         asm volatile("bar.sync 1, 256;" ::: "memory");
         double* dst = MODE == 0 ? e_stats : e_bn_sums;
-        for (int i = threadIdx.x - (PW + 1) * 32; i < BN; i += 256) {
+        for (int i = threadIdx.x - 64; i < BN; i += 256) {
           const float a1 = s_stat[i], a2 = s_stat[256 + i];
           if (a1 != 0.f || a2 != 0.f) {
             atomicAdd(dst + (nt * BN + i) % e_OCr, (double)a1);
@@ -1488,7 +1332,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
     }
   }
   if (CTA2) cluster_sync_all();   // neither CTA leaves (or frees TMEM) while its peer may still signal it
-  if (warp == PW) { if (CTA2) tmem_dealloc2(tmem_base, (uint32_t)p.tmem_cols); else tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols); }
+  if (warp == 1) { if (CTA2) tmem_dealloc2(tmem_base, (uint32_t)p.tmem_cols); else tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols); }
 }
 
 // ------------------------------------------------------------------------------------------ weights
@@ -1533,19 +1377,21 @@ __global__ void pack_weights_s2fold_kernel(const float* __restrict__ w, bf16* __
 }
 
 // ------------------------------------------------------------------------------------------ host
-static int g_tc_options = 25 + 8192 + 16384;  // bit 0: resident weights, bit 1: cp.async producer, bit 2: L2 prefetch warp, bit 3: W-fold,
-                               // bit 4: column-pair fold for stride-2 dgrad
+// yg_set_tc_options (include/yogo_b200.h): bits 7-11 = profiling knobs of the engine (TcParams::debug), bit 21 = fp32 tensors as
+// split-bf16 convolutions (api.cu)
+constexpr int TC_OPTION_BITS = (31 << 7) | (1 << 21);
+static int g_tc_options = 0;
 // W-fold factor for stride-1 convolutions with few channels (see pack_weights_kernel): fold while the folded
 // input channel count stays <= 64 and everything remains a legal UMMA shape.
 static int fold_factor(int Cin, int Cout, int W, int stride) {
-  if (stride != 1 || !(g_tc_options & 8)) return 1;
+  if (stride != 1) return 1;
   for (int g = 4; g >= 2; g >>= 1)
     if (W % g == 0 && g * Cin <= 64 && g * Cout <= 256 && (g * Cin) % 16 == 0 && (g * Cout) % 16 == 0) return g;
   return 1;
 }
 // Stride-2 dgrad with few input channels: fold output column pairs (2 classes x N = 2*Cin instead of 4 x N = Cin).
 static bool s2fold_dgrad(int Cin, int W, int stride) {
-  return stride == 2 && (g_tc_options & 16) && W % 2 == 0 && 2 * Cin <= 64 && (2 * Cin) % 16 == 0;
+  return stride == 2 && W % 2 == 0 && 2 * Cin <= 64 && (2 * Cin) % 16 == 0;
 }
 // bit kk set <=> K step kk (16 folded channels) of folded tap column sp touches a sub-pixel with non-zero weights.
 // kdim_is_input: K runs over (pi, ci) [fprop / wgrad-B], otherwise over (q, co) [dgrad].
@@ -1648,8 +1494,6 @@ struct TwParams {
   int ngroups;                 // groups per filter column
   int ncols;                   // filter columns = work-unit columns (3 for 3x3, 1 for 1x1)
   TwGroup g[3][2];
-  TcSrc asrc;        // dz as seen by the cp.async producer
-  TcSrc bsrc[4];     // x (or its parity sub-grids)
   float* partial;
   int share_a;          // stride 2 (two parity groups per tile): ONE stage per tile holds the dz tile once and both x boxes
                         // (the dz tile used to be fetched from L2 once per group - the kernel is L2-bandwidth bound)
@@ -1673,12 +1517,10 @@ __device__ __forceinline__ uint64_t umma_desc_mn(uint32_t saddr, uint32_t lbo_by
   return d;
 }
 
-template <int KB, int KA, int PROD>
-__global__ void __launch_bounds__((PROD ? 2 : 1) * 32 + 160, 1)
+template <int KB, int KA>
+__global__ void __launch_bounds__(192, 1)
 wgrad_tc_kernel(const __grid_constant__ TwMaps maps, const __grid_constant__ TwParams p) {
-  constexpr int PW = PROD ? 2 : 1;                        // producer warps; MMA warp = PW; epilogue PW+1..PW+4
-  constexpr int NTHREADS = PW * 32 + 160;
-  constexpr int CPRA = KA / 8, CPRB = KB / 8;             // 16-byte chunks per operand row
+  constexpr int NTHREADS = 192;                           // warp 0 producer, warp 1 MMA, warps 2-5 epilogue
   constexpr uint32_t ROWB = KB * 2;                       // bytes per pixel row of a B block
   constexpr uint32_t LAYOUT_B = KB == 64 ? 2u : (KB == 32 ? 4u : 6u);
   constexpr uint32_t ROWA = KA * 2;                       // A blocks are KA couts wide (64: SWIZZLE_128B, 32: 64B)
@@ -1702,7 +1544,7 @@ wgrad_tc_kernel(const __grid_constant__ TwMaps maps, const __grid_constant__ TwP
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&maps.a);
     for (int i = 0; i < 4; ++i) prefetch_tmap(&maps.b[i]);
-    for (int i = 0; i < p.nstages; ++i) { mbar_init(&full_bar[i], PROD ? 64 : 1); mbar_init(&empty_bar[i], 1); }
+    for (int i = 0; i < p.nstages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
     mbar_init(&done_bar[0], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -1717,7 +1559,7 @@ wgrad_tc_kernel(const __grid_constant__ TwMaps maps, const __grid_constant__ TwP
   if (p.do_bias)
     for (int i = threadIdx.x; i < 512; i += NTHREADS) reinterpret_cast<uint32_t*>(ones)[i] = 0x3F803F80u;
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  if (warp == PW) tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
+  if (warp == 1) tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -1726,116 +1568,41 @@ wgrad_tc_kernel(const __grid_constant__ TwMaps maps, const __grid_constant__ TwP
   const bool do_bias = p.do_bias != 0;
   const int bias_period = p.ncols * p.n_ntiles, bias_phase = sg + p.ncols * nt;
 
-  if (warp < PW) {
-    if (PROD == 0) {
-      {
-        // whole warp, uniform control flow; the elected lane issues (see elect_one)
-        const uint32_t leader = elect_one();
-        int stage = 0;
-        uint32_t phase = 0;
-        const int nstages = p.nstages, ngroups = p.ngroups, nbblocks = p.nbblocks;
-        for (int tile = slice; tile < p.total_tiles; tile += p.nslices) {
-          int t = tile;
-          const int tw = t % p.tiles_w; t /= p.tiles_w;
-          const int th = t % p.tiles_h;
-          const int n = t / p.tiles_h;
-          const bool share = p.share_a != 0;
-          for (int gi = 0; gi < ngroups; ++gi) {
-            const TwGroup& g = p.g[sg][gi];
-            unsigned char* sa = smem + (size_t)stage * p.stage_bytes;
-            unsigned char* sb = sa + MBLOCKS * p.a_block_bytes + (share ? (size_t)gi * nbblocks * p.b_block_bytes : 0);
-            if (!share || gi == 0) {
-              mbar_wait(&empty_bar[stage], phase ^ 1u, p.error_flag, 11);
-              int brows = g.rows;
-              if (share) for (int g2 = 1; g2 < ngroups; ++g2) brows += p.g[sg][g2].rows;
-              const uint32_t bytes = (uint32_t)(a_blocks * p.a_block_bytes + nbblocks * brows * TC_TW * (int)ROWB);
-              mbar_expect_tx_p(&full_bar[stage], bytes, leader);
-              for (int ab = 0; ab < a_blocks; ++ab)
-                tma_load_4d_p(sa + (size_t)ab * p.a_block_bytes, &maps.a, &full_bar[stage], mt * 128 + ab * KA, tw * TC_TW,
-                              th * TC_TH, n, leader);
-            }
-            for (int bb = 0; bb < nbblocks; ++bb)
-              tma_load_4d_p(sb + (size_t)bb * p.b_block_bytes, &maps.b[g.map], &full_bar[stage], nt * BNW + bb * KB,
-                            tw * TC_TW + g.dw, th * TC_TH + g.dh, n, leader);
-            if (!share || gi == ngroups - 1) {
-              if (++stage == nstages) { stage = 0; phase ^= 1u; }
-            }
-          }
-        }
-      }
-    } else {
-      // cp.async producer (64 threads): both operands written in their swizzled MN-major layouts by hand
-      const int ptid = threadIdx.x;
-      int stage = 0;
-      uint32_t phase = 0;
-      int issued = 0;
-      int hist[2] = {0, 0};
-      for (int tile = slice; tile < p.total_tiles; tile += p.nslices) {
-        int t = tile;
-        const int tw = t % p.tiles_w; t /= p.tiles_w;
-        const int th = t % p.tiles_h;
-        const int n = t / p.tiles_h;
-        for (int gi = 0; gi < p.ngroups; ++gi) {
-          const TwGroup& g = p.g[sg][gi];
-          const TcSrc& src = p.bsrc[g.map];
+  if (warp == 0) {
+    // whole warp, uniform control flow; the elected lane issues (see elect_one)
+    const uint32_t leader = elect_one();
+    int stage = 0;
+    uint32_t phase = 0;
+    const int nstages = p.nstages, ngroups = p.ngroups, nbblocks = p.nbblocks;
+    for (int tile = slice; tile < p.total_tiles; tile += p.nslices) {
+      int t = tile;
+      const int tw = t % p.tiles_w; t /= p.tiles_w;
+      const int th = t % p.tiles_h;
+      const int n = t / p.tiles_h;
+      const bool share = p.share_a != 0;
+      for (int gi = 0; gi < ngroups; ++gi) {
+        const TwGroup& g = p.g[sg][gi];
+        unsigned char* sa = smem + (size_t)stage * p.stage_bytes;
+        unsigned char* sb = sa + MBLOCKS * p.a_block_bytes + (share ? (size_t)gi * nbblocks * p.b_block_bytes : 0);
+        if (!share || gi == 0) {
           mbar_wait(&empty_bar[stage], phase ^ 1u, p.error_flag, 11);
-          const uint32_t sa = smem_u32(smem + (size_t)stage * p.stage_bytes);
-          const uint32_t sb = sa + (uint32_t)MBLOCKS * (uint32_t)p.a_block_bytes;
-          // A = dz tile: a_blocks x (128 pixel rows x KA couts)
-          const int na = a_blocks * 128 * CPRA;
-          for (int i = ptid; i < na; i += 64) {
-            const int j = i % CPRA, prow = (i / CPRA) % 128, ab = i / (CPRA * 128);
-            const int h = th * TC_TH + prow / TC_TW, w = tw * TC_TW + prow % TC_TW;
-            const bool ok = h < p.asrc.Hd && w < p.asrc.Wd;
-            const bf16* gp = ok ? p.asrc.base + (long long)n * p.asrc.sn + (long long)h * p.asrc.sh +
-                                      (long long)w * p.asrc.sw + mt * 128 + ab * KA + j * 8
-                                : p.asrc.base;
-            const uint32_t off = (uint32_t)prow * ROWA;
-            const uint32_t dst = sa + (uint32_t)ab * (uint32_t)p.a_block_bytes + off +
-                                 ((uint32_t)(j ^ (int)((off >> 7) & (CPRA - 1))) << 4);
-            const int nbytes = ok ? 16 : 0;
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(gp), "r"(nbytes) : "memory");
-          }
-          // B = x halo tile: nbblocks x (rows*16 pixel rows x KB cins)
-          const int rowsB = g.rows * TC_TW;
-          const int nb = p.nbblocks * rowsB * CPRB;
-          for (int i = ptid; i < nb; i += 64) {
-            const int j = i % CPRB, prow = (i / CPRB) % rowsB, bb = i / (CPRB * rowsB);
-            const int h = th * TC_TH + g.dh + prow / TC_TW, w = tw * TC_TW + g.dw + prow % TC_TW;
-            const bool ok = h >= 0 && h < src.Hd && w >= 0 && w < src.Wd;
-            const bf16* gp = ok ? src.base + (long long)n * src.sn + (long long)h * src.sh + (long long)w * src.sw +
-                                      nt * BNW + bb * KB + j * 8
-                                : src.base;
-            const uint32_t off = (uint32_t)prow * ROWB;
-            const uint32_t dst = sb + (uint32_t)bb * (uint32_t)p.b_block_bytes + off +
-                                 ((uint32_t)(j ^ (int)((off >> 7) & (CPRB - 1))) << 4);
-            const int nbytes = ok ? 16 : 0;
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(gp), "r"(nbytes) : "memory");
-          }
-          asm volatile("cp.async.commit_group;" ::: "memory");
-          ++issued;
-          if (issued > 2) {
-            asm volatile("cp.async.wait_group 2;" ::: "memory");
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            mbar_arrive(&full_bar[hist[0]]);
-          }
-          hist[0] = hist[1];
-          hist[1] = stage;
-          if (++stage == p.nstages) { stage = 0; phase ^= 1u; }
+          int brows = g.rows;
+          if (share) for (int g2 = 1; g2 < ngroups; ++g2) brows += p.g[sg][g2].rows;
+          const uint32_t bytes = (uint32_t)(a_blocks * p.a_block_bytes + nbblocks * brows * TC_TW * (int)ROWB);
+          mbar_expect_tx_p(&full_bar[stage], bytes, leader);
+          for (int ab = 0; ab < a_blocks; ++ab)
+            tma_load_4d_p(sa + (size_t)ab * p.a_block_bytes, &maps.a, &full_bar[stage], mt * 128 + ab * KA, tw * TC_TW,
+                          th * TC_TH, n, leader);
         }
-      }
-      if (issued >= 2) {
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_arrive(&full_bar[hist[0]]);
-      }
-      if (issued >= 1) {
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_arrive(&full_bar[hist[1]]);
+        for (int bb = 0; bb < nbblocks; ++bb)
+          tma_load_4d_p(sb + (size_t)bb * p.b_block_bytes, &maps.b[g.map], &full_bar[stage], nt * BNW + bb * KB,
+                        tw * TC_TW + g.dw, th * TC_TH + g.dh, n, leader);
+        if (!share || gi == ngroups - 1) {
+          if (++stage == nstages) { stage = 0; phase ^= 1u; }
+        }
       }
     }
-  } else if (warp == PW) {
+  } else if (warp == 1) {
     // D=f32, A=B=bf16, both MN-major (bits 15,16), N = BNW, M = 128
     const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
                            ((uint32_t)(BNW >> 3) << 17) | ((128u >> 4) << 24);
@@ -1967,7 +1734,7 @@ wgrad_tc_kernel(const __grid_constant__ TwMaps maps, const __grid_constant__ TwP
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  if (warp == PW) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
+  if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
 }
 
 // Sums the per-CTA partials in a fixed order.  The kernel ran on (possibly W-folded) dimensions Coutf = g*Cout,
@@ -2104,10 +1871,10 @@ int conv_wgrad_tc(const void* x, const void* dz, float* dw, float* dbias, int N,
   p.ncols = 3;
   for (int r = 0; r < 3; ++r) p.row_slot[r] = r;
   // stride 2 with one B block per tap: filter rows 0 and 2 take the adjacent slots 0 and 1 so that one MMA covers both
-  if (stride == 2 && p.BNW == kb && !(g_tc_options & (1 << 19))) { p.merge2 = 1; p.row_slot[0] = 0; p.row_slot[2] = 1; p.row_slot[1] = 2; }
+  if (stride == 2 && p.BNW == kb) { p.merge2 = 1; p.row_slot[0] = 0; p.row_slot[2] = 1; p.row_slot[1] = 2; }
   // base L4 wgrad 0.50 -> 0.38 ms (1235 TFLOP/s): three N = 64 MMAs (48 cycles each, bound by the shared-memory operand fetch)
-  // become one N = 192 MMA (96 cycles of math, 80 of fetch); results are bit-identical.  Option bit 19 turns it off.
-  p.merge3 = (stride == 1 && kb == 64 && p.BNW == 64 && !(g_tc_options & (1 << 19))) ? 1 : 0;
+  // become one N = 192 MMA (96 cycles of math, 80 of fetch); results are bit-identical.
+  p.merge3 = (stride == 1 && kb == 64 && p.BNW == 64) ? 1 : 0;
   p.N = N; p.Cin = Cin; p.Cout = Cout;
   p.tiles_h = cdiv(Ho, TC_TH); p.tiles_w = cdiv(Wo, TC_TW);
   p.total_tiles = N * p.tiles_h * p.tiles_w;
@@ -2116,11 +1883,10 @@ int conv_wgrad_tc(const void* x, const void* dz, float* dw, float* dbias, int N,
   p.a_block_bytes = TC_TH * TC_TW * ka * 2;
   p.b_block_bytes = (max_rows * TC_TW * kb * 2 + 1023) & ~1023;
   p.stage_bytes = (128 / ka) * p.a_block_bytes + p.nbblocks * p.b_block_bytes;
-  // stride 2: both parity groups of a tile in one stage, sharing the dz tile (TMA producer only; option bit 20 turns it off)
+  // stride 2: both parity groups of a tile in one stage, sharing the dz tile
   {
     const int shared_stage = (128 / ka) * p.a_block_bytes + 2 * p.nbblocks * p.b_block_bytes;
-    const bool cp_async_prod = kb <= 32 && (g_tc_options & 2);
-    if (stride == 2 && !cp_async_prod && !(g_tc_options & (1 << 20)) && TC_SMEM_BUDGET / shared_stage >= 2) {
+    if (stride == 2 && TC_SMEM_BUDGET / shared_stage >= 2) {
       p.share_a = 1;
       p.stage_bytes = shared_stage;
     }
@@ -2143,7 +1909,6 @@ int conv_wgrad_tc(const void* x, const void* dz, float* dw, float* dbias, int N,
     uint32_t box[4] = {(uint32_t)ka, TC_TW, TC_TH, 1};
     rc = make_map(&maps.a, dz, 4, dims, str, box, ka);
     if (rc) return rc;
-    p.asrc = TcSrc{(const bf16*)dz, Wo, Ho, (long long)Cout, (long long)Wo * Cout, (long long)Ho * Wo * Cout};
   }
   const bf16* xb = (const bf16*)x;
   if (stride == 1) {
@@ -2153,7 +1918,6 @@ int conv_wgrad_tc(const void* x, const void* dz, float* dw, float* dbias, int N,
     rc = make_map(&maps.b[0], xb, 4, dims, str, box, kb);
     if (rc) return rc;
     for (int i = 1; i < 4; ++i) maps.b[i] = maps.b[0];
-    for (int i = 0; i < 4; ++i) p.bsrc[i] = TcSrc{xb, W, H, (long long)Cin, (long long)W * Cin, (long long)H * W * Cin};
     p.ngroups = 1;
     for (int s = 0; s < 3; ++s) {
       TwGroup& g = p.g[s][0];
@@ -2170,8 +1934,6 @@ int conv_wgrad_tc(const void* x, const void* dz, float* dw, float* dbias, int N,
         uint32_t box[4] = {(uint32_t)kb, TC_TW, (uint32_t)(ph ? TC_TH + 1 : TC_TH), 1};
         rc = make_map(&maps.b[ph * 2 + pw], xb + ((long long)ph * W + pw) * Cin, 4, dims, str, box, kb);
         if (rc) return rc;
-        p.bsrc[ph * 2 + pw] = TcSrc{xb + ((long long)ph * W + pw) * Cin, W2, H2, 2LL * Cin, 2LL * W * Cin,
-                                    (long long)H * W * Cin};
       }
     p.ngroups = 2;
     for (int s = 0; s < 3; ++s) {
@@ -2192,20 +1954,15 @@ int conv_wgrad_tc(const void* x, const void* dz, float* dw, float* dbias, int N,
   }
   p.error_flag = g_error_flag;
   const size_t smem = (size_t)nst * p.stage_bytes + 1024 + 1024 + 2048;   // align slack, barriers, ones block
-const int prodw = (kb <= 32 && nst >= 3 && (g_tc_options & 2)) ? 1 : 0;
-#define TW_LAUNCH(KBV, KAV, PRODV)                                                                                       \
+#define TW_LAUNCH(KBV, KAV)                                                                                            \
   do {                                                                                                                   \
-    YG_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel<KBV, KAV, PRODV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    wgrad_tc_kernel<KBV, KAV, PRODV><<<grid, (PRODV ? 2 : 1) * 32 + 160, smem, st>>>(maps, p);                           \
+    YG_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel<KBV, KAV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
+    wgrad_tc_kernel<KBV, KAV><<<grid, 192, smem, st>>>(maps, p);                                                         \
   } while (0)
   if (ka == 64) {
-    if (kb == 64) TW_LAUNCH(64, 64, 0);
-    else if (kb == 32) { if (prodw) TW_LAUNCH(32, 64, 1); else TW_LAUNCH(32, 64, 0); }
-    else { if (prodw) TW_LAUNCH(16, 64, 1); else TW_LAUNCH(16, 64, 0); }
+    if (kb == 64) TW_LAUNCH(64, 64); else if (kb == 32) TW_LAUNCH(32, 64); else TW_LAUNCH(16, 64);
   } else {
-    if (kb == 64) TW_LAUNCH(64, 32, 0);
-    else if (kb == 32) { if (prodw) TW_LAUNCH(32, 32, 1); else TW_LAUNCH(32, 32, 0); }
-    else { if (prodw) TW_LAUNCH(16, 32, 1); else TW_LAUNCH(16, 32, 0); }
+    if (kb == 64) TW_LAUNCH(64, 32); else if (kb == 32) TW_LAUNCH(32, 32); else TW_LAUNCH(16, 32);
   }
 #undef TW_LAUNCH
   YG_LAUNCH_CHECK("wgrad_tc_kernel");
@@ -2260,7 +2017,7 @@ static int launch_engine(TcMaps& maps, TcParams& p, int KCc, int mode, int max_r
     // resident weights: all 9 x kchunks tiles stay in smem if at least 3 A stages still fit
     p.b_resident = 0;
     p.resb_bytes = 0;
-    if ((g_tc_options & 1) && p.n_ntiles == 1 && (TC_SMEM_BUDGET - resb) / p.a_stage_bytes >= 3) {
+    if (p.n_ntiles == 1 && (TC_SMEM_BUDGET - resb) / p.a_stage_bytes >= 3) {
       p.b_resident = 1;
       p.resb_bytes = resb;
     }
@@ -2268,18 +2025,12 @@ static int launch_engine(TcMaps& maps, TcParams& p, int KCc, int mode, int max_r
     if (p.b_resident || TC_SMEM_BUDGET / (p.a_stage_bytes + p.b_stage_bytes) >= 3) break;
   }
   if (two_d && !p.b_resident) { set_error("tcgen05 conv: 2-D halo boxes need resident weights"); return YG_ERR_INVALID; }
-  const int prod = (p.b_resident && KCc <= 32 && (g_tc_options & 2)) ? 1 : 0;
   const int stage_bytes = p.a_stage_bytes + (p.b_resident ? 0 : p.b_stage_bytes);
   int nst = (TC_SMEM_BUDGET - p.resb_bytes) / stage_bytes;
-  if (nst > 16) nst = 16;
   // Four stages at most: deeper A pipelines are not faster anywhere and measurably slower where the producer can run far ahead
   // (same box, ms: L3 dgrad 0.350 with every stage that fits, 0.331 / 0.325 / 0.323 with 6 / 4 / 3; CTA-pair L4 dgrad 0.439 /
-  // 0.439 / 0.428 / 0.429).  Option bits 24-26: 1..6 = cap at 2..7 stages, 7 = no cap.
-  {
-    const int capsel = (g_tc_options >> 24) & 7;
-    const int cap = capsel == 0 ? 4 : (capsel == 7 ? 16 : capsel + 1);
-    if (nst > cap) nst = cap;
-  }
+  // 0.439 / 0.428 / 0.429).
+  if (nst > 4) nst = 4;
   if (nst < 2) {
     set_error("tcgen05 conv: stage of %d bytes does not fit twice in shared memory", stage_bytes);
     return YG_ERR_INVALID;
@@ -2295,63 +2046,54 @@ static int launch_engine(TcMaps& maps, TcParams& p, int KCc, int mode, int max_r
     YG_CUDA(cudaMalloc(&g_error_flag, sizeof(int)));
     YG_CUDA(cudaMemset(g_error_flag, 0, sizeof(int)));
   }
+  // MMA issue list (see TcParams::flat_ab) in issue order: group, tap, 16-wide K step.  The structurally zero K steps of
+  // W-folded layers differ per K chunk, so those layers get one list per chunk.
   {
-    int e = 0;
-    for (int c = 0; c < p.ncls; ++c) {
-      const TcClass& C = p.cls[c];
-      for (int gi = C.g0; gi < C.g0 + C.ng; ++gi) {
-        const TcGroup& g = p.g[gi];
-        const int pos = (gi - C.g0) % C.gpi;   // position of the group inside its pipeline item
-        p.ebeg[gi] = e;
-        for (int tp = 0; tp < g.ntaps; ++tp, ++e) {
-          const uint32_t a_off = (uint32_t)(pos * p.a_box_bytes) +
-                                 (uint32_t)((g.ro[tp] * g.cols + g.co[tp]) * KCc * 2 + p.shift_exp[gi]);
-          const uint32_t b_off = p.b_resident ? (uint32_t)(g.widx[tp] * p.kchunks * p.b_tap_bytes)
-                                              : (uint32_t)((pos * p.bt_stride + tp) * p.b_tap_bytes);
-          p.tab_a[e] = a_off >> 4; p.tab_b[e] = b_off >> 4; p.tab_km[e] = g.kmask[tp];
+    const int ksteps = KCc / 16;
+    const uint32_t layout = KCc == 64 ? 2u : (KCc == 32 ? 4u : 6u);
+    bool masked = false;
+    for (int gi = 0; gi < ngroups_all; ++gi)
+      for (int tp = 0; tp < p.g[gi].ntaps; ++tp) masked = masked || p.g[gi].kmask[tp] != 0xFFFFFFFFu;
+    const int nlists = masked ? p.kchunks : 1;
+    if (nlists > TC_MAX_LISTS || (masked && nlists * ksteps > 32)) {
+      set_error("tcgen05 conv: %d K chunks of %d channels exceed the MMA issue lists", nlists, KCc);
+      return YG_ERR_INVALID;
+    }
+    int n = 0;
+    for (int L = 0; L < nlists; ++L) {
+      for (int c = 0; c < p.ncls; ++c) {
+        const TcClass& C = p.cls[c];
+        for (int gi = C.g0; gi < C.g0 + C.ng; ++gi) {
+          const TcGroup& g = p.g[gi];
+          const int pos = (gi - C.g0) % C.gpi;   // position of the group inside its pipeline item
           // A descriptor high word: the 8-pixel row groups of the M = 128 operand are SBO apart.  Legacy 16-wide
           // boxes: consecutive groups are contiguous (8 pixel rows); 2-D boxes (8-wide tiles): one box row apart.
           const uint32_t sbo = (uint32_t)((two_d ? g.cols : 8) * KCc * 2);
-          const uint32_t layout = KCc == 64 ? 2u : (KCc == 32 ? 4u : 6u);
-          p.tab_hi[e] = ((sbo >> 4) & 0x3FFFu) | (1u << 14) | (layout << 29);
-        }
-        p.ebeg[gi + 1] = e;
-      }
-    }
-  }
-  p.flat_on = 0;
-  if (!(g_tc_options & (1 << 22))) {
-    const int ksteps = KCc / 16;
-    bool masked = false, ok = true;
-    for (int e = 0; e < p.ebeg[ngroups_all]; ++e) masked = masked || p.tab_km[e] != 0xFFFFFFFFu;
-    // every MMA of a pipeline item shares the high A descriptor word of the item's first entry
-    for (int c = 0; c < p.ncls && ok; ++c)
-      for (int g0 = p.cls[c].g0; g0 < p.cls[c].g0 + p.cls[c].ng; g0 += p.cls[c].gpi)
-        for (int e = p.ebeg[g0]; e < p.ebeg[std::min(g0 + p.cls[c].gpi, ngroups_all)]; ++e) ok = ok && p.tab_hi[e] == p.tab_hi[p.ebeg[g0]];
-    const int nlists = masked ? p.kchunks : 1;
-    if (nlists > 2) ok = false;
-    int n = 0;
-    for (int L = 0; L < nlists && ok; ++L) {
-      for (int g = 0; g < ngroups_all && ok; ++g) {
-        p.flat_rng[L][g] = n;
-        for (int e = p.ebeg[g]; e < p.ebeg[g + 1] && ok; ++e) {
-          const unsigned km = p.tab_km[e] == 0xFFFFFFFFu ? (1u << ksteps) - 1u : (p.tab_km[e] >> (L * ksteps)) & ((1u << ksteps) - 1u);
-          for (int k = 0; k < ksteps; ++k) {
-            if (!((km >> k) & 1u)) continue;
-            const uint32_t a = p.tab_a[e] + 2u * k, b = p.tab_b[e] + 2u * k;
-            if (n >= 108 || a > 0xFFFFu || b > 0xFFFFu) { ok = false; break; }
-            p.flat_ab[n++] = a | (b << 16);
+          p.a_hi[gi] = ((sbo >> 4) & 0x3FFFu) | (1u << 14) | (layout << 29);
+          p.flat_rng[L][gi] = n;
+          for (int tp = 0; tp < g.ntaps; ++tp) {
+            const uint32_t a_off = (uint32_t)(pos * p.a_box_bytes + (g.ro[tp] * g.cols + g.co[tp]) * KCc * 2);
+            const uint32_t b_off = p.b_resident ? (uint32_t)(g.widx[tp] * p.kchunks * p.b_tap_bytes)
+                                                : (uint32_t)((pos * p.bt_stride + tp) * p.b_tap_bytes);
+            const unsigned km = g.kmask[tp] == 0xFFFFFFFFu ? (1u << ksteps) - 1u : (g.kmask[tp] >> (L * ksteps)) & ((1u << ksteps) - 1u);
+            for (int k = 0; k < ksteps; ++k) {
+              if (!((km >> k) & 1u)) continue;
+              const uint32_t a = (a_off >> 4) + 2u * k, b = (b_off >> 4) + 2u * k;   // 32 bytes per K step
+              if (n >= TC_MAX_MMAS || a > 0xFFFFu || b > 0xFFFFu) {
+                set_error("tcgen05 conv: MMA issue list overflow (entry %d, A offset %u, B offset %u units)", n, a, b);
+                return YG_ERR_INVALID;
+              }
+              p.flat_ab[n++] = a | (b << 16);
+            }
           }
         }
       }
       p.flat_rng[L][ngroups_all] = n;
     }
     p.flat_perkc = masked ? 1 : 0;
-    p.flat_on = ok ? 1 : 0;
   }
   p.error_flag = g_error_flag;
   p.debug = (g_tc_options >> 7) & 31;
-  p.pf_ahead = (g_tc_options & 4) ? 2 : 0;
   const size_t smem = (size_t)nst * stage_bytes + p.resb_bytes + 1024 /*align*/ + 512 /*barriers*/ +
                       (2 * 256 + 5 * 512 + 16) * sizeof(float) + 64;
   int dev = 0, sms = 148;
@@ -2359,19 +2101,9 @@ static int launch_engine(TcMaps& maps, TcParams& p, int KCc, int mode, int max_r
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   int grid = p.total_tiles < sms ? p.total_tiles : sms;
   if (p.cta2) {
-    if (p.ncls > 1) {
-      // class-per-round order: total = ncls * rounds * grid tiles, spatial indices >= tpc are padding
-      p.tpc = p.total_tiles / p.ncls;
-      const int padded = (p.tpc + 1) & ~1;
-      grid = (padded < sms ? padded : sms) & ~1;
-      p.cls_round = 1;
-      p.grid = grid;
-      p.total_tiles = p.ncls * cdiv(p.tpc, grid) * grid;
-    } else {
-      const int padded = (p.total_tiles + 1) & ~1;
-      grid = (padded < sms ? padded : sms) & ~1;
-    }
-    if (KCc != 64 || mode > 1 || grid < 2 || !p.b_resident || p.n_ntiles != 1) {
+    const int padded = (p.total_tiles + 1) & ~1;
+    grid = (padded < sms ? padded : sms) & ~1;
+    if (KCc != 64 || mode > 1 || grid < 2 || !p.b_resident || p.n_ntiles != 1 || p.ncls != 1) {
       set_error("tcgen05 conv: CTA-pair configuration not supported");
       return YG_ERR_INVALID;
     }
@@ -2380,20 +2112,20 @@ static int launch_engine(TcMaps& maps, TcParams& p, int KCc, int mode, int max_r
   {
     auto magic = [](int d) { return ((1ull << 32) + (unsigned long long)d - 1) / (unsigned long long)d; };
     p.fd_ncls = magic(p.ncls); p.fd_rot = magic(p.cls_rot); p.fd_nnt = magic(p.n_ntiles);
-    p.fd_tw = magic(p.tiles_w); p.fd_th = magic(p.tiles_h); p.fd_grid = magic(grid); p.fd_ocr = magic(p.OCr > 0 ? p.OCr : 1);
-    const long long dmax = std::max(std::max(std::max(p.ncls, p.n_ntiles), grid), std::max(std::max(p.tiles_w, p.tiles_h), p.cls_rot));
+    p.fd_tw = magic(p.tiles_w); p.fd_th = magic(p.tiles_h); p.fd_ocr = magic(p.OCr > 0 ? p.OCr : 1);
+    const long long dmax = std::max(std::max(p.ncls, p.n_ntiles), std::max(std::max(p.tiles_w, p.tiles_h), p.cls_rot));
     if ((long long)p.total_tiles * dmax >= (1ll << 32)) { set_error("tcgen05 conv: %d tiles exceed the fast-division range", p.total_tiles); return YG_ERR_INVALID; }
   }
-#define TC_LAUNCH(KCV, MODEV, PRODV)                                                                                    \
+#define TC_LAUNCH(KCV, MODEV)                                                                                           \
   do {                                                                                                                  \
-    YG_CUDA(cudaFuncSetAttribute(conv_tc_kernel<KCV, MODEV, PRODV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    conv_tc_kernel<KCV, MODEV, PRODV><<<grid, (PRODV ? 2 : 1) * 32 + 320, smem, st>>>(maps, p);                         \
+    YG_CUDA(cudaFuncSetAttribute(conv_tc_kernel<KCV, MODEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));  \
+    conv_tc_kernel<KCV, MODEV><<<grid, 352, smem, st>>>(maps, p);                                                       \
   } while (0)
   if (p.cta2) {
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3(grid, 1, 1);
-    cfg.blockDim = dim3(32 + 320, 1, 1);
+    cfg.blockDim = dim3(352, 1, 1);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
@@ -2402,27 +2134,30 @@ static int launch_engine(TcMaps& maps, TcParams& p, int KCc, int mode, int max_r
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     if (mode == 0) {
-      YG_CUDA(cudaFuncSetAttribute(conv_tc_kernel<64, 0, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      YG_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<64, 0, 0, 1>, maps, p));
+      YG_CUDA(cudaFuncSetAttribute(conv_tc_kernel<64, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      YG_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<64, 0, 1>, maps, p));
     } else {
-      YG_CUDA(cudaFuncSetAttribute(conv_tc_kernel<64, 1, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      YG_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<64, 1, 0, 1>, maps, p));
+      YG_CUDA(cudaFuncSetAttribute(conv_tc_kernel<64, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      YG_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<64, 1, 1>, maps, p));
     }
   } else if (mode == 0) {
-    if (KCc == 64) TC_LAUNCH(64, 0, 0);
-    else if (KCc == 32) { if (prod) TC_LAUNCH(32, 0, 1); else TC_LAUNCH(32, 0, 0); }
-    else { if (prod) TC_LAUNCH(16, 0, 1); else TC_LAUNCH(16, 0, 0); }
+    if (KCc == 64) TC_LAUNCH(64, 0); else if (KCc == 32) TC_LAUNCH(32, 0); else TC_LAUNCH(16, 0);
   } else {
-    if (KCc == 64) TC_LAUNCH(64, 1, 0);
-    else if (KCc == 32) { if (prod) TC_LAUNCH(32, 1, 1); else TC_LAUNCH(32, 1, 0); }
-    else { if (prod) TC_LAUNCH(16, 1, 1); else TC_LAUNCH(16, 1, 0); }
+    if (KCc == 64) TC_LAUNCH(64, 1); else if (KCc == 32) TC_LAUNCH(32, 1); else TC_LAUNCH(16, 1);
   }
 #undef TC_LAUNCH
   YG_LAUNCH_CHECK("conv_tc_kernel");
   return YG_OK;
 }
 
-int set_tc_options(int v) { g_tc_options = v; return 0; }
+int set_tc_options(int v) {
+  if (v & ~TC_OPTION_BITS) {
+    set_error("yg_set_tc_options: unknown option bits 0x%x (only bits 7-11 and 21 exist)", (unsigned)(v & ~TC_OPTION_BITS));
+    return YG_ERR_INVALID;
+  }
+  g_tc_options = v;
+  return YG_OK;
+}
 int get_tc_options() { return g_tc_options; }
 int tc_debug_read(unsigned long long* out, int n) {
   if (n > 256 * 16) n = 256 * 16;
@@ -2434,8 +2169,6 @@ int tc_debug_read(unsigned long long* out, int n) {
 // choose KC so that at least 2 stages fit
 static int fit_kc(int K, int BN, int max_rows) {
   int kc = pick_kc(K);
-  if ((g_tc_options & 32) && kc > 32) kc = 32;   // experiment knobs: cap the K chunk (swizzle row) at 64 / 32 bytes
-  if ((g_tc_options & 64) && kc > 16) kc = 16;
   while (kc >= 16) {
     const int stage = ((max_rows * TC_TW * kc * 2 + 1023) & ~1023) + 3 * BN * kc * 2;
     if (K % kc == 0 && TC_SMEM_BUDGET / stage >= 2) return kc;
@@ -2444,7 +2177,7 @@ static int fit_kc(int K, int BN, int max_rows) {
   return 0;
 }
 
-// 2-D halo boxes (option bit 13): ONE TMA box per (tile, K chunk) - (TH+2) x (TW+2) pixels for a stride-1 3x3 - instead
+// 2-D halo boxes: ONE TMA box per (tile, K chunk) - (TH+2) x (TW+2) pixels for a stride-1 3x3 - instead
 // of one column-shifted box per filter column.  The tile is 16 rows x 8 pixels, so every 8-pixel row group of the
 // M = 128 operand lies inside one box row and the groups are a constant SBO = box row pitch apart; a tap (r, s) is
 // just a start-address offset of (r * box_cols + s) pixel rows (the 128B / 64B / 32B swizzle is a function of the
@@ -2454,7 +2187,7 @@ static int fit_kc(int K, int BN, int max_rows) {
 constexpr int T2_TH = 16, T2_TW = 8;
 static bool two_d_fits(int K, int BN, int n_ntiles, int ntaps_total, int box_px, int ngroups, int* kc_out) {
   // (BN = weight rows kept per CTA: the whole N tile, or half of it for a CTA pair)
-  if (!(g_tc_options & 8192) || !(g_tc_options & 1) || n_ntiles != 1) return false;
+  if (n_ntiles != 1) return false;
   const int kc = pick_kc(K);
   if (!kc) return false;
   const int a_box = (box_px * kc * 2 + 1023) & ~1023;
@@ -2535,7 +2268,7 @@ int conv_fwd_tc(const void* x, const float* w, void* y, int N, int H, int W, int
   bool two_d = two_d1;
   // weights too large to stay resident in one CTA: a CTA pair keeps half of every weight tile each (cta_group::2)
   bool cta2 = false;
-  if (!two_d && (g_tc_options & 16384) && Cout == BN && BN % 32 == 0 && pick_kc(Cin) == 64 &&
+  if (!two_d && Cout == BN && BN % 32 == 0 && pick_kc(Cin) == 64 &&
       two_d_fits(Cin, BN / 2, 1, 9, stride == 1 ? (T2_TH + 2) * (T2_TW + 2) : (T2_TH + 1) * (T2_TW + 1), stride == 1 ? 1 : 4, &kc2))
     two_d = cta2 = true;
   const int KCc = two_d ? kc2 : fit_kc(Cin, BN, max_rows);
@@ -2600,13 +2333,11 @@ int conv_fwd_tc(const void* x, const float* w, void* y, int N, int H, int W, int
     rc = make_map(&maps.a[0], xb, 4, dims, str, box, KCc);
     if (rc) return rc;
     for (int i = 1; i < 4; ++i) maps.a[i] = maps.a[0];
-    for (int i = 0; i < 4; ++i) p.src[i] = TcSrc{xb, W, H, (long long)Cin, (long long)W * Cin, (long long)H * W * Cin};
     ngroups = 3;
     for (int s = 0; s < 3; ++s) {
       TcGroup& g = p.g[s];
       g.map = 0; g.dh = -1; g.dw = s - 1; g.rows = TC_TH + 2; g.ntaps = 3;
       for (int r = 0; r < 3; ++r) { g.ro[r] = r; g.widx[r] = r * 3 + s; g.kmask[r] = fold_kmask(fg, Cin_r, s, true); }
-      if (g_tc_options & 4096) { g.dw = 0; p.shift_exp[s] = (s - 1) * KCc * 2; }   // experiment: column shift by descriptor offset
     }
   } else {
     // parity sub-grids: element (h2, w2) of map (ph, pw) is x[2*h2+ph][2*w2+pw]
@@ -2619,8 +2350,6 @@ int conv_fwd_tc(const void* x, const float* w, void* y, int N, int H, int W, int
         uint32_t box[4] = {(uint32_t)KCc, TC_TW, (uint32_t)(ph ? TC_TH + 1 : TC_TH), 1};
         rc = make_map(&maps.a[ph * 2 + pw], xb + ((long long)ph * W + pw) * Cin, 4, dims, str, box, KCc);
         if (rc) return rc;
-        p.src[ph * 2 + pw] = TcSrc{xb + ((long long)ph * W + pw) * Cin, W2, H2, 2LL * Cin, 2LL * W * Cin,
-                                   (long long)H * W * Cin};
       }
     // input row 2*ho + r - 1: r=0 -> (ph=1, h2=ho-1), r=1 -> (ph=0, h2=ho), r=2 -> (ph=1, h2=ho)
     ngroups = 6;
@@ -2671,13 +2400,13 @@ int conv_dgrad_tc(const void* dz, const float* w, void* dx, int N, int H, int W,
   const bool two_d1 = two_d_fits(Cout, BN, Cin / BN, s2f ? 6 : 9,
                                  stride == 1 ? (T2_TH + 2) * (T2_TW + 2) : (T2_TH + 1) * (T2_TW + 1), 1, &kc2);
   bool two_d = two_d1, cta2 = false;
-  // (stride-2 dgrad as pairs - four parity classes in class-per-round order, option bit 15 - is implemented and correct but
-  //  slower: 0.64 vs 0.47 ms on base L5; its tiles carry 8-32 MMAs each and the pair's barrier round trips dominate)
+  // (no pairs for stride-2 dgrad: as four parity classes in a class-per-round tile order they measured slower, 0.64 vs 0.47 ms
+  //  on base L5; its tiles carry 8-32 MMAs each and the pair's barrier round trips dominate)
   // pairs also where the weights WOULD fit one CTA when N = 64 (unfolded): an M = 128, N = 64 MMA is bound by its
   // shared-memory operand fetch (4 KB of A + 2 KB of B for 32 cycles of math); in a pair each CTA fetches half of B.
-  // base L4 dgrad 0.49 -> 0.44 ms; the W-folded 16-channel layer does not gain (0.42 -> 0.43).  Option bit 18 turns it off.
-  const bool force_pair = !(g_tc_options & (1 << 18)) && two_d && stride == 1 && BN == 64 && fg == 1;
-  if ((!two_d || force_pair) && (g_tc_options & 16384) && !s2f && (stride == 1 || (g_tc_options & 32768)) && Cin == BN && BN % 32 == 0 &&
+  // base L4 dgrad 0.49 -> 0.44 ms; the W-folded 16-channel layer does not gain (0.42 -> 0.43).
+  const bool force_pair = two_d && stride == 1 && BN == 64 && fg == 1;
+  if ((!two_d || force_pair) && stride == 1 && Cin == BN && BN % 32 == 0 &&
       pick_kc(Cout) == 64 &&
       two_d_fits(Cout, BN / 2, 1, 9, stride == 1 ? (T2_TH + 2) * (T2_TW + 2) : (T2_TH + 1) * (T2_TW + 1), 1, &kc2))
     two_d = cta2 = true;   // CTA pair, see conv_fwd_tc
@@ -2709,8 +2438,6 @@ int conv_dgrad_tc(const void* dz, const float* w, void* dx, int N, int H, int W,
     if (rc) return rc;
   }
   maps.a[2] = maps.a[0]; maps.a[3] = maps.a[0];
-  for (int i = 0; i < 4; ++i)
-    p.src[i] = TcSrc{gb, Wo, Ho, (long long)Cout, (long long)Wo * Cout, (long long)Ho * Wo * Cout};
   // 2-D halo boxes over dz (see two_d_fits): map index = box shape (rows = T2_TH + a, cols = T2_TW + b)
   auto dz_map = [&](int mi, int rows, int cols) -> int {
     uint64_t dims[4] = {(uint64_t)Cout, (uint64_t)Wo, (uint64_t)Ho, (uint64_t)N};
@@ -2952,7 +2679,6 @@ int head_fwd_tc(const void* x, const float* w, const float* bias, float* out, fl
     rc = make_map(&maps.a[0], xb, 4, dims, str, box, KCc);
     if (rc) return rc;
     for (int i = 1; i < 4; ++i) maps.a[i] = maps.a[0];
-    for (int i = 0; i < 4; ++i) p.src[i] = TcSrc{xb, Sx, Sy, (long long)Cin, (long long)Sx * Cin, (long long)Sy * Sx * Cin};
   }
   TcGroup& g = p.g[0];
   g.map = 0; g.dh = 0; g.dw = 0; g.rows = TC_TH; g.ntaps = 1; g.ro[0] = 0; g.widx[0] = 0; g.kmask[0] = 0xFFFFFFFFu;
@@ -3016,7 +2742,6 @@ int head_bwd_tc(const void* dt, const void* x, const float* w, void* dx, float* 
       rc = make_map(&maps.a[0], dtb, 4, dims, str, box, KCc);
       if (rc) return rc;
       for (int i = 1; i < 4; ++i) maps.a[i] = maps.a[0];
-      for (int i = 0; i < 4; ++i) p.src[i] = TcSrc{dtb, Sx, Sy, (long long)DP, (long long)Sx * DP, (long long)Sy * Sx * DP};
     }
     TcGroup& g = p.g[0];
     g.map = 0; g.dh = 0; g.dw = 0; g.rows = TC_TH; g.ntaps = 1; g.ro[0] = 0; g.widx[0] = 0;
@@ -3068,7 +2793,6 @@ int head_bwd_tc(const void* dt, const void* x, const float* w, void* dx, float* 
       uint32_t box[4] = {(uint32_t)ka, TC_TW, TC_TH, 1};
       rc = make_map(&maps.a, dtb, 4, dims, str, box, ka);
       if (rc) return rc;
-      p.asrc = TcSrc{dtb, Sx, Sy, (long long)DP, (long long)Sx * DP, (long long)Sy * Sx * DP};
     }
     {
       const bf16* xb = (const bf16*)x;
@@ -3078,7 +2802,6 @@ int head_bwd_tc(const void* dt, const void* x, const float* w, void* dx, float* 
       rc = make_map(&maps.b[0], xb, 4, dims, str, box, kb);
       if (rc) return rc;
       for (int i = 1; i < 4; ++i) maps.b[i] = maps.b[0];
-      for (int i = 0; i < 4; ++i) p.bsrc[i] = TcSrc{xb, Sx, Sy, (long long)Cin, (long long)Sx * Cin, (long long)Sy * Sx * Cin};
     }
     p.ngroups = 1;
     TwGroup& g = p.g[0][0];
@@ -3088,8 +2811,8 @@ int head_bwd_tc(const void* dt, const void* x, const float* w, void* dx, float* 
     const size_t smem = (size_t)nst * p.stage_bytes + 1024 + 1024 + 2048;
 #define HW_LAUNCH(KBV)                                                                                                 \
   do {                                                                                                                 \
-    YG_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel<KBV, 32, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    wgrad_tc_kernel<KBV, 32, 0><<<grid, 192, smem, st>>>(maps, p);                                                     \
+    YG_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel<KBV, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    wgrad_tc_kernel<KBV, 32><<<grid, 192, smem, st>>>(maps, p);                                                     \
   } while (0)
     if (kb == 64) HW_LAUNCH(64); else if (kb == 32) HW_LAUNCH(32); else HW_LAUNCH(16);
 #undef HW_LAUNCH

@@ -1,5 +1,6 @@
-// Weight gradient of the small-channel 3x3 convolutions (Cin 16/32, Cout 32/64, stride 1/2) on the warp-level tensor
-// cores.  Replaces cuDNN wgrad for base_model layers 2 and 3 (/root/reference/yogo/model_defns.py:39-47).
+// Weight gradient of the 16 -> 32 channel stride-1 3x3 convolution on the warp-level tensor cores.  Replaces cuDNN wgrad
+// for base_model layer 2 (/root/reference/yogo/model_defns.py:39-47).  (The 32 -> 64 stride-2 layer 3 is faster on the
+// tcgen05 wgrad: this kernel is bound there by the mma.sync rate, 0.55 vs 0.47 ms.)
 //
 // The tcgen05 wgrad needs M = 128: with 32 or 64 output channels it runs W-folded (4x / 2x structurally-zero MACs) and its
 // three filter-column units re-read every tile, which makes it L2-bandwidth bound (0.5 ms for 1.2 GB of tensors).  Here:
@@ -307,7 +308,7 @@ bool wgrad_hmma_supported(int dtype, int W, int Cin, int Cout, int ks, int strid
   if (dtype != YG_BF16 || ks != 3) return false;
   const int Wo = (W + 2 - 3) / stride + 1;
   if (Wo < 1) return false;
-  return (Cin == 16 && Cout == 32 && stride == 1) || (Cin == 32 && Cout == 64 && stride == 2);
+  return Cin == 16 && Cout == 32 && stride == 1;
 }
 
 size_t wgrad_hmma_workspace(int Cin, int Cout) { return (size_t)HW_GRID * ((size_t)Cout * Cin * 9 + Cout) * sizeof(float) + 256; }
@@ -319,7 +320,6 @@ int conv_wgrad_hmma(const void* x, const void* dz, float* dw, float* dbias, int 
   if (!ws || ws_bytes < need) { set_error("conv_wgrad_hmma: workspace %zu < %zu", ws_bytes, need); return YG_ERR_WORKSPACE; }
   (void)ks;
   if (Cin == 16 && Cout == 32 && stride == 1) return launch_hmma<16, 32, 1>(x, dz, dw, dbias, N, H, W, clip, ws, st);
-  if (Cin == 32 && Cout == 64 && stride == 2) return launch_hmma<32, 64, 2>(x, dz, dw, dbias, N, H, W, clip, ws, st);
   set_error("conv_wgrad_hmma: unsupported shape");
   return YG_ERR_INVALID;
 }
