@@ -119,6 +119,19 @@ int yg_conv_first_bwd_finalize(const float* P, const float* Sg, const double* gr
                                const float* gamma, const float* mean, const float* invstd, double count,
                                int batch_stats, float clip, int Cout, float* dw, float* dbias, float* dgamma,
                                float* dbeta, void* stream);
+/* Gradient wrt the fp32 NCHW image x (N,Cin,H,W) of the first layer: dx (fp32 NCHW, overwritten, not clamped) =
+ * conv_transpose(dz, w) with dz = d(loss)/d(conv output) recomputed from x and da = grad wrt the block's (post-activation,
+ * post-Dropout2d) output (NHWC, dtype) exactly as yg_conv_first_bwd does: g' = da * dropscale * act'(pre), then
+ * dz = bn_scale*(g' - bn_dy_mean - xhat*bn_dyx_mean) for train-mode BatchNorm (the means of g' and g'*xhat over the
+ * N*Ho*Wo pixels), dz = bn_scale*g' when both means are NULL (running statistics), dz = g' when `be` has no BN.
+ * `be` and fwd_shift as for yg_conv_first_bwd (be->saved and be->bn_sums are not used).
+ * yg_conv_first_bn_means: those two means on the Gram path, from its raw P[Cout*9] / Sg[Cout] (yg_conv_first_bwd with
+ * bn_dy_mean == NULL and clip 0): dy_mean = Sg/count, dyx_mean = invstd*(sum_t w_t P_t + (bias - mean)*Sg)/count. */
+int yg_conv_first_dgrad(const float* x, const float* w, const void* da, int dtype, int N, int H, int W, int Cin, int Cout,
+                        int stride, const yg_bwd_epilogue* be, const float* fwd_shift, const float* bn_dy_mean,
+                        const float* bn_dyx_mean, float* dx, void* stream);
+int yg_conv_first_bn_means(const float* P, const float* Sg, const float* w, const float* bias, const float* mean,
+                           const float* invstd, double count, int Cout, float* dy_mean, float* dyx_mean, void* stream);
 
 /* Alignment: activation tensors handed to the convolution entry points should be 32-byte aligned (torch allocations are
  * 256-byte aligned); tensors that are only 16-byte aligned run on the generic SIMT path. */
@@ -180,13 +193,20 @@ int yg_head_fwd(const void* x, int dtype, const float* w, const float* bias, flo
                 float anchor_w, float anchor_h, float width_mult, float height_mult,
                 int inference, const float* cxs, const float* cys, void* stream);
 /* dpred (N,5+C,Sy,Sx) fp32 + t_raw -> dx NHWC (with the previous block's bwd epilogue),
- * dw (OIHW [5+C,Cin,1,1]) and dbias, clamped. Training head only (inference == 0). */
+ * dw (OIHW [5+C,Cin,1,1]) and dbias, clamped.  dw == NULL skips both parameter gradients (dbias is ignored): the
+ * backward of a frozen model.  dpred is the gradient wrt the raw class logits: for a head run with inference != 0 pass
+ * it through yg_head_softmax_bwd first. */
 size_t yg_head_bwd_workspace(int N, int Sy, int Sx, int Cin, int num_classes);
 int yg_head_bwd(const float* dpred, const float* t_raw, const void* x, const float* w, void* dx, int dtype,
                 float* dw, float* dbias, int N, int Sy, int Sx, int Cin, int num_classes,
                 float anchor_w, float anchor_h, float width_mult, float height_mult,
                 const yg_bwd_epilogue* be, float clip, void* workspace, size_t workspace_bytes,
                 void* stream);
+/* Softmax backward of the inference head (yg_head_fwd with inference != 0): out (N,5+C,Sy,Sx) fp32 = dpred with its class
+ * planes replaced by p * (dp - sum_j p_j dp_j), p = softmax of the raw class logits in t_raw computed as yg_head_fwd
+ * computes it; planes 0-4 are copied.  out must not overlap dpred. */
+int yg_head_softmax_bwd(const float* dpred, const float* t_raw, float* out, int N, int Sy, int Sx, int num_classes,
+                        void* stream);
 
 /* ---- YOGOLoss forward + backward in one pass -----------------------------------------
  * replaces yogo_loss.py:38-129 (+ torchvision box_convert / complete_box_iou_loss).

@@ -82,6 +82,15 @@ _PROTOS = {
         [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_double, c_int, c_float, c_int,
          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
     ),
+    "yg_conv_first_dgrad": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, C.POINTER(BwdEpilogue), c_void_p,
+         c_void_p, c_void_p, c_void_p, c_void_p],
+    ),
+    "yg_conv_first_bn_means": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_double, c_int, c_void_p, c_void_p, c_void_p],
+    ),
     "yg_conv_fwd": (
         c_int,
         [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, C.POINTER(FwdEpilogue), c_void_p],
@@ -127,6 +136,7 @@ _PROTOS = {
         [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
          c_float, c_float, c_float, c_float, C.POINTER(BwdEpilogue), c_float, c_void_p, c_size_t, c_void_p],
     ),
+    "yg_head_softmax_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_yogo_loss_workspace": (c_size_t, [c_int] * 3),
     "yg_yogo_loss_fwd_bwd": (
         c_int,

@@ -2761,8 +2761,8 @@ int head_bwd_tc(const void* dt, const void* x, const float* w, void* dx, float* 
     rc = launch_engine(maps, p, KCc, 1, TC_TH, st);
     if (rc) return rc;
   }
-  // ---------------- dW = dt^T . x
-  {
+  // ---------------- dW = dt^T . x (skipped when the caller needs no parameter gradients)
+  if (dw) {
     const size_t need = head_bwd_tc_workspace(Cin);
     if (!ws || ws_bytes < need) { set_error("head_bwd_tc: workspace %zu < %zu", ws_bytes, need); return YG_ERR_WORKSPACE; }
     TwMaps maps;

@@ -1009,6 +1009,156 @@ __global__ void __launch_bounds__(FM_WARPS * 32, 8) first_gram_mma_kernel(const 
   if (threadIdx.x < 54) atomicAdd(&gram[threadIdx.x], red[threadIdx.x]);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Input gradient of the first layer: dx = conv_transpose(dz, W) onto the fp32 NCHW image, with dz = d(loss)/d(conv output)
+// recomputed from (image, da) the way conv_first_bwd_kernel / first_bwd16_kernel do it (same stencil order, same
+// pre-activation expression, so a pre-activation on the LeakyReLU kink takes the same slope as in the weight gradient).
+// One CTA = FD_OH x FD_OW output pixels = (FD_OH*stride) x (FD_OW*stride) input pixels, per 16-channel chunk:
+//   phase 1: dz of the tile's output pixels plus the one-pixel halo its input pixels read, into shared memory
+//   phase 2: each thread gathers the taps of its input pixels from shared memory (no atomics).  At stride 2 a warp holds
+//            32 input pixels of one row and one column parity, so every lane of it takes the same taps (1 or 2 per axis).
+// ------------------------------------------------------------------------------------------------
+constexpr int FD_OH = 8, FD_OW = 32, FD_CO = 16, FD_THREADS = 128;
+constexpr int FD_DZS = FD_CO + 4;   // shared-memory pitch of one dz pixel: float4 reads of 8 consecutive pixels hit 32 banks
+constexpr int FD_DZ_PIX = (FD_OH + 2) * (FD_OW + 2);   // stride 1: one halo pixel on each side (stride 2: one at the end)
+
+// input pixel p of a tile -> (row, column) inside the tile; at stride 2 a run of 32 is one row and one column parity
+template <int STRIDE>
+__device__ __forceinline__ void fd_pixel(int p, int& ihl, int& iwl) {
+  if (STRIDE == 2) { ihl = p / 64; const int rem = p % 64; iwl = 2 * (rem % 32) + rem / 32; }
+  else { ihl = p / FD_OW; iwl = p % FD_OW; }
+}
+
+template <typename T, int STRIDE>
+__global__ void __launch_bounds__(FD_THREADS, 3) first_dgrad_kernel(
+    const float* __restrict__ x, const float* __restrict__ w, const T* __restrict__ da, float* __restrict__ dx,
+    int H, int W, int Cin, int Ho, int Wo, int Cout, BwdEpi be, const float* __restrict__ fwd_shift,
+    const float* __restrict__ dy_mean, const float* __restrict__ dyx_mean, int tiles_h, int tiles_w) {
+  __shared__ __align__(16) float ws[3 * 9 * FD_CO];        // [ci * 9 + tap][co]
+  __shared__ float cst[8 * FD_CO];                          // scl, sft, mean, istd, m1, m2, fsh, dropscale
+  __shared__ __align__(16) float dz[FD_DZ_PIX * FD_DZS];
+  const int tile = blockIdx.x;
+  const int n = tile / (tiles_h * tiles_w), tr = tile - n * tiles_h * tiles_w;
+  const int oh0 = (tr / tiles_w) * FD_OH, ow0 = (tr % tiles_w) * FD_OW;
+  constexpr int stride = STRIDE, NPT = STRIDE * STRIDE * FD_OH * FD_OW / FD_THREADS;   // input pixels per thread
+  const int ih0 = oh0 * stride, iw0 = ow0 * stride;
+  const int tih = FD_OH * stride, tiw = FD_OW * stride;
+  // output pixels the tile's input pixels receive from: ho * stride - 1 + r = ih, r = 0..2
+  const int ho_lo = max(0, (ih0 - 1 + stride - 1) / stride), ho_hi = min(Ho - 1, (ih0 + tih) / stride);
+  const int wo_lo = max(0, (iw0 - 1 + stride - 1) / stride), wo_hi = min(Wo - 1, (iw0 + tiw) / stride);
+  const int nrow = ho_hi - ho_lo + 1, ncol = wo_hi - wo_lo + 1;
+  const bool bn = be.bn_scale != nullptr, bn_batch = bn && dy_mean != nullptr;
+  float acc[NPT][3];
+#pragma unroll
+  for (int k = 0; k < NPT; ++k)
+#pragma unroll
+    for (int ci = 0; ci < 3; ++ci) acc[k][ci] = 0.f;
+
+  for (int co0 = 0; co0 < Cout; co0 += FD_CO) {
+    __syncthreads();   // the previous chunk's dz / weights are no longer read
+    load_first_weights<FD_CO>(ws, w, Cin, Cout, co0);
+    if (threadIdx.x < FD_CO) {
+      const int c = threadIdx.x, co = co0 + c;
+      const bool ok = co < Cout;
+      cst[c] = (bn && ok) ? be.bn_scale[co] : 1.f;
+      cst[FD_CO + c] = (bn && ok) ? be.bn_shift[co] : 0.f;
+      cst[2 * FD_CO + c] = (bn && ok) ? be.bn_mean[co] : 0.f;
+      cst[3 * FD_CO + c] = (bn && ok) ? be.bn_invstd[co] : 1.f;
+      cst[4 * FD_CO + c] = (bn_batch && ok) ? dy_mean[co] : 0.f;
+      cst[5 * FD_CO + c] = (bn_batch && ok) ? dyx_mean[co] : 0.f;
+      cst[6 * FD_CO + c] = (fwd_shift && ok) ? fwd_shift[co] : 0.f;
+      cst[7 * FD_CO + c] = (be.dropscale && ok) ? be.dropscale[(long long)n * Cout + co] : 1.f;
+    }
+    __syncthreads();
+    // ---- phase 1: dz of the (halo) output pixels
+    for (int q = threadIdx.x; q < nrow * ncol; q += FD_THREADS) {
+      const int ho = ho_lo + q / ncol, wo = wo_lo + q % ncol;
+      float a[FD_CO];
+      first_conv_pixel<float, FD_CO>(x, ws, n, ho, wo, H, W, Cin, stride, a);
+      const T* dp = da + (((long long)n * Ho + ho) * Wo + wo) * Cout + co0;
+      float* out = dz + q * FD_DZS;
+#pragma unroll
+      for (int c = 0; c < FD_CO; ++c) {
+        float d = 0.f;
+        if (co0 + c < Cout) {
+          float g = to_f<T>(dp[c]) * cst[7 * FD_CO + c];
+          const float yv = a[c] + cst[6 * FD_CO + c];   // conv output (+bias when no BN)
+          float pre = yv;
+          if (bn) pre = yv * cst[c] + cst[FD_CO + c];
+          g *= act_grad(pre, be.act);
+          if (bn_batch) {
+            const float xhat = (yv - cst[2 * FD_CO + c]) * cst[3 * FD_CO + c];
+            d = cst[c] * (g - cst[4 * FD_CO + c] - xhat * cst[5 * FD_CO + c]);
+          } else {
+            d = bn ? cst[c] * g : g;
+          }
+        }
+        out[c] = d;
+      }
+    }
+    __syncthreads();
+    // ---- phase 2: transposed 3x3 convolution, gathered per input pixel
+#pragma unroll
+    for (int k = 0; k < NPT; ++k) {
+      int ihl, iwl;
+      fd_pixel<STRIDE>(threadIdx.x + k * FD_THREADS, ihl, iwl);
+      const int ih = ih0 + ihl, iw = iw0 + iwl;
+      if (ih >= H || iw >= W) continue;
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        const int th = ih + 1 - r;
+        if (th < 0 || (stride == 2 && (th & 1))) continue;
+        const int ho = th / stride;
+        if (ho >= Ho) continue;
+#pragma unroll
+        for (int s = 0; s < 3; ++s) {
+          const int tw = iw + 1 - s;
+          if (tw < 0 || (stride == 2 && (tw & 1))) continue;
+          const int wo = tw / stride;
+          if (wo >= Wo) continue;
+          const float* d = dz + ((ho - ho_lo) * ncol + (wo - wo_lo)) * FD_DZS;
+#pragma unroll
+          for (int c4 = 0; c4 < FD_CO / 4; ++c4) {
+            const float4 dv = reinterpret_cast<const float4*>(d)[c4];
+#pragma unroll
+            for (int ci = 0; ci < 3; ++ci) {
+              if (ci < Cin) {
+                const float4 wv = reinterpret_cast<const float4*>(ws + (ci * 9 + r * 3 + s) * FD_CO)[c4];
+                acc[k][ci] += dv.x * wv.x + dv.y * wv.y + dv.z * wv.z + dv.w * wv.w;
+              }
+            }
+          }
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < NPT; ++k) {
+    int ihl, iwl;
+    fd_pixel<STRIDE>(threadIdx.x + k * FD_THREADS, ihl, iwl);
+    const int ih = ih0 + ihl, iw = iw0 + iwl;
+    if (ih >= H || iw >= W) continue;
+#pragma unroll
+    for (int ci = 0; ci < 3; ++ci)
+      if (ci < Cin) dx[(((long long)n * Cin + ci) * H + ih) * W + iw] = acc[k][ci];
+  }
+}
+
+// m1 = sum(g') / M and m2 = sum(g' xhat) / M of the Gram path from its raw P / Sg (the clamped dgamma / dbeta cannot be used)
+__global__ void first_bn_means_kernel(const float* __restrict__ P, const float* __restrict__ Sg, const float* __restrict__ w,
+                                      const float* __restrict__ bias, const float* __restrict__ mean,
+                                      const float* __restrict__ invstd, double count, int Cout, float* __restrict__ m1,
+                                      float* __restrict__ m2) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= Cout) return;
+  const double bi = bias ? (double)bias[c] : 0.0;
+  double wp = 0.0;
+  for (int t = 0; t < 9; ++t) wp += (double)w[c * 9 + t] * (double)P[c * 9 + t];
+  const double sg = Sg[c];
+  m1[c] = (float)(sg / count);
+  m2[c] = (float)((double)invstd[c] * (wp + (bi - (double)mean[c]) * sg) / count);
+}
+
 constexpr int FL_BWD_BLOCKS = 592;
 
 // aligned 16-bit tap loads: stride 2, even width (every row starts on an even offset) and an even base address
@@ -1312,5 +1462,43 @@ extern "C" int yg_conv_first_bwd_finalize(const float* P, const float* Sg, const
                                                                              count, batch_stats, clip, Cout, dw, dbias,
                                                                              dgamma, dbeta);
   YG_LAUNCH_CHECK("first_bwd_finalize");
+  return YG_OK;
+}
+
+extern "C" int yg_conv_first_dgrad(const float* x, const float* w, const void* da, int dtype, int N, int H, int W, int Cin,
+                                   int Cout, int stride, const yg_bwd_epilogue* bep, const float* fwd_shift,
+                                   const float* bn_dy_mean, const float* bn_dyx_mean, float* dx, void* stream) {
+  YG_CHECK_ARG(x && w && da && dx, "conv_first_dgrad: null pointer");
+  YG_CHECK_ARG(Cin >= 1 && Cin <= 3, "conv_first_dgrad: Cin must be 1..3, got %d", Cin);
+  YG_CHECK_ARG(Cout >= 1, "conv_first_dgrad: Cout %d", Cout);
+  YG_CHECK_ARG(stride == 1 || stride == 2, "conv_first_dgrad: stride %d", stride);
+  YG_CHECK_ARG(dtype == YG_F32 || dtype == YG_BF16, "conv_first_dgrad: dtype %d", dtype);
+  YG_CHECK_ARG((bn_dy_mean == nullptr) == (bn_dyx_mean == nullptr), "conv_first_dgrad: pass both BN means or neither");
+  BwdEpi be = make_bwd_epi(bep);
+  YG_CHECK_ARG(!be.bn_scale || (be.bn_shift && be.bn_mean && be.bn_invstd), "conv_first_dgrad: incomplete BN epilogue");
+  YG_CHECK_ARG(be.bn_scale || !bn_dy_mean, "conv_first_dgrad: BN means without BN");
+  if (N == 0 || H == 0 || W == 0) return YG_OK;
+  const int Ho = (H + 2 - 3) / stride + 1, Wo = (W + 2 - 3) / stride + 1;
+  const int tiles_h = cdiv(Ho, FD_OH), tiles_w = cdiv(Wo, FD_OW);
+  const long long nblk = (long long)N * tiles_h * tiles_w;
+  YG_CHECK_ARG(nblk < (1LL << 31), "conv_first_dgrad: image too large");
+  cudaStream_t st = (cudaStream_t)stream;
+#define LAUNCH(T, S) first_dgrad_kernel<T, S><<<(unsigned)nblk, FD_THREADS, 0, st>>>(x, w, (const T*)da, dx, H, W, Cin, Ho, Wo, \
+                                                   Cout, be, fwd_shift, bn_dy_mean, bn_dyx_mean, tiles_h, tiles_w)
+  if (dtype == YG_BF16) { if (stride == 2) LAUNCH(bf16, 2); else LAUNCH(bf16, 1); }
+  else { if (stride == 2) LAUNCH(float, 2); else LAUNCH(float, 1); }
+#undef LAUNCH
+  YG_LAUNCH_CHECK("conv_first_dgrad");
+  return YG_OK;
+}
+
+extern "C" int yg_conv_first_bn_means(const float* P, const float* Sg, const float* w, const float* bias, const float* mean,
+                                      const float* invstd, double count, int Cout, float* dy_mean, float* dyx_mean,
+                                      void* stream) {
+  YG_CHECK_ARG(P && Sg && w && mean && invstd && dy_mean && dyx_mean && Cout > 0 && count > 0,
+               "conv_first_bn_means: bad arguments");
+  first_bn_means_kernel<<<cdiv(Cout, 64), 64, 0, (cudaStream_t)stream>>>(P, Sg, w, bias, mean, invstd, count, Cout, dy_mean,
+                                                                        dyx_mean);
+  YG_LAUNCH_CHECK("first_bn_means");
   return YG_OK;
 }

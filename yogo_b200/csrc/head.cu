@@ -435,6 +435,39 @@ __global__ void __launch_bounds__(256) head_dt_kernel(const float* __restrict__ 
   if (threadIdx.x < D) db_partial[(long long)blockIdx.x * D + threadIdx.x] = sdb[threadIdx.x];
 }
 
+// Softmax backward of the inference head: the class planes of dpred (d loss / d softmax output) become d loss / d logits,
+// p * (dp - sum_j p_j dp_j), with p recomputed from the raw logits exactly as head_fwd_kernel computes it; planes 0-4 are
+// copied.  One thread per grid cell.
+template <int DMAX>
+__global__ void __launch_bounds__(256) head_softmax_bwd_kernel(const float* __restrict__ dpred, const float* __restrict__ t_raw,
+                                                               float* __restrict__ out, long long npix, int SS, int D) {
+  const long long p = (long long)blockIdx.x * 256 + threadIdx.x;
+  if (p >= npix) return;
+  const int n = (int)(p / SS), cell = (int)(p % SS);
+  const float* g = dpred + (long long)n * D * SS + cell;
+  float* o = out + (long long)n * D * SS + cell;
+  const float* t = t_raw + p * D;
+#pragma unroll
+  for (int d = 0; d < 5; ++d) o[(long long)d * SS] = g[(long long)d * SS];
+  float e[DMAX];
+  float mx = -INFINITY;
+#pragma unroll
+  for (int d = 5; d < DMAX; ++d)
+    if (d < D) { e[d] = t[d]; mx = fmaxf(mx, e[d]); }
+  float se = 0.f;
+#pragma unroll
+  for (int d = 5; d < DMAX; ++d)
+    if (d < D) { e[d] = expf(e[d] - mx); se += e[d]; }
+  const float inv = 1.f / se;
+  float dot = 0.f;
+#pragma unroll
+  for (int d = 5; d < DMAX; ++d)
+    if (d < D) { e[d] *= inv; dot += e[d] * g[(long long)d * SS]; }
+#pragma unroll
+  for (int d = 5; d < DMAX; ++d)
+    if (d < D) o[(long long)d * SS] = e[d] * (g[(long long)d * SS] - dot);
+}
+
 }  // namespace yg
 using namespace yg;
 
@@ -496,7 +529,7 @@ extern "C" int yg_head_bwd(const float* dpred, const float* t_raw, const void* x
                            const yg_bwd_epilogue* bep, float clip, void* workspace, size_t workspace_bytes,
                            void* stream) {
   const int D = 5 + num_classes;
-  YG_CHECK_ARG(dpred && t_raw && x && w && dw, "head_bwd: null pointer");
+  YG_CHECK_ARG(dpred && t_raw && x && w, "head_bwd: null pointer");
   YG_CHECK_ARG(num_classes >= 1 && D <= 32, "head_bwd: 5+num_classes must be <= 32, got %d", D);
   const long long npix = (long long)N * Sy * Sx;
   const size_t need = yg_head_bwd_workspace(N, Sy, Sx, Cin, num_classes);
@@ -516,7 +549,7 @@ extern "C" int yg_head_bwd(const float* dpred, const float* t_raw, const void* x
     if (nb > HD_DT_BLOCKS) nb = HD_DT_BLOCKS;
     head_dt_kernel<<<nb, 256, 0, st>>>(dpred, t_raw, dt, dbp, npix, Sy, Sx, D, anchor_w, anchor_h, width_mult, height_mult);
     YG_LAUNCH_CHECK("head_dt");
-    if (dbias) {
+    if (dw && dbias) {
       head_bias_reduce_kernel<<<cdiv(D * 32, 256), 256, 0, st>>>(dbp, dbias, D, nb, clip);
       YG_LAUNCH_CHECK("head_bias_reduce");
     }
@@ -543,6 +576,7 @@ extern "C" int yg_head_bwd(const float* dpred, const float* t_raw, const void* x
 #undef LAUNCHW_T
 #undef LAUNCHW
     YG_LAUNCH_CHECK("head_bwd_warp");
+    if (!dw) return YG_OK;
     const long long nw2 = (long long)D * Cin;
     head_reduce_kernel<<<cdiv(nw2 + D, 256), 256, 0, st>>>((const float*)workspace, dw, dbias, nw2, D, blocks, clip);
     YG_LAUNCH_CHECK("head_reduce");
@@ -562,8 +596,23 @@ extern "C" int yg_head_bwd(const float* dpred, const float* t_raw, const void* x
   else { if (DM == 16) LAUNCH(float, 16); else LAUNCH(float, 32); }
 #undef LAUNCH
   YG_LAUNCH_CHECK("head_bwd");
+  if (!dw) return YG_OK;
   const long long nw = (long long)D * Cin;
   head_reduce_kernel<<<cdiv(nw + D, 256), 256, 0, st>>>((const float*)workspace, dw, dbias, nw, D, blocks, clip);
   YG_LAUNCH_CHECK("head_reduce");
+  return YG_OK;
+}
+
+extern "C" int yg_head_softmax_bwd(const float* dpred, const float* t_raw, float* out, int N, int Sy, int Sx, int num_classes,
+                                   void* stream) {
+  const int D = 5 + num_classes;
+  YG_CHECK_ARG(dpred && t_raw && out, "head_softmax_bwd: null pointer");
+  YG_CHECK_ARG(num_classes >= 1 && D <= 32, "head_softmax_bwd: 5+num_classes must be <= 32, got %d", D);
+  const long long npix = (long long)N * Sy * Sx;
+  if (npix == 0) return YG_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (D <= 16) head_softmax_bwd_kernel<16><<<cdiv(npix, 256), 256, 0, st>>>(dpred, t_raw, out, npix, Sy * Sx, D);
+  else head_softmax_bwd_kernel<32><<<cdiv(npix, 256), 256, 0, st>>>(dpred, t_raw, out, npix, Sy * Sx, D);
+  YG_LAUNCH_CHECK("head_softmax_bwd");
   return YG_OK;
 }

@@ -371,8 +371,11 @@ class Runner:
         return outp, (saved if want_grad else None)
 
     # ---------------------------------------------------------------- backward
-    @L.on_device(lambda self, saved, dpred: dpred)
-    def backward(self, saved, dpred: torch.Tensor) -> List[Optional[torch.Tensor]]:
+    @L.on_device(lambda self, saved, dpred, **kw: dpred)
+    def backward(self, saved, dpred: torch.Tensor, want_params: bool = True,
+                 want_input: bool = False) -> Tuple[List[Optional[torch.Tensor]], Optional[torch.Tensor]]:
+        """Gradients of the parameters (in plan order; all of them, or none with want_params=False: nothing that only
+        produces parameter gradients runs then) and, with want_input, of the fp32 input as (N, Cin, H, W)."""
         own = self.owner
         lib = L.lib()
         st = L.stream()
@@ -385,6 +388,7 @@ class Runner:
         grads: Dict[int, torch.Tensor] = {}
         dpred = dpred.contiguous().float()
         views = self.grad_views or {}
+        dx: Optional[torch.Tensor] = None
 
         def gbuf(p: torch.Tensor) -> torch.Tensor:
             v = views.get(id(p))
@@ -428,20 +432,27 @@ class Runner:
         Cl = head.in_channels
         Sy, Sx, nc = saved["Sy"], saved["Sx"], saved["nc"]
         aw, ah, wm, hm = saved["consts"]
+        if own.inference:
+            # the class planes of the output are softmax probabilities: turn their gradient into the logits' gradient
+            dlogit = torch.empty_like(dpred)
+            L.check(lib.yg_head_softmax_bwd(dpred.data_ptr(), saved["t_raw"].data_ptr(), dlogit.data_ptr(), N, Sy, Sx,
+                                            nc, st))
+            dpred = dlogit
         last = len(plan.blocks) - 1
         ep, sums = bwd_ep(last)
         g = torch.empty((N, Sy, Sx, Cl), dtype=dt, device=dev)
-        dw_h = gbuf(head.weight)
-        db_h = gbuf(head.bias)
+        dw_h = gbuf(head.weight) if want_params else None
+        db_h = gbuf(head.bias) if want_params else None
         nbytes = lib.yg_head_bwd_workspace(N, Sy, Sx, Cl, nc)
         ws = L.workspace.get("head_bwd", nbytes, dev)
         L.check(lib.yg_head_bwd(dpred.data_ptr(), saved["t_raw"].data_ptr(), saved["head_in"].data_ptr(),
-                                _f32(head.weight).data_ptr(), g.data_ptr(), dcode, dw_h.data_ptr(), db_h.data_ptr(),
+                                _f32(head.weight).data_ptr(), g.data_ptr(), dcode, L.ptr(dw_h), L.ptr(db_h),
                                 N, Sy, Sx, Cl, nc, aw, ah, wm, hm, C.byref(ep) if ep is not None else None, clip,
                                 ws.data_ptr(), nbytes, st))
-        grads[id(head.weight)] = dw_h
-        grads[id(head.bias)] = db_h
-        done(head.weight, head.bias)
+        if want_params:
+            grads[id(head.weight)] = dw_h
+            grads[id(head.bias)] = db_h
+            done(head.weight, head.bias)
 
         # ---- conv blocks, last to first
         for i in range(last, -1, -1):
@@ -457,22 +468,36 @@ class Runner:
                     for t in ts:
                         if t is not None:
                             t.clamp_(-clip, clip)
-            dw = gbuf(blk.conv.weight)
-            db = gbuf(blk.conv.bias) if blk.conv.bias is not None else None
+            dw = gbuf(blk.conv.weight) if want_params else None
+            db = gbuf(blk.conv.bias) if (want_params and blk.conv.bias is not None) else None
             if rec["first_direct"]:
                 x, x_code = saved["x"], saved["x_code"]
                 nb = lib.yg_conv_first_bwd_workspace(blk.cin, blk.cout)
                 ws = L.workspace.get("first_bwd", nb, dev)
                 m1 = m2 = None
+                bn_train = blk.bn is not None and rec["bn_train"]
                 if blk.bn is not None and "gram" in rec:
                     # one pass over (da, image): P = sum g*x_t, Sg = sum g; everything else in closed form
                     P = torch.empty(blk.cout * 9, dtype=torch.float32, device=dev)
                     Sg = torch.empty(blk.cout, dtype=torch.float32, device=dev)
                     epp = L.BwdEpilogue(None, blk.act, L.ptr(rec["dropscale"]), rec["scale"].data_ptr(),
                                         rec["shift"].data_ptr(), rec["mean"].data_ptr(), rec["invstd"].data_ptr(), None)
-                    L.check(lib.yg_conv_first_bwd(x.data_ptr(), x_code, wt.data_ptr(), g.data_ptr(), dcode, N, h, w,
-                                                  blk.cin, blk.cout, blk.stride, C.byref(epp), L.ptr(rec.get("fwd_shift")),
-                                                  None, None, P.data_ptr(), Sg.data_ptr(), 0.0, ws.data_ptr(), nb, st))
+                    if want_params or bn_train:
+                        L.check(lib.yg_conv_first_bwd(x.data_ptr(), x_code, wt.data_ptr(), g.data_ptr(), dcode, N, h, w,
+                                                      blk.cin, blk.cout, blk.stride, C.byref(epp),
+                                                      L.ptr(rec.get("fwd_shift")), None, None, P.data_ptr(), Sg.data_ptr(),
+                                                      0.0, ws.data_ptr(), nb, st))
+                    if want_input:
+                        if bn_train:
+                            m1 = torch.empty(blk.cout, dtype=torch.float32, device=dev)
+                            m2 = torch.empty_like(m1)
+                            L.check(lib.yg_conv_first_bn_means(P.data_ptr(), Sg.data_ptr(), wt.data_ptr(),
+                                                               L.ptr(rec.get("fwd_shift")), rec["mean"].data_ptr(),
+                                                               rec["invstd"].data_ptr(), float(N * ho * wo), blk.cout,
+                                                               m1.data_ptr(), m2.data_ptr(), st))
+                        dx = self._first_dgrad(saved, blk, rec, wt, g, epp, rec.get("fwd_shift"), m1, m2)
+                    if not want_params:
+                        continue
                     dgam = gbuf(blk.bn.weight)
                     dbet = gbuf(blk.bn.bias)
                     L.check(lib.yg_conv_first_bwd_finalize(P.data_ptr(), Sg.data_ptr(), rec["gram"].data_ptr(),
@@ -492,34 +517,43 @@ class Runner:
                     done(blk.conv.weight, blk.conv.bias, blk.bn.weight, blk.bn.bias)
                     continue
                 if blk.bn is not None:
-                    sums = self._zeros64(2 * blk.cout, dev)
-                    ep1 = L.BwdEpilogue(None, blk.act, L.ptr(rec["dropscale"]), rec["scale"].data_ptr(),
-                                        rec["shift"].data_ptr(), rec["mean"].data_ptr(), rec["invstd"].data_ptr(),
-                                        sums.data_ptr())
-                    L.check(lib.yg_conv_first_bwd(x.data_ptr(), x_code, wt.data_ptr(), g.data_ptr(), dcode, N, h, w,
-                                                  blk.cin, blk.cout, blk.stride, C.byref(ep1), L.ptr(rec.get("fwd_shift")),
-                                                  None, None, None, None, clip, None, 0, st))
-                    dgam = gbuf(blk.bn.weight)
-                    dbet = gbuf(blk.bn.bias)
-                    L.check(lib.yg_bn_bwd_apply(None, None, dcode, N, ho * wo, blk.cout, sums.data_ptr(),
-                                                rec["gamma"].data_ptr(), rec["mean"].data_ptr(),
-                                                rec["invstd"].data_ptr(), dgam.data_ptr(), dbet.data_ptr(), clip,
-                                                1, st))
-                    grads[id(blk.bn.weight)] = dgam
-                    grads[id(blk.bn.bias)] = dbet
+                    if want_params or bn_train:
+                        sums = self._zeros64(2 * blk.cout, dev)
+                        ep1 = L.BwdEpilogue(None, blk.act, L.ptr(rec["dropscale"]), rec["scale"].data_ptr(),
+                                            rec["shift"].data_ptr(), rec["mean"].data_ptr(), rec["invstd"].data_ptr(),
+                                            sums.data_ptr())
+                        L.check(lib.yg_conv_first_bwd(x.data_ptr(), x_code, wt.data_ptr(), g.data_ptr(), dcode, N, h, w,
+                                                      blk.cin, blk.cout, blk.stride, C.byref(ep1),
+                                                      L.ptr(rec.get("fwd_shift")), None, None, None, None, clip, None, 0, st))
+                    if want_params:
+                        dgam = gbuf(blk.bn.weight)
+                        dbet = gbuf(blk.bn.bias)
+                        L.check(lib.yg_bn_bwd_apply(None, None, dcode, N, ho * wo, blk.cout, sums.data_ptr(),
+                                                    rec["gamma"].data_ptr(), rec["mean"].data_ptr(),
+                                                    rec["invstd"].data_ptr(), dgam.data_ptr(), dbet.data_ptr(), clip,
+                                                    1, st))
+                        grads[id(blk.bn.weight)] = dgam
+                        grads[id(blk.bn.bias)] = dbet
                     if rec["bn_train"]:
                         M = float(N * ho * wo)
                         m1 = (sums[: blk.cout] / M).float().contiguous()
                         m2 = (sums[blk.cout :] / M).float().contiguous()
-                    else:
+                    elif want_params:
                         m1 = torch.zeros(blk.cout, dtype=torch.float32, device=dev)
                         m2 = torch.zeros_like(m1)
                     ep2 = L.BwdEpilogue(None, blk.act, L.ptr(rec["dropscale"]), rec["scale"].data_ptr(),
                                         rec["shift"].data_ptr(), rec["mean"].data_ptr(), rec["invstd"].data_ptr(), None)
                 else:
                     ep2 = L.BwdEpilogue(None, blk.act, L.ptr(rec["dropscale"]), None, None, None, None, None)
+                fsh = rec.get("fwd_shift") if blk.bn is not None else (_f32(blk.conv.bias) if blk.conv.bias is not None else None)
+                if want_input:
+                    # running statistics: dz = scale * g' (the zero means above only serve the weight-gradient pass)
+                    dx = self._first_dgrad(saved, blk, rec, wt, g, ep2, fsh, m1 if rec["bn_train"] else None,
+                                           m2 if rec["bn_train"] else None)
+                if not want_params:
+                    continue
                 L.check(lib.yg_conv_first_bwd(x.data_ptr(), x_code, wt.data_ptr(), g.data_ptr(), dcode, N, h, w,
-                                              blk.cin, blk.cout, blk.stride, C.byref(ep2), L.ptr(rec.get("fwd_shift") if blk.bn is not None else (_f32(blk.conv.bias) if blk.conv.bias is not None else None)),
+                                              blk.cin, blk.cout, blk.stride, C.byref(ep2), L.ptr(fsh),
                                               L.ptr(m1), L.ptr(m2), dw.data_ptr(), L.ptr(db), clip_w, ws.data_ptr(), nb, st))
                 if in_scale:
                     dw.mul_(in_scale)
@@ -531,37 +565,53 @@ class Runner:
                      blk.bn.bias if blk.bn is not None else None)
                 continue
             if blk.bn is not None:
-                dgam = gbuf(blk.bn.weight)
-                dbet = gbuf(blk.bn.bias)
+                dgam = gbuf(blk.bn.weight) if want_params else None
+                dbet = gbuf(blk.bn.bias) if want_params else None
                 if sums is None:
                     sums = self._zeros64(2 * blk.cout, dev)
                     L.check(lib.yg_bn_bwd_sums(g.data_ptr(), rec["saved"].data_ptr(), dcode, N, ho * wo, blk.cout,
                                                rec["mean"].data_ptr(), rec["invstd"].data_ptr(), sums.data_ptr(), st))
                 L.check(lib.yg_bn_bwd_apply(g.data_ptr(), rec["saved"].data_ptr(), dcode, N, ho * wo, blk.cout,
                                             sums.data_ptr(), rec["gamma"].data_ptr(), rec["mean"].data_ptr(),
-                                            rec["invstd"].data_ptr(), dgam.data_ptr(), dbet.data_ptr(), clip,
+                                            rec["invstd"].data_ptr(), L.ptr(dgam), L.ptr(dbet), clip,
                                             1 if rec["bn_train"] else 0, st))
-                grads[id(blk.bn.weight)] = dgam
-                grads[id(blk.bn.bias)] = dbet
+                if want_params:
+                    grads[id(blk.bn.weight)] = dgam
+                    grads[id(blk.bn.bias)] = dbet
             # g is now d(loss)/d(conv output of block i)
-            db_from_wgrad = db
-            nb = lib.yg_conv_wgrad_workspace(N, h, w, blk.cin, blk.cout, blk.ksize, blk.stride)
-            ws = L.workspace.get("wgrad", nb, dev)
-            L.check(lib.yg_conv_wgrad(rec["in"].data_ptr(), g.data_ptr(), dw.data_ptr(), L.ptr(db_from_wgrad), dcode, N, h, w,
-                                      blk.cin, blk.cout, blk.ksize, blk.stride, clip, ws.data_ptr(), nb, st))
-            grads[id(blk.conv.weight)] = dw
-            if db is not None:
-                grads[id(blk.conv.bias)] = db
-            done(blk.conv.weight, blk.conv.bias, blk.bn.weight if blk.bn is not None else None,
-                 blk.bn.bias if blk.bn is not None else None)
-            if i > 0:
-                ep, sums = bwd_ep(i - 1)
+            if want_params:
+                db_from_wgrad = db
+                nb = lib.yg_conv_wgrad_workspace(N, h, w, blk.cin, blk.cout, blk.ksize, blk.stride)
+                ws = L.workspace.get("wgrad", nb, dev)
+                L.check(lib.yg_conv_wgrad(rec["in"].data_ptr(), g.data_ptr(), dw.data_ptr(), L.ptr(db_from_wgrad), dcode, N, h,
+                                          w, blk.cin, blk.cout, blk.ksize, blk.stride, clip, ws.data_ptr(), nb, st))
+                grads[id(blk.conv.weight)] = dw
+                if db is not None:
+                    grads[id(blk.conv.bias)] = db
+                done(blk.conv.weight, blk.conv.bias, blk.bn.weight if blk.bn is not None else None,
+                     blk.bn.bias if blk.bn is not None else None)
+            if i > 0 or want_input:
+                ep, sums = bwd_ep(i - 1) if i > 0 else (None, None)
                 gprev = torch.empty((N, h, w, blk.cin), dtype=dt, device=dev)
                 L.check(lib.yg_conv_dgrad(g.data_ptr(), wt.data_ptr(), gprev.data_ptr(), dcode, N, h, w, blk.cin,
                                           blk.cout, blk.ksize, blk.stride, C.byref(ep) if ep is not None else None, st))
                 g = gprev
+        if want_input and dx is None:
+            dx = g.permute(0, 3, 1, 2).float().contiguous()   # plumbing: NHWC gradient of the first conv's input -> NCHW
         # gradients already written into trainer-owned views are not returned through autograd
-        return [None if id(p) in views else grads.get(id(p)) for p in plan.params]
+        return [None if id(p) in views else grads.get(id(p)) for p in plan.params], dx
+
+    def _first_dgrad(self, saved, blk: ConvBlock, rec, wt: torch.Tensor, g: torch.Tensor, ep: L.BwdEpilogue, fwd_shift,
+                     m1, m2):
+        """d(loss)/d(image) of a direct first block (yg_conv_first_dgrad), fp32 (N, Cin, H, W)."""
+        x = saved["x"]   # fp32: a uint8 image cannot require a gradient
+        N, H, W = saved["N"], rec["h"], rec["w"]
+        dx = torch.empty((N, blk.cin, H, W), dtype=torch.float32, device=x.device)
+        L.check(L.lib().yg_conv_first_dgrad(x.data_ptr(), wt.data_ptr(), g.data_ptr(),
+                                            L.dtype_code(saved["dtype"]), N, H, W, blk.cin, blk.cout, blk.stride,
+                                            C.byref(ep), L.ptr(fwd_shift), L.ptr(m1), L.ptr(m2), dx.data_ptr(),
+                                            L.stream()))
+        return dx
 
 
 class _YOGOFunction(torch.autograd.Function):
@@ -570,18 +620,24 @@ class _YOGOFunction(torch.autograd.Function):
         out, saved = runner.forward(x, want_grad=True)
         ctx.runner = runner
         ctx.saved = saved
+        ctx.x_meta = (x.shape, x.dtype)
         return out
 
     @staticmethod
     def backward(ctx, dpred):
-        grads = ctx.runner.backward(ctx.saved, dpred)
+        # parameter gradients are all or nothing: a frozen model skips every weight-gradient pass
+        grads, dx = ctx.runner.backward(ctx.saved, dpred, want_params=any(ctx.needs_input_grad[2:]),
+                                        want_input=ctx.needs_input_grad[1])
         ctx.saved = None
-        return (None, None, *grads)
+        if dx is not None:
+            shape, dtype = ctx.x_meta
+            dx = dx.reshape(shape).to(dtype)   # (C, H, W) inputs and non-fp32 float inputs, which the engine casts to fp32
+        return (None, dx, *grads)
 
 
 def run(runner: Runner, x: torch.Tensor) -> torch.Tensor:
     params = runner.plan.params
-    need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+    need_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
     if need_grad:
         return _YOGOFunction.apply(runner, x, *params)
     out, _ = runner.forward(x, want_grad=False)
