@@ -338,6 +338,18 @@ int yg_flip_labels(const float* in, float* out, int N, int Sy, int Sx, int hflip
  * to 1 when a label centre falls outside the grid (the reference raises IndexError). */
 int yg_format_labels_batch(const float* labels, const int* offsets, int B, int max_labels, int Sy, int Sx,
                            int* owner, float* out, int* err, void* stream);
+/* Device-resident dataset (data/device_dataset.py), one batch of an epoch per call of each, all graph-capturable:
+ * yg_dd_draw: state (3 x uint64) = [seed, call counter, batch cursor]; writes flags (int32) = [hflip, vflip, batch]
+ * (hflip = u < p_hflip, vflip = u' < p_vflip with u, u' uniform in [0, 1) from Philox keyed by seed, stream_id and the
+ * counter; batch = cursor mod nbatches) and advances counter and cursor.  The table holds nbatches * stride entries.  yg_dd_gather_images: out[n] = the flags' flips of store[table[batch * stride
+ * + n]], n < N <= stride, (N, C, H, W) uint8 / fp32, C in {1, 3}.  yg_dd_build_labels: out (N, 6, Sy, Sx) fp32 = what
+ * yg_flip_labels gives for the stacked dense labels of the same images; records: 8 int32 per labelled cell {cell, the six
+ * channel values' bits, 0}, sorted by cell within a stored image, rec_off (int64) the record range of each stored image. */
+int yg_dd_draw(void* state, int* flags, float p_hflip, float p_vflip, int stream_id, int nbatches, void* stream);
+int yg_dd_gather_images(const void* store, void* out, int dtype, const int* table, const int* flags, int stride,
+                        int N, int C, int H, int W, void* stream);
+int yg_dd_build_labels(const int* table, const int* flags, int stride, const void* records, const long long* rec_off,
+                       int N, int Sy, int Sx, float* out, void* stream);
 
 /* ---- optimizer (SURVEY.md 8f N1): fused AdamW over one flat fp32 buffer ---------------
  * replaces torch.optim.AdamW.step (train.py:213-217, 324). grads are pre-scaled by

@@ -185,6 +185,9 @@ _PROTOS = {
     "yg_flip_labels": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_format_labels_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "yg_dropout_scales": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p]),
+    "yg_dd_draw": (c_int, [c_void_p, c_void_p, c_float, c_float, c_int, c_int, c_void_p]),
+    "yg_dd_gather_images": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "yg_dd_build_labels": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "yg_adamw_flat_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p]),
     "yg_adamw_flat": (
         c_int,

@@ -8,10 +8,36 @@ namespace yg {
 
 // one block = FLIP_ROWS consecutive output rows, one thread = one V-element vector at a time;
 // out[y][x] = in[vflip ? H-1-y : y][hflip ? W-1-x : x].  32-bit index arithmetic; the only 64-bit division is one per block.
+// `Src` says where output plane p (= n * C + c) comes from and which flips apply: FlipArgs (the batch flip, plane p of the
+// input, flips from the arguments) or GatherSrc (the device-resident dataset: plane of a stored image, flips from memory).
 constexpr int FLIP_ROWS = 16;
-template <typename T, int V>
+struct FlipArgs {
+  int hflip, vflip;
+  __device__ __forceinline__ void load() {}
+  __device__ __forceinline__ long long plane(long long p) const { return p; }
+};
+// batch `flags[2]` of an epoch's index table (row stride `stride`): output image n is stored image table[batch * stride + n]
+struct GatherSrc {
+  const int* table;
+  const int* flags;   // [hflip, vflip, batch] written by dd_draw_kernel
+  int stride, C;
+  int hflip, vflip;
+  long long base;
+  __device__ __forceinline__ void load() {
+    hflip = flags[0];
+    vflip = flags[1];
+    base = (long long)flags[2] * stride;
+  }
+  __device__ __forceinline__ long long plane(long long p) const {
+    const int pi = (int)p, n = pi / C;
+    return (long long)__ldg(table + base + n) * C + (pi - n * C);
+  }
+};
+template <typename T, int V, typename Src>
 __global__ void __launch_bounds__(256) flip_images_kernel(const T* __restrict__ in, T* __restrict__ out, long long rows, int H,
-                                                          int W, int hflip, int vflip) {
+                                                          int W, Src src) {
+  src.load();
+  const int hflip = src.hflip, vflip = src.vflip;
   const int vpr = W / V;   // vectors per row
   struct alignas(sizeof(T) * V) Vec { T e[V]; };
   const long long row0 = (long long)blockIdx.x * FLIP_ROWS;
@@ -25,7 +51,7 @@ __global__ void __launch_bounds__(256) flip_images_kernel(const T* __restrict__ 
     while (y >= H) { y -= H; ++plane; }
     const int sy = vflip ? H - 1 - y : y;
     const int sv = hflip ? vpr - 1 - vx : vx;
-    const Vec v = *reinterpret_cast<const Vec*>(in + (plane * H + sy) * (long long)W + sv * V);
+    const Vec v = *reinterpret_cast<const Vec*>(in + (src.plane(plane) * H + sy) * (long long)W + sv * V);
     Vec o;
     if (hflip) {
 #pragma unroll
@@ -112,12 +138,12 @@ extern "C" int yg_flip_images(const void* in, void* out, int dtype, int N, int C
   cudaStream_t st = (cudaStream_t)stream;
   const bool al = (((uintptr_t)in | (uintptr_t)out) & 15) == 0;
   if (dtype == YG_U8) {
-    if (al && W % 16 == 0) flip_images_kernel<uint8_t, 16><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)in, (uint8_t*)out, rows, H, W, hflip, vflip);
-    else if (al && W % 8 == 0) flip_images_kernel<uint8_t, 8><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)in, (uint8_t*)out, rows, H, W, hflip, vflip);
-    else flip_images_kernel<uint8_t, 1><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)in, (uint8_t*)out, rows, H, W, hflip, vflip);
+    if (al && W % 16 == 0) flip_images_kernel<uint8_t, 16><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)in, (uint8_t*)out, rows, H, W, FlipArgs{hflip, vflip});
+    else if (al && W % 8 == 0) flip_images_kernel<uint8_t, 8><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)in, (uint8_t*)out, rows, H, W, FlipArgs{hflip, vflip});
+    else flip_images_kernel<uint8_t, 1><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)in, (uint8_t*)out, rows, H, W, FlipArgs{hflip, vflip});
   } else {
-    if (al && W % 4 == 0) flip_images_kernel<float, 4><<<flip_grid(rows), 256, 0, st>>>((const float*)in, (float*)out, rows, H, W, hflip, vflip);
-    else flip_images_kernel<float, 1><<<flip_grid(rows), 256, 0, st>>>((const float*)in, (float*)out, rows, H, W, hflip, vflip);
+    if (al && W % 4 == 0) flip_images_kernel<float, 4><<<flip_grid(rows), 256, 0, st>>>((const float*)in, (float*)out, rows, H, W, FlipArgs{hflip, vflip});
+    else flip_images_kernel<float, 1><<<flip_grid(rows), 256, 0, st>>>((const float*)in, (float*)out, rows, H, W, FlipArgs{hflip, vflip});
   }
   YG_LAUNCH_CHECK("flip_images");
   return YG_OK;
@@ -216,5 +242,115 @@ extern "C" int yg_dropout_scales(float* out, const void* table, int nblocks, int
   yg::dropout_scales_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(out, (const int4*)table, nblocks, total,
                                                                     (unsigned long long*)state, (long long* const*)counters, ncounters);
   YG_LAUNCH_CHECK("dropout_scales");
+  return YG_OK;
+}
+
+
+// ------------------------------------------------------------------------------------------------
+// Device-resident dataset (data/device_dataset.py): every batch of an epoch is built on the device from the decoded store,
+// so that a CUDA-graph replay of the training step draws, gathers and rasterises its own batch.
+//   draw:   one (hflip, vflip) pair per batch (the reference flips whole batches in the collate function,
+//           data_transforms.py:51-98) from Philox keyed by (seed, call counter); state = [seed, counter, batch cursor] in
+//           device memory, advanced by the kernel itself like dropout_scales; flags = [hflip, vflip, batch] of the batch
+//           just drawn, read by the two kernels below and by callers.
+//   images: flip_images_kernel with GatherSrc (one HBM pass, vector accesses).
+//   labels: the (B, 6, Sy, Sx) tensor flip_batch(stack(labels), h, v) produces, from per-image compact cell records.
+// ------------------------------------------------------------------------------------------------
+namespace yg {
+__global__ void dd_draw_kernel(unsigned long long* __restrict__ state, int* __restrict__ flags, float ph, float pv,
+                               uint32_t stream_id, int nbatches) {
+  const unsigned long long seed = state[0], call = state[1], cursor = state[2];
+  const uint4 r = philox4x32_10(make_uint4(stream_id, 0x464C4950u, (uint32_t)call, (uint32_t)(call >> 32)),
+                                make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+  const float uh = (float)(r.x >> 8) * (1.0f / 16777216.0f), uv = (float)(r.y >> 8) * (1.0f / 16777216.0f);  // [0, 1)
+  flags[0] = uh < ph;   // p = 0: never, p = 1: always
+  flags[1] = uv < pv;
+  flags[2] = (int)(cursor % (unsigned long long)nbatches);   // a draw past the epoch's end starts it again
+  state[1] = call + 1ull;
+  state[2] = cursor + 1ull;
+}
+
+// records: two int4 per labelled cell {cell, 6 channel values as float bits, 0}, sorted by cell within each stored image;
+// rec_off[i], rec_off[i + 1]: record range of stored image i.  One block = `rpb` output rows of one image: it writes the
+// mirrored default of its rows (channels that the flip complements are 1 - 0 = 1, the rest 0, as flip_labels_kernel gives
+// for an unlabelled cell), then its labelled cells, whose sources are one contiguous record range (rows map to rows).
+__global__ void __launch_bounds__(256) dd_labels_kernel(const int* __restrict__ table, const int* __restrict__ flags, int stride,
+                                                        const int4* __restrict__ rec, const long long* __restrict__ rec_off,
+                                                        int Sy, int Sx, int rpb, float* __restrict__ out) {
+  const int hflip = flags[0], vflip = flags[1];
+  const int b = blockIdx.y;
+  const int img = table[(long long)flags[2] * stride + b];
+  const int r0 = blockIdx.x * rpb, r1 = min(Sy, r0 + rpb);
+  const int plane = Sy * Sx;
+  float* o = out + (long long)b * 6 * plane;
+  const float one = __fsub_rn(1.f, 0.f);
+#pragma unroll
+  for (int k = 0; k < 6; ++k) {
+    const float d = (hflip && (k == 1 || k == 3)) || (vflip && (k == 2 || k == 4)) ? one : 0.f;
+    for (int c = r0 * Sx + threadIdx.x; c < r1 * Sx; c += blockDim.x) o[k * plane + c] = d;
+  }
+  __syncthreads();   // the labelled cells below overwrite defaults written by other threads of this block
+  const int s0 = vflip ? Sy - r1 : r0, s1 = vflip ? Sy - r0 : r1;   // source rows of output rows [r0, r1)
+  const long long lo = rec_off[img], hi = rec_off[img + 1];
+  long long a = lo, e = hi;
+  while (a < e) { const long long m = (a + e) >> 1; if (rec[2 * m].x < s0 * Sx) a = m + 1; else e = m; }
+  const long long first = a;
+  e = hi;
+  while (a < e) { const long long m = (a + e) >> 1; if (rec[2 * m].x < s1 * Sx) a = m + 1; else e = m; }
+  for (long long i = first + threadIdx.x; i < a; i += blockDim.x) {
+    const int4 h0 = rec[2 * i], h1 = rec[2 * i + 1];
+    const int sy = h0.x / Sx, sx = h0.x - sy * Sx;
+    const int oc = (vflip ? Sy - 1 - sy : sy) * Sx + (hflip ? Sx - 1 - sx : sx);
+    float v[6] = {__int_as_float(h0.y), __int_as_float(h0.z), __int_as_float(h0.w),
+                  __int_as_float(h1.x), __int_as_float(h1.y), __int_as_float(h1.z)};
+    if (hflip) { const float t = v[1]; v[1] = __fsub_rn(1.f, v[3]); v[3] = __fsub_rn(1.f, t); }
+    if (vflip) { const float t = v[2]; v[2] = __fsub_rn(1.f, v[4]); v[4] = __fsub_rn(1.f, t); }
+#pragma unroll
+    for (int k = 0; k < 6; ++k) o[k * plane + oc] = v[k];
+  }
+}
+}  // namespace yg
+
+extern "C" int yg_dd_draw(void* state, int* flags, float p_hflip, float p_vflip, int stream_id, int nbatches, void* stream) {
+  YG_CHECK_ARG(state && flags && nbatches > 0, "dd_draw: bad arguments");
+  YG_CHECK_ARG(p_hflip >= 0.f && p_hflip <= 1.f && p_vflip >= 0.f && p_vflip <= 1.f, "dd_draw: p outside [0, 1]");
+  yg::dd_draw_kernel<<<1, 1, 0, (cudaStream_t)stream>>>((unsigned long long*)state, flags, p_hflip, p_vflip,
+                                                         (uint32_t)stream_id, nbatches);
+  YG_LAUNCH_CHECK("dd_draw");
+  return YG_OK;
+}
+
+extern "C" int yg_dd_gather_images(const void* store, void* out, int dtype, const int* table, const int* flags, int stride,
+                                   int N, int C, int H, int W, void* stream) {
+  YG_CHECK_ARG(dtype == YG_U8 || dtype == YG_F32, "dd_gather_images: dtype %d", dtype);
+  YG_CHECK_ARG(C == 1 || C == 3, "dd_gather_images: C = %d (1 or 3)", C);
+  const long long rows = (long long)N * C * H;
+  if (rows == 0 || W == 0) return YG_OK;
+  YG_CHECK_ARG(store && out && table && flags && store != out && N <= stride, "dd_gather_images: bad arguments");
+  YG_CHECK_ARG(rows / FLIP_ROWS < (1LL << 31), "dd_gather_images: too many rows");
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool al = (((uintptr_t)store | (uintptr_t)out) & 15) == 0;
+  const GatherSrc g{table, flags, stride, C, 0, 0, 0};
+  if (dtype == YG_U8) {
+    if (al && W % 16 == 0) flip_images_kernel<uint8_t, 16><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)store, (uint8_t*)out, rows, H, W, g);
+    else if (al && W % 8 == 0) flip_images_kernel<uint8_t, 8><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)store, (uint8_t*)out, rows, H, W, g);
+    else flip_images_kernel<uint8_t, 1><<<flip_grid(rows), 256, 0, st>>>((const uint8_t*)store, (uint8_t*)out, rows, H, W, g);
+  } else {
+    if (al && W % 4 == 0) flip_images_kernel<float, 4><<<flip_grid(rows), 256, 0, st>>>((const float*)store, (float*)out, rows, H, W, g);
+    else flip_images_kernel<float, 1><<<flip_grid(rows), 256, 0, st>>>((const float*)store, (float*)out, rows, H, W, g);
+  }
+  YG_LAUNCH_CHECK("dd_gather_images");
+  return YG_OK;
+}
+
+extern "C" int yg_dd_build_labels(const int* table, const int* flags, int stride, const void* records, const long long* rec_off,
+                                  int N, int Sy, int Sx, float* out, void* stream) {
+  if (N == 0 || Sy == 0 || Sx == 0) return YG_OK;
+  YG_CHECK_ARG(table && flags && records && rec_off && out && N <= stride, "dd_build_labels: bad arguments");
+  YG_CHECK_ARG(N <= 65535 && (long long)Sy * Sx * 6 < (1LL << 31), "dd_build_labels: batch %d or grid too large", N);
+  const int rpb = Sx >= 2048 ? 1 : 2048 / Sx;
+  dim3 grid(cdiv(Sy, rpb), N, 1);
+  dd_labels_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(table, flags, stride, (const int4*)records, rec_off, Sy, Sx, rpb, out);
+  YG_LAUNCH_CHECK("dd_build_labels");
   return YG_OK;
 }

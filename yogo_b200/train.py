@@ -385,6 +385,65 @@ class DataParallelTrainer:
             nxt = nxt2
             slot = (slot + 1) % nslot
 
+    def steps_from_device(self, dd, epoch: int):
+        """Generator: one training step per batch of `epoch` of the device-resident dataset `dd`
+        (`yogo_b200.data.DeviceResidentDataset`), yielding the loss tensor.  In graph mode (after `enable_cuda_graph`
+        with `dd`'s batch shape) every full batch is one replay of a graph that draws the flips, gathers the images, builds
+        the labels into the static input slot 0 and then runs the captured step; the host only stages the 32 hyper-parameter
+        bytes and launches it.  The ragged last batch, and every batch without graph mode, runs eagerly through the same
+        kernels."""
+        dev = self.flat_p.device
+        with torch.cuda.device(dev):
+            dd.begin_epoch(epoch)
+        graph = self._device_graph(dd) if self._graph is not None else None
+        for n in dd.batch_sizes(epoch):
+            if graph is not None and n == dd.batch_size:
+                self._check_views()
+                self.step_count += 1
+                self._hyper.copy_(self._hyper_host(self.step_count))
+                graph[2].replay()
+                yield graph[3].clone()
+            else:
+                yield self.step(*dd.next_batch(n))
+
+    def _device_graph(self, dd):
+        """(dd, step graph it was captured beside, graph, loss) of `dd`'s batch step, captured on first use with the warm-up / snapshot / restore discipline
+        of `enable_cuda_graph`, in the memory pool of its graphs.  `dd`'s draw counter and cursor are restored too."""
+        cached = getattr(self, "_dev_graph", None)
+        if cached is not None and cached[0] is dd and cached[1] is self._graphs[0]:
+            return cached
+        imgs, labels = self._static[0]
+        if tuple(imgs.shape) != (dd.batch_size,) + tuple(dd.image_shape) or imgs.dtype != dd.image_dtype or \
+                tuple(labels.shape) != (dd.batch_size, 6) + tuple(dd.grid):
+            raise ValueError(f"steps_from_device: the captured step takes images {tuple(imgs.shape)} {imgs.dtype} and labels "
+                             f"{tuple(labels.shape)}, the dataset's batches are ({dd.batch_size}, {dd.image_shape}) "
+                             f"{dd.image_dtype} and ({dd.batch_size}, 6, {dd.grid})")
+        dev = self.flat_p.device
+
+        def body():
+            dd.next_batch_into(imgs, labels)
+            loss = self.forward_backward(imgs, labels)
+            self._adamw_dev()
+            return loss
+
+        snap, dd_state, rng = self.snapshot(), dd.state(), torch.cuda.get_rng_state(dev)
+        self._hyper.copy_(self._hyper_host(1))
+        s = torch.cuda.Stream(device=dev)
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            body()
+        torch.cuda.current_stream().wait_stream(s)
+        torch.cuda.synchronize()
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph, pool=self._graphs[0].pool(), capture_error_mode="thread_local" if self.world > 1 else "global"):
+            loss = body()
+        self.restore(snap)
+        dd.set_state(dd_state)
+        torch.cuda.set_rng_state(rng, dev)
+        torch.cuda.synchronize()
+        self._dev_graph = (dd, self._graphs[0], graph, loss)
+        return self._dev_graph
+
     # ------------------------------------------------------------------ checkpoint state (train.py:262-293)
     def optimizer_state_dict(self) -> Dict:
         """`torch.optim.AdamW.state_dict()` layout (what the reference stores under "optimizer_state_dict"): per-parameter
