@@ -351,6 +351,49 @@ int yg_dd_gather_images(const void* store, void* out, int dtype, const int* tabl
 int yg_dd_build_labels(const int* table, const int* flags, int stride, const void* records, const long long* rec_off,
                        int N, int Sy, int Sx, float* out, void* stream);
 
+/* ---- PNG decoding: 8-bit grayscale, non-interlaced files (yogo_b200.data.decode_png_batch) ----------------------
+ * One call decodes n files of the same H x W.  `files` (device, files_bytes) holds what the host uploaded; the host has
+ * walked each file's chunks and lists every IDAT as a yg_png_chunk and each image as a yg_png_image:
+ *   chunk.src     offset in `files` of the chunk's type field (the CRC covers type + payload);
+ *   chunk.dst     offset of its payload in the workspace's stream region (the image's zlib stream, chunks back to back);
+ *   chunk.length  payload bytes; chunk.crc the stored CRC-32;
+ *   image.stream  offset of the image's zlib stream in the stream region (a multiple of 16), image.length its bytes;
+ *   image.chunk_begin / chunk_end  its range of `chunks`.
+ * yg_png_gray8_workspace(n, H, W, stream_bytes) is the workspace for a stream region of stream_bytes (the end of the
+ * last stream, rounded up to 16); it must be 16-byte aligned (the inflate reads it in 16-byte loads), chunks and images
+ * 8-byte aligned.  out is (n, 1, H, W) uint8.  status[n] (int32) is always written with a
+ * yg_png_status; the output of an image whose status is not YG_PNG_OK is undefined.  Kernels: IDAT gather + CRC,
+ * inflate (one warp per image), unfilter + Adler-32 (one warp per image), all on `stream`. */
+enum {
+  YG_PNG_OK = 0,
+  YG_PNG_BAD_CRC = 1,            /* an IDAT CRC-32 does not match */
+  YG_PNG_BAD_ZLIB_HEADER = 2,    /* CM != 8, CINFO > 7, FCHECK, or a preset dictionary */
+  YG_PNG_BAD_BLOCK_TYPE = 3,     /* BTYPE 3 */
+  YG_PNG_BAD_STORED_LENGTH = 4,  /* stored block LEN != ~NLEN */
+  YG_PNG_BAD_CODE_LENGTHS = 5,   /* over-subscribed or incomplete code, bad repeat, too many symbols, no end-of-block */
+  YG_PNG_BAD_SYMBOL = 6,         /* length symbol 286/287, distance symbol 30/31 or an unused distance code */
+  YG_PNG_BAD_DISTANCE = 7,       /* distance beyond the bytes produced or the window */
+  YG_PNG_OUTPUT_OVERFLOW = 8,    /* more than H * (1 + W) bytes */
+  YG_PNG_TRUNCATED = 9,          /* the stream ends early, or its image data is short */
+  YG_PNG_TRAILING_DATA = 10,     /* bytes after the Adler-32 */
+  YG_PNG_BAD_ADLER = 11,         /* Adler-32 mismatch */
+  YG_PNG_BAD_FILTER = 12,        /* scanline filter byte > 4 */
+  YG_PNG_BAD_LAYOUT = 13         /* a chunk or stream outside the buffers it was described in */
+};
+typedef struct {
+  long long src, dst;
+  int length;
+  unsigned int crc;
+} yg_png_chunk;
+typedef struct {
+  long long stream, length;
+  int chunk_begin, chunk_end;
+} yg_png_image;
+size_t yg_png_gray8_workspace(int n, int H, int W, long long stream_bytes);
+int yg_png_decode_gray8(const void* files, long long files_bytes, const yg_png_chunk* chunks, const yg_png_image* images,
+                        int n, int H, int W, unsigned char* out, int* status, void* workspace, size_t ws_bytes,
+                        void* stream);
+
 /* ---- optimizer (SURVEY.md 8f N1): fused AdamW over one flat fp32 buffer ---------------
  * replaces torch.optim.AdamW.step (train.py:213-217, 324). grads are pre-scaled by
  * grad_scale (1/world_size after an all-reduce SUM). */

@@ -188,6 +188,11 @@ _PROTOS = {
     "yg_dd_draw": (c_int, [c_void_p, c_void_p, c_float, c_float, c_int, c_int, c_void_p]),
     "yg_dd_gather_images": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_dd_build_labels": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "yg_png_gray8_workspace": (c_size_t, [c_int, c_int, c_int, c_longlong]),
+    "yg_png_decode_gray8": (
+        c_int,
+        [c_void_p, c_longlong, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
+    ),
     "yg_adamw_flat_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p]),
     "yg_adamw_flat": (
         c_int,

@@ -152,6 +152,81 @@ def _read_image(path: Path) -> torch.Tensor:
     return read_image(str(path), ImageReadMode.GRAY)
 
 
+# Files of `predict` are decoded in groups of this many images per SM (rounded up to whole batches): the inflate kernel
+# runs one warp per image, so a group needs several warps per SM to hide the latency of its serial decode.  8 per SM
+# (1184 images on a B200, about 2.5 GB of output, scratch and streams at 772x1032) measured as fast as 16 per SM in
+# `predict`, whose rate is bound by the host work of each group (profiles/png_decode_bench.jsonl), at half the memory.
+DECODE_IMAGES_PER_SM = 8
+
+
+def _read_files(paths: Sequence[Path]) -> list:
+    """Raw bytes of the PNG files (torchvision.io.read_file) and decoded .npy arrays, or the exception a read raised."""
+    from torchvision.io import read_file
+
+    items = []
+    for q in paths:
+        try:
+            items.append(_read_image(q) if q.suffix.lower() == ".npy" else read_file(str(q)))
+        except Exception as e:   # raised again when its batch is loaded, like the per-batch read of the reference
+            items.append(e)
+    return items
+
+
+class _FolderDecoder:
+    """Images of `paths` for `predict`, decoded on the GPU in groups of whole batches (data.png.decode_entries) while a
+    small thread pool reads the next group's files.  `prepare(lo)` decodes the group that holds batch `lo`; an error
+    there (out of memory, a failed launch) is not a file's error and propagates.  `batch(lo, hi)` then returns what
+    ``torch.stack([_read_image(q) for q in paths[lo:hi]])`` returns, on `dev`, and raises what it raises."""
+
+    def __init__(self, paths: Sequence[Path], dev: torch.device, batch_size: int):
+        import math
+        from concurrent.futures import ThreadPoolExecutor
+
+        sms = torch.cuda.get_device_properties(dev).multi_processor_count
+        self.group = max(1, math.ceil(sms * DECODE_IMAGES_PER_SM / batch_size)) * batch_size
+        self.paths, self.dev = list(paths), dev
+        self.workers = 4
+        self.pool = ThreadPoolExecutor(max_workers=self.workers)
+        self.index = -1                    # group whose entries are held
+        self.entries: list = []
+        self.pending = self._submit(0)     # (group index, read futures)
+
+    def _submit(self, g: int):
+        paths = self.paths[g * self.group:(g + 1) * self.group]
+        step = -(-len(paths) // self.workers) if paths else 1
+        return g, [self.pool.submit(_read_files, paths[i:i + step]) for i in range(0, len(paths), step)]
+
+    def prepare(self, lo: int) -> None:
+        from torchvision.io import ImageReadMode, decode_image
+
+        from .data.png import decode_entries
+
+        g = lo // self.group
+        if g == self.index:
+            return
+        self.index, self.entries = -1, []
+        _, futs = self.pending if self.pending[0] == g else self._submit(g)
+        items = [it for f in futs for it in f.result()]
+        self.pending = self._submit(g + 1)
+        pngs = [i for i, it in enumerate(items) if isinstance(it, torch.Tensor) and it.dim() == 1]
+        decoded, _ = decode_entries([items[i] for i in pngs], self.dev, lambda x: decode_image(x, ImageReadMode.GRAY))
+        entries = [it if isinstance(it, BaseException) else (it.unsqueeze(0).to(self.dev), 0) for it in items]
+        for i, e in zip(pngs, decoded):
+            entries[i] = e
+        self.index, self.entries = g, entries
+
+    def batch(self, lo: int, hi: int) -> torch.Tensor:
+        from .data.png import stack_entries
+
+        g = lo // self.group
+        if g != self.index or (hi - 1) // self.group != g:
+            raise AssertionError(f"batch [{lo}, {hi}) is not inside the prepared decode group {self.index}")
+        return stack_entries(self.entries[lo - g * self.group:hi - g * self.group])
+
+    def close(self) -> None:
+        self.pool.shutdown(wait=True, cancel_futures=True)
+
+
 @torch.no_grad()
 def predict(
     path_to_pth: str,
@@ -232,7 +307,10 @@ def predict(
         fnames_all = [str(q) for q in paths]
 
     def load_batch(lo: int, hi: int) -> torch.Tensor:
-        b = images[lo:hi] if images is not None else torch.stack([_read_image(q) for q in paths[lo:hi]])
+        if images is not None:
+            b = images[lo:hi]
+        else:
+            b = folder.batch(lo, hi)
         if crop_h is not None:   # CenterCrop((crop_h, img_w))
             top = int(round((b.shape[-2] - crop_h) / 2.0))
             b = b[..., top:top + crop_h, :]
@@ -252,49 +330,56 @@ def predict(
     normalize = bool(model.normalize_images)
     if normalize:
         model.set_fused_input_scale(1.0 / 255.0)   # uint8 batches: the /255 happens inside the first-layer kernel
-    for i, lo in enumerate(range(0, n_images, batch_size)):
-        hi = min(lo + batch_size, n_images)
-        try:
-            img_batch = load_batch(lo, hi)
-        except RuntimeError as e:   # malformed images: warn and continue, like the reference
-            warnings.warn(f"got error {e}; continuing")
-            continue
-        x = img_batch.to(dev, non_blocking=True)
-        if normalize and x.dtype != torch.uint8:
-            x = x.float() / 255.0
-        # full batches replay the forward from a CUDA graph (a batch of one 772x1032 image is ~60 us of GPU work behind
-        # ~250 us of launches); the ragged last batch runs eagerly
-        if dev.type == "cuda" and tuple(x.shape) == (batch_size,) + tuple(x.shape[1:]) and n_images >= 2 * batch_size:
-            key = (tuple(x.shape), x.dtype)
-            if graphed.get("key") != key:
-                graphed["key"], graphed["fwd"] = key, GraphedForward(model, x.shape, x.dtype)
-            res = graphed["fwd"](x)
-        else:
-            res = model(x)
-        if results is None and return_full_predictions:
-            results = torch.zeros((n_images, res.shape[1], res.shape[2], res.shape[3]))
-        if save_preds:
-            out_fnames = [Path(output_dir) / Path(f).with_suffix(".txt").name for f in fnames_all[lo:hi]]
-            save_predictions(out_fnames, res, obj_thresh=obj_thresh, iou_thresh=iou_thresh)
-        if save_npy:
-            rows, keep_count, _, _ = format_preds_batch(res, box_format="xyxy")
-            for j, r in enumerate(split_formatted(rows, keep_count)):
-                fp = r.cpu().numpy().T
-                n = fp.shape[1]
-                labels = np.argmax(fp[5:, :], axis=0).astype(np.uint8)
-                np_results.append(np.vstack((
-                    np.ones(n).astype(np.float32) * (lo + j), fp[0, :] * in_w, fp[1, :] * int(img_h.item()),
-                    fp[2, :] * in_w, fp[3, :] * int(img_h.item()), fp[4, :], labels.astype(np.float32),
-                    fp[5:, ][labels, np.arange(n)], fp[5:, :])))
-        if count_predictions:
-            _, _, _, counts = format_preds_batch(
-                res, obj_thresh=obj_thresh, iou_thresh=iou_thresh,
-                min_class_confidence_threshold=min_class_confidence_threshold)
-            tot_counts += counts
-        if return_full_predictions:
-            results[lo:hi, ...] = res.cpu()
-        if pbar is not None:
-            pbar.update(hi - lo)
+    folder = _FolderDecoder(paths, dev, batch_size) if images is None else None
+    try:
+        for i, lo in enumerate(range(0, n_images, batch_size)):
+            hi = min(lo + batch_size, n_images)
+            if folder is not None:
+                folder.prepare(lo)
+            try:
+                img_batch = load_batch(lo, hi)
+            except RuntimeError as e:   # malformed images: warn and continue, like the reference
+                warnings.warn(f"got error {e}; continuing")
+                continue
+            x = img_batch.to(dev, non_blocking=True)
+            if normalize and x.dtype != torch.uint8:
+                x = x.float() / 255.0
+            # full batches replay the forward from a CUDA graph (a batch of one 772x1032 image is ~60 us of GPU work behind
+            # ~250 us of launches); the ragged last batch runs eagerly
+            if dev.type == "cuda" and tuple(x.shape) == (batch_size,) + tuple(x.shape[1:]) and n_images >= 2 * batch_size:
+                key = (tuple(x.shape), x.dtype)
+                if graphed.get("key") != key:
+                    graphed["key"], graphed["fwd"] = key, GraphedForward(model, x.shape, x.dtype)
+                res = graphed["fwd"](x)
+            else:
+                res = model(x)
+            if results is None and return_full_predictions:
+                results = torch.zeros((n_images, res.shape[1], res.shape[2], res.shape[3]))
+            if save_preds:
+                out_fnames = [Path(output_dir) / Path(f).with_suffix(".txt").name for f in fnames_all[lo:hi]]
+                save_predictions(out_fnames, res, obj_thresh=obj_thresh, iou_thresh=iou_thresh)
+            if save_npy:
+                rows, keep_count, _, _ = format_preds_batch(res, box_format="xyxy")
+                for j, r in enumerate(split_formatted(rows, keep_count)):
+                    fp = r.cpu().numpy().T
+                    n = fp.shape[1]
+                    labels = np.argmax(fp[5:, :], axis=0).astype(np.uint8)
+                    np_results.append(np.vstack((
+                        np.ones(n).astype(np.float32) * (lo + j), fp[0, :] * in_w, fp[1, :] * int(img_h.item()),
+                        fp[2, :] * in_w, fp[3, :] * int(img_h.item()), fp[4, :], labels.astype(np.float32),
+                        fp[5:, ][labels, np.arange(n)], fp[5:, :])))
+            if count_predictions:
+                _, _, _, counts = format_preds_batch(
+                    res, obj_thresh=obj_thresh, iou_thresh=iou_thresh,
+                    min_class_confidence_threshold=min_class_confidence_threshold)
+                tot_counts += counts
+            if return_full_predictions:
+                results[lo:hi, ...] = res.cpu()
+            if pbar is not None:
+                pbar.update(hi - lo)
+    finally:
+        if folder is not None:
+            folder.close()
     if pbar is not None:
         pbar.close()
 
