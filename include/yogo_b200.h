@@ -350,6 +350,24 @@ int yg_dd_gather_images(const void* store, void* out, int dtype, const int* tabl
                         int N, int C, int H, int W, void* stream);
 int yg_dd_build_labels(const int* table, const int* flags, int stride, const void* records, const long long* rec_off,
                        int N, int Sy, int Sx, float* out, void* stream);
+/* Sharded store (a dataset larger than one GPU, spread over the ranks of one host; data/device_dataset.py):
+ * yg_dd_gather_images_peers writes what yg_dd_gather_images writes, bit for bit, but stored slot s is image
+ * s % shard_items of shards[s / shard_items]; shards is a DEVICE array of W base pointers (this rank's own shard and the
+ * peers' shards opened with yg_dd_shard_open), each the start of an allocation.
+ * Shard memory: yg_dd_shard_alloc is a plain cudaMalloc on the current device (its own allocation, so that its IPC
+ * handle maps exactly the buffer); yg_dd_shard_export writes its YG_IPC_HANDLE_BYTES-byte handle to `handle` (host
+ * memory); yg_dd_shard_open maps a handle exported by ANOTHER process of this host on the current device (peer access
+ * enabled lazily); yg_dd_shard_close unmaps it; yg_dd_shard_free frees an own shard.  Teardown is a protocol across
+ * processes: every importer synchronises and closes its handles, all processes meet in a barrier, and only then does each
+ * owner free (freeing memory another process still has open is undefined in CUDA). */
+#define YG_IPC_HANDLE_BYTES 64
+int yg_dd_gather_images_peers(const void* const* shards, long long shard_items, void* out, int dtype, const int* table,
+                              const int* flags, int stride, int N, int C, int H, int W, void* stream);
+int yg_dd_shard_alloc(size_t bytes, void** ptr);
+int yg_dd_shard_export(const void* ptr, void* handle);
+int yg_dd_shard_open(const void* handle, void** ptr);
+int yg_dd_shard_close(void* ptr);
+int yg_dd_shard_free(void* ptr);
 
 /* ---- PNG decoding: 8-bit grayscale, non-interlaced files (yogo_b200.data.decode_png_batch) ----------------------
  * One call decodes n files of the same H x W.  `files` (device, files_bytes) holds what the host uploaded; the host has

@@ -15,6 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libyogo_b200.so")
 
 YG_F32, YG_BF16, YG_U8 = 0, 1, 2
+YG_IPC_HANDLE_BYTES = 64
 ACT_NONE, ACT_LRELU, ACT_SILU = 0, 1, 2
 IMPL_AUTO, IMPL_SIMT, IMPL_TCGEN05 = 0, 1, 2
 
@@ -188,6 +189,14 @@ _PROTOS = {
     "yg_dd_draw": (c_int, [c_void_p, c_void_p, c_float, c_float, c_int, c_int, c_void_p]),
     "yg_dd_gather_images": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "yg_dd_build_labels": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "yg_dd_gather_images_peers": (
+        c_int, [c_void_p, c_longlong, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p],
+    ),
+    "yg_dd_shard_alloc": (c_int, [c_size_t, C.POINTER(c_void_p)]),
+    "yg_dd_shard_export": (c_int, [c_void_p, c_void_p]),
+    "yg_dd_shard_open": (c_int, [c_void_p, C.POINTER(c_void_p)]),
+    "yg_dd_shard_close": (c_int, [c_void_p]),
+    "yg_dd_shard_free": (c_int, [c_void_p]),
     "yg_png_gray8_workspace": (c_size_t, [c_int, c_int, c_int, c_longlong]),
     "yg_png_decode_gray8": (
         c_int,

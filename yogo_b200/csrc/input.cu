@@ -3,6 +3,9 @@
 // (6, Sy, Sx) label tensor (/root/reference/yogo/data/yogo_dataset.py:24-46), whole batch per launch.
 // HBM-bound byte/element shuffles: 8- or 16-byte accesses on both sides, nothing is re-read.
 #include "common.cuh"
+#include <string.h>
+#include <algorithm>
+#include <type_traits>
 
 namespace yg {
 
@@ -309,6 +312,63 @@ __global__ void __launch_bounds__(256) dd_labels_kernel(const int* __restrict__ 
     for (int k = 0; k < 6; ++k) o[k * plane + oc] = v[k];
   }
 }
+
+// Sharded store (each rank of one host keeps a contiguous 1/W of the slots, peers' shards mapped over NVLink): stored
+// slot s is image s % shard_items of shards[s / shard_items].  One block = `rpb` consecutive rows of one output plane, so
+// the source plane is resolved once per block; every thread issues PG_UNROLL independent vector loads before its first
+// store, which keeps enough bytes in flight to cover a remote round trip.  Same output as flip_images_kernel<GatherSrc>.
+constexpr int PG_THREADS = 256, PG_UNROLL = 8;
+template <typename T, int V>
+__global__ void __launch_bounds__(PG_THREADS) dd_gather_peers_kernel(const T* const* __restrict__ shards, long long shard_items,
+                                                                     T* __restrict__ out, const int* __restrict__ table,
+                                                                     const int* __restrict__ flags, int stride, int C, int H,
+                                                                     int W, int rpb, int blocks_per_plane) {
+  struct alignas(sizeof(T) * V) Vec { T e[V]; };
+  const int hflip = flags[0], vflip = flags[1];
+  const int plane = blockIdx.x / blocks_per_plane;   // n * C + c
+  const int y0 = (blockIdx.x - plane * blocks_per_plane) * rpb;
+  const int n = plane / C, c = plane - n * C;
+  const long long s = table[(long long)flags[2] * stride + n];
+  const long long shard = s / shard_items, item = s - shard * shard_items;
+  const long long plane_elems = (long long)H * W;
+  const T* src = shards[shard] + (item * C + c) * plane_elems;
+  T* dst = out + (long long)plane * plane_elems + (long long)y0 * W;
+  const int vpr = W / V;
+  const int total = min(rpb, H - y0) * vpr;
+  for (int i0 = threadIdx.x; i0 < total; i0 += PG_THREADS * PG_UNROLL) {
+    Vec v[PG_UNROLL];
+#pragma unroll
+    for (int u = 0; u < PG_UNROLL; ++u) {
+      const int idx = i0 + u * PG_THREADS;
+      if (idx < total) {
+        const int r = idx / vpr, vx = idx - r * vpr;
+        const int sy = vflip ? H - 1 - (y0 + r) : y0 + r;
+        const int sv = hflip ? vpr - 1 - vx : vx;
+        v[u] = *reinterpret_cast<const Vec*>(src + (long long)sy * W + sv * V);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < PG_UNROLL; ++u) {
+      const int idx = i0 + u * PG_THREADS;
+      if (idx < total) {
+        const int r = idx / vpr, vx = idx - r * vpr;
+        Vec o = v[u];
+        if (hflip) {
+          if constexpr (sizeof(T) == 1 && V >= 4) {   // byte reversal as word swaps + byte permutes
+            uint32_t* ow = reinterpret_cast<uint32_t*>(o.e);
+            const uint32_t* iw = reinterpret_cast<const uint32_t*>(v[u].e);
+#pragma unroll
+            for (int k = 0; k < V / 4; ++k) ow[k] = __byte_perm(iw[V / 4 - 1 - k], 0, 0x0123);
+          } else {
+#pragma unroll
+            for (int k = 0; k < V; ++k) o.e[k] = v[u].e[V - 1 - k];
+          }
+        }
+        *reinterpret_cast<Vec*>(dst + (long long)r * W + vx * V) = o;
+      }
+    }
+  }
+}
 }  // namespace yg
 
 extern "C" int yg_dd_draw(void* state, int* flags, float p_hflip, float p_vflip, int stream_id, int nbatches, void* stream) {
@@ -340,6 +400,86 @@ extern "C" int yg_dd_gather_images(const void* store, void* out, int dtype, cons
     else flip_images_kernel<float, 1><<<flip_grid(rows), 256, 0, st>>>((const float*)store, (float*)out, rows, H, W, g);
   }
   YG_LAUNCH_CHECK("dd_gather_images");
+  return YG_OK;
+}
+
+extern "C" int yg_dd_gather_images_peers(const void* const* shards, long long shard_items, void* out, int dtype,
+                                         const int* table, const int* flags, int stride, int N, int C, int H, int W,
+                                         void* stream) {
+  YG_CHECK_ARG(dtype == YG_U8 || dtype == YG_F32, "dd_gather_images_peers: dtype %d", dtype);
+  YG_CHECK_ARG(C == 1 || C == 3, "dd_gather_images_peers: C = %d (1 or 3)", C);
+  const long long rows = (long long)N * C * H;
+  if (rows == 0 || W == 0) return YG_OK;
+  YG_CHECK_ARG(shards && out && table && flags && shard_items > 0 && N <= stride && H > 0 && W > 0,
+               "dd_gather_images_peers: bad arguments");
+  YG_CHECK_ARG(rows / FLIP_ROWS < (1LL << 31), "dd_gather_images_peers: too many rows");
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool al = ((uintptr_t)out & 15) == 0;   // shard bases are allocation starts (256-byte aligned)
+  auto launch = [&](auto* tp, auto vw) -> int {
+    using T = std::remove_pointer_t<decltype(tp)>;
+    constexpr int V = decltype(vw)::value;
+    const int vpr = W / V;
+    const int rpb = std::max(1, std::min(H, PG_THREADS * PG_UNROLL / vpr));
+    const int bpp = (H + rpb - 1) / rpb;
+    const long long blocks = (long long)N * C * bpp;
+    YG_CHECK_ARG(blocks < (1LL << 31), "dd_gather_images_peers: too many rows");
+    dd_gather_peers_kernel<T, V><<<(unsigned)blocks, PG_THREADS, 0, st>>>((const T* const*)shards, shard_items, (T*)out, table,
+                                                                          flags, stride, C, H, W, rpb, bpp);
+    return YG_OK;
+  };
+  using std::integral_constant;
+  int rc;
+  if (dtype == YG_U8) {
+    if (al && W % 16 == 0) rc = launch((uint8_t*)nullptr, integral_constant<int, 16>{});
+    else if (al && W % 8 == 0) rc = launch((uint8_t*)nullptr, integral_constant<int, 8>{});
+    else rc = launch((uint8_t*)nullptr, integral_constant<int, 1>{});
+  } else {
+    if (al && W % 4 == 0) rc = launch((float*)nullptr, integral_constant<int, 4>{});
+    else rc = launch((float*)nullptr, integral_constant<int, 1>{});
+  }
+  if (rc != YG_OK) return rc;
+  YG_LAUNCH_CHECK("dd_gather_images_peers");
+  return YG_OK;
+}
+
+// Shard memory of a sharded store: plain cudaMalloc (an allocation of its own, so its IPC handle maps exactly this
+// buffer), exported to and opened by the other processes of the host.  Teardown order is the caller's protocol
+// (DeviceResidentDataset.close): every importer closes its handle before the owner frees.
+static_assert(sizeof(cudaIpcMemHandle_t) == YG_IPC_HANDLE_BYTES, "IPC handle size");
+
+extern "C" int yg_dd_shard_alloc(size_t bytes, void** ptr) {
+  YG_CHECK_ARG(ptr && bytes > 0, "dd_shard_alloc: bad arguments");
+  *ptr = nullptr;
+  YG_CUDA(cudaMalloc(ptr, bytes));
+  return YG_OK;
+}
+
+extern "C" int yg_dd_shard_export(const void* ptr, void* handle) {
+  YG_CHECK_ARG(ptr && handle, "dd_shard_export: bad arguments");
+  cudaIpcMemHandle_t h;
+  YG_CUDA(cudaIpcGetMemHandle(&h, const_cast<void*>(ptr)));
+  memcpy(handle, &h, sizeof(h));
+  return YG_OK;
+}
+
+extern "C" int yg_dd_shard_open(const void* handle, void** ptr) {
+  YG_CHECK_ARG(handle && ptr, "dd_shard_open: bad arguments");
+  *ptr = nullptr;
+  cudaIpcMemHandle_t h;
+  memcpy(&h, handle, sizeof(h));
+  YG_CUDA(cudaIpcOpenMemHandle(ptr, h, cudaIpcMemLazyEnablePeerAccess));
+  return YG_OK;
+}
+
+extern "C" int yg_dd_shard_close(void* ptr) {
+  YG_CHECK_ARG(ptr, "dd_shard_close: null pointer");
+  YG_CUDA(cudaIpcCloseMemHandle(ptr));
+  return YG_OK;
+}
+
+extern "C" int yg_dd_shard_free(void* ptr) {
+  YG_CHECK_ARG(ptr, "dd_shard_free: null pointer");
+  YG_CUDA(cudaFree(ptr));
   return YG_OK;
 }
 

@@ -9,6 +9,11 @@ all-gathers so that every rank holds the full store) and afterwards builds each 
 own state from device memory, so they run inside the captured training step (``DataParallelTrainer.steps_from_device``)
 and the host does no per-step data work.
 
+A store too large for one GPU is sharded instead (``placement``): when the full store does not fit beside the training
+reserve but a 1/W shard does, and all ranks run on one host, each rank keeps only the images it decoded, in a buffer of
+its own that the other ranks map through CUDA IPC, and the gather kernel reads the other ranks' images over NVLink.  The
+batches are bit-identical to the replicated store's.  A sharded store must be released with the collective ``close()``.
+
 What it computes: batch i of epoch e is ``flip_batch(collate([dataset[j] for j in idx]), h, v)`` where ``idx`` is batch
 i of the reference's ``DistributedSampler(shuffle=True, seed=seed, drop_last=False)`` with ``set_epoch(e)``, in batches
 of ``batch_size`` with the ragged last batch kept, and ``(h, v)`` are drawn on the device with the flip modules' ``p``.
@@ -20,8 +25,10 @@ Deviations from the reference's DataLoader:
 """
 from __future__ import annotations
 
+import socket
 import warnings
-from typing import Iterator, List, Tuple
+from ctypes import byref, c_void_p, create_string_buffer
+from typing import Callable, Iterator, List, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
@@ -92,6 +99,133 @@ def check_capacity(needed: int, free: int, reserve: int = DEFAULT_RESERVE_BYTES)
                          f"{free} bytes free ({free / 2**30:.2f} GiB), of which {reserve} are kept for training")
 
 
+def _rank_ranges(hosts: Sequence) -> str:
+    """'ranks 0-3 on host a, 4-7 on host b' for the per-rank host names `hosts`."""
+    parts, start = [], 0
+    for r in range(1, len(hosts) + 1):
+        if r == len(hosts) or hosts[r] != hosts[start]:
+            span = f"{start}" if r - 1 == start else f"{start}-{r - 1}"
+            parts.append(f"{span} on host {hosts[start]}")
+            start = r
+    return "ranks " + ", ".join(parts)
+
+
+def placement(full_bytes: int, shard_bytes: int, free: Sequence[int], reserve: Sequence[int], hosts: Sequence) -> str:
+    """Where the images of a store go, from what every rank observed (per rank: `free` device bytes, the `reserve` kept
+    for training, `hosts` = (host name, boot id)): 'replicated' when `full_bytes` fit beside the reserve on every rank,
+    'sharded' when only `shard_bytes` (a rank's 1/W of the image slots plus the replicated label and index tables) fit
+    and every rank runs on one host.  ValueError otherwise, naming both byte counts, the free bytes and why sharding was
+    not possible.  Every rank passes the same gathered lists, so every rank takes the same branch."""
+    world = len(free)
+    available = [f - r for f, r in zip(free, reserve)]
+    worst = min(range(world), key=lambda r: available[r])
+    if full_bytes <= available[worst]:
+        return "replicated"
+    if world == 1:
+        check_capacity(full_bytes, free[0], reserve[0])
+    need = (f"the device-resident dataset needs {full_bytes} bytes ({full_bytes / 2**30:.2f} GiB) but rank {worst} has "
+            f"{free[worst]} bytes free ({free[worst] / 2**30:.2f} GiB), of which {reserve[worst]} are kept for training")
+    if shard_bytes > available[worst]:
+        raise ValueError(f"{need}; a shard over {world} ranks needs {shard_bytes} bytes ({shard_bytes / 2**30:.2f} GiB) "
+                         f"per rank, which does not fit either")
+    if len(set(hosts)) > 1:
+        raise ValueError(f"{need}; a shard over {world} ranks ({shard_bytes} bytes per rank) would fit, but a sharded "
+                         f"store needs every rank on one host and there are {_rank_ranges([h[0] for h in hosts])}")
+    return "sharded"
+
+
+def _host_id() -> Tuple[str, str]:
+    """(host name, boot id): two processes can map each other's device memory only on the same running host."""
+    try:
+        with open("/proc/sys/kernel/random/boot_id") as f:
+            boot = f.read().strip()
+    except OSError:
+        boot = ""
+    return socket.gethostname(), boot
+
+
+class _CudaBuffer:
+    """`__cuda_array_interface__` of raw device bytes, so that torch.as_tensor gives a (non-owning) uint8 view."""
+
+    def __init__(self, ptr: int, nbytes: int):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+
+
+class ShardMemory:
+    """This rank's image shard of a sharded store and the peers' shards it has mapped.
+
+    The own shard is its own cudaMalloc allocation (exportable by IPC handle).  Teardown is collective: `close()`
+    synchronises, meets the other ranks in a barrier, closes every mapped peer shard, meets them again and only then frees
+    the own shard, so no rank frees memory a peer can still read.  A ShardMemory collected without `close()` closes its
+    mappings but never frees the own shard (its memory returns at process exit).  `lib`, `barrier` and `synchronize` are
+    parameters so that the protocol can be checked with a fake library."""
+
+    def __init__(self, lib, nbytes: int, barrier: Callable[[], None], synchronize: Callable[[], None]):
+        self._lib, self._barrier, self._sync = lib, barrier, synchronize
+        self.nbytes = int(nbytes)
+        self.peers: List[int] = []     # opened peer pointers
+        self.shared = False            # every rank exported its handle: peers may map the own shard
+        self.closed = True             # nothing to release until the allocation succeeded
+        p = c_void_p()
+        L.check(lib.yg_dd_shard_alloc(self.nbytes, byref(p)))
+        self.ptr = int(p.value)
+        self.closed = False
+
+    def export(self) -> bytes:
+        buf = create_string_buffer(L.YG_IPC_HANDLE_BYTES)
+        L.check(self._lib.yg_dd_shard_export(self.ptr, buf))
+        return buf.raw
+
+    def mark_shared(self) -> None:
+        """Called on every rank once every rank has exported its handle (the handles are exchanged next): from here on
+        the own shard is freed only through the collective `close()`.  Set on all ranks or on none, so the barriers of a
+        failed build's cleanup always pair up."""
+        self.shared = True
+
+    def open(self, handle: bytes) -> int:
+        p = c_void_p()
+        L.check(self._lib.yg_dd_shard_open(handle, byref(p)))
+        self.peers.append(int(p.value))
+        return self.peers[-1]
+
+    def _close_peers(self) -> None:
+        while self.peers:
+            L.check(self._lib.yg_dd_shard_close(self.peers.pop()))
+
+    def close(self) -> None:
+        """Collective: every rank of the store calls it."""
+        if self.closed:
+            return
+        self.closed = True
+        self._sync()
+        self._barrier()          # no rank still reads a shard
+        self._close_peers()
+        self._barrier()          # no rank still maps a shard
+        L.check(self._lib.yg_dd_shard_free(self.ptr))
+
+    def release_after_failed_build(self) -> None:
+        """Free after an exception of the build.  Once the shard is shared (every rank exported, handles exchanged), every
+        rank raises together (the build gathers every rank's status), so the barriers of `close` pair up; before that no
+        peer can have mapped the shard and it is freed at once."""
+        if self.shared:
+            self.close()
+        else:
+            self.closed = True
+            L.check(self._lib.yg_dd_shard_free(self.ptr))
+
+    def __del__(self):
+        if self.closed:
+            return
+        self.closed = True
+        try:
+            self._sync()
+            self._close_peers()
+        except Exception:
+            pass
+        warnings.warn("DeviceResidentDataset: a sharded store was collected without close(); its shard "
+                      f"({self.nbytes} bytes) stays allocated until the process exits, since a peer may still map it")
+
+
 def compact_labels(labels: torch.Tensor) -> torch.Tensor:
     """(6, Sy, Sx) fp32 -> (k, 8) int32 records {cell, six channel bit patterns, 0} of the k cells with any non-zero bit,
     in cell order.  The label kernel writes +0.0 (mirrored) into every other cell, so the dense tensor round-trips exactly."""
@@ -132,12 +266,19 @@ class DeviceResidentDataset:
         self.reserve_bytes = int(reserve_bytes)
         self._images = self._records = self._rec_off = self._slots = self._table = None
         self._state = self._flags = None
+        self._mem: ShardMemory = None
+        self._shard_ptrs = None
+        self.sharded = False
+        self._closed = False
         with torch.cuda.device(self.device):
             try:
                 self._build(dataset, num_workers)
             except BaseException:
                 self._images = self._records = self._rec_off = self._slots = self._table = None
-                self._state = self._flags = None
+                self._state = self._flags = self._shard_ptrs = None
+                if self._mem is not None:
+                    mem, self._mem = self._mem, None
+                    mem.release_after_failed_build()
                 raise
 
     # ------------------------------------------------------------------ build
@@ -175,10 +316,27 @@ class DeviceResidentDataset:
         item_bytes = C * H * W * (1 if idt == torch.uint8 else 4)
         n_slots = chunk * world
         samples = -(-n_items // world)
-        # images and index tables are known now; label records are checked again once decoded
-        check_capacity(store_bytes(n_slots, item_bytes, 0, samples, self.batch_size), torch.cuda.mem_get_info(dev)[0],
-                       self.reserve_bytes)
-        self._images = torch.zeros((n_slots, C, H, W), dtype=idt, device=dev)
+        # images and index tables are known now; label records are checked again once decoded.  The store is
+        # replicated when it fits on every rank, else sharded (each rank keeps the `chunk` slots it decodes) if a shard
+        # fits and the ranks can map each other's memory.
+        full = store_bytes(n_slots, item_bytes, 0, samples, self.batch_size)
+        shard = full - (n_slots - chunk) * item_bytes + world * 8
+        seen = [(torch.cuda.mem_get_info(dev)[0], self.reserve_bytes, None)]
+        if world > 1:
+            seen = [None] * world
+            dist.all_gather_object(seen, (torch.cuda.mem_get_info(dev)[0], self.reserve_bytes, _host_id()), group=self.pg)
+        self.sharded = placement(full, shard, *zip(*seen)) == "sharded"
+        if self.sharded:
+            pg = self.pg
+            self._mem = ShardMemory(L.lib(), chunk * item_bytes, lambda: dist.barrier(group=pg),
+                                    lambda: torch.cuda.synchronize(dev))
+            self._images = torch.as_tensor(_CudaBuffer(self._mem.ptr, chunk * item_bytes), device=dev).view(idt)
+            self._images = self._images.view(chunk, C, H, W)
+            self._images.zero_()
+            slot0 = 0
+        else:
+            self._images = torch.zeros((n_slots, C, H, W), dtype=idt, device=dev)
+            slot0 = rank * chunk
 
         valid = torch.zeros(chunk, dtype=torch.uint8)
         records: List[torch.Tensor] = []
@@ -203,7 +361,7 @@ class DeviceResidentDataset:
                 records.append(rec)
                 counts[pos + j] = rec.shape[0]
                 valid[pos + j] = 1
-            s0 = rank * chunk + pos
+            s0 = slot0 + pos
             self._images[s0:s0 + len(batch)].copy_(imgs)
             pos += len(batch)
             batch = next(it, None)
@@ -211,11 +369,13 @@ class DeviceResidentDataset:
         recs = torch.cat(records) if records else torch.zeros((0, RECORD_WORDS), dtype=torch.int32)
 
         if world > 1:
-            # images: in-place all-gather of the equal per-rank slot ranges; labels: variable-size, padded to the largest
-            flat = self._images.view(torch.uint8).reshape(-1)
-            part = chunk * item_bytes
-            dist.all_gather_into_tensor(flat, flat[rank * part:(rank + 1) * part], group=self.pg)
-            del flat
+            # images (replicated): in-place all-gather of the equal per-rank slot ranges; labels: variable-size, padded to
+            # the largest
+            if not self.sharded:
+                flat = self._images.view(torch.uint8).reshape(-1)
+                part = chunk * item_bytes
+                dist.all_gather_into_tensor(flat, flat[rank * part:(rank + 1) * part], group=self.pg)
+                del flat
             meta = torch.cat([valid.to(torch.int64), counts]).to(dev)
             metas = torch.empty((world, 2 * chunk), dtype=torch.int64, device=dev)
             dist.all_gather_into_tensor(metas, meta, group=self.pg)
@@ -256,10 +416,69 @@ class DeviceResidentDataset:
         self._table = torch.zeros(self.num_batches() * self.batch_size, dtype=torch.int32, device=dev)
         self._state = torch.tensor([self.seed, 0, 0], dtype=torch.int64, device=dev)
         self._flags = torch.zeros(4, dtype=torch.int32, device=dev)
-        self.nbytes = (self._images.numel() * self._images.element_size() + self._records.numel() * 4 +
-                       self._rec_off.numel() * 8 + self._table.numel() * 4)
+        if self.sharded:
+            self._map_shards()
+        self.shard_bytes = self._images.numel() * self._images.element_size()
+        self.nbytes = (self.shard_bytes + self._records.numel() * 4 + self._rec_off.numel() * 8 + self._table.numel() * 4 +
+                       (self._shard_ptrs.numel() * 8 if self.sharded else 0))
         self.epoch = None
         torch.cuda.synchronize(dev)
+
+    def _on_every_rank(self, what: str, fn):
+        """`fn()` on every rank; if it raises on any rank, every rank raises (naming each failure) instead of one rank
+        raising while the others wait in the next collective.  The status gather is a barrier."""
+        out, err = None, None
+        try:
+            out = fn()
+        except Exception as e:
+            err = f"{type(e).__name__}: {e}"
+        errs = [None] * self.world
+        dist.all_gather_object(errs, err, group=self.pg)
+        bad = [f"rank {r}: {e}" for r, e in enumerate(errs) if e is not None]
+        if bad:
+            raise L.YogoB200Error(f"DeviceResidentDataset: {what} failed on " + "; ".join(bad))
+        return out
+
+    def _map_shards(self) -> None:
+        """Exchange the shards' IPC handles, map every peer's shard and upload the W base pointers.  Each rank's shard is
+        complete before its handle leaves (device synchronise), and the final status gather keeps every rank from
+        reading before all are mapped."""
+        dev, mem = self.device, self._mem
+
+        def export():
+            torch.cuda.synchronize(dev)
+            return mem.export()
+
+        handle = self._on_every_rank("exporting the shard", export)
+        mem.mark_shared()        # every rank reported a handle: on all ranks or, after a raise above, on none
+        handles = [None] * self.world
+        dist.all_gather_object(handles, handle, group=self.pg)
+
+        def open_peers():
+            ptrs = [mem.ptr if r == self.rank else mem.open(h) for r, h in enumerate(handles)]
+            self._shard_ptrs = torch.tensor(ptrs, dtype=torch.int64).to(dev)
+            torch.cuda.synchronize(dev)
+
+        self._on_every_rank("mapping the peers' shards (a sharded store needs CUDA IPC between the ranks of one host)",
+                            open_peers)
+
+    def close(self) -> None:
+        """Release the store; afterwards `next_batch_into` and `begin_epoch` raise.  For a sharded store this is
+        collective, every rank calls it (before destroy_process_group): device synchronise, barrier, unmap the peers'
+        shards, barrier, free the own shard."""
+        if self._closed:
+            return
+        self._closed = True
+        self._images = self._records = self._rec_off = self._slots = self._table = None
+        self._state = self._flags = self._shard_ptrs = None
+        if self._mem is not None:
+            mem, self._mem = self._mem, None
+            with torch.cuda.device(self.device):
+                mem.close()
+
+    def _check_open(self) -> None:
+        if self._closed:
+            raise L.YogoB200Error("DeviceResidentDataset: the store was closed")
 
     # ------------------------------------------------------------------ sampling
     def __len__(self) -> int:
@@ -279,6 +498,7 @@ class DeviceResidentDataset:
 
     def begin_epoch(self, epoch: int) -> None:
         """Upload the epoch's index table (the only host-to-device transfer of an epoch) and rewind the batch cursor."""
+        self._check_open()
         idx = torch.tensor([i for b in self.epoch_batches(epoch) for i in b], dtype=torch.int64)
         table = torch.full((self._table.numel(),), int(self._slots[0]), dtype=torch.int32)
         table[:idx.numel()] = self._slots[idx]
@@ -290,6 +510,7 @@ class DeviceResidentDataset:
     def next_batch_into(self, images: torch.Tensor, labels: torch.Tensor) -> None:
         """Draw the flips of the next batch of the current epoch and write it into `images` (n, C, H, W) and `labels`
         (n, 6, Sy, Sx), n = this batch's size.  Graph-capturable: nothing is read back to the host."""
+        self._check_open()
         n = images.shape[0]
         C, H, W = self.image_shape
         Sy, Sx = self.grid
@@ -299,8 +520,13 @@ class DeviceResidentDataset:
         lib, st = L.lib(), L.stream()
         L.check(lib.yg_dd_draw(self._state.data_ptr(), self._flags.data_ptr(), self.p_hflip, self.p_vflip, self.rank,
                                 self.num_batches(), st))
-        L.check(lib.yg_dd_gather_images(self._images.data_ptr(), images.data_ptr(), L.dtype_code(self.image_dtype),
-                                        self._table.data_ptr(), self._flags.data_ptr(), self.batch_size, n, C, H, W, st))
+        if self.sharded:
+            L.check(lib.yg_dd_gather_images_peers(self._shard_ptrs.data_ptr(), self._images.shape[0], images.data_ptr(),
+                                                  L.dtype_code(self.image_dtype), self._table.data_ptr(),
+                                                  self._flags.data_ptr(), self.batch_size, n, C, H, W, st))
+        else:
+            L.check(lib.yg_dd_gather_images(self._images.data_ptr(), images.data_ptr(), L.dtype_code(self.image_dtype),
+                                            self._table.data_ptr(), self._flags.data_ptr(), self.batch_size, n, C, H, W, st))
         L.check(lib.yg_dd_build_labels(self._table.data_ptr(), self._flags.data_ptr(), self.batch_size,
                                        self._records.data_ptr(), self._rec_off.data_ptr(), n, Sy, Sx, labels.data_ptr(), st))
 
